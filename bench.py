@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- object-iterations/sec of the fused superquadric optimiser on B200 (see DESIGN.md, 'Measurement').
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -23,6 +23,9 @@ cpu_baseline / --impl reference   the reference's optimiser loop (oracle/torch_o
 sfu     roofline.sfu: one MUFU.RCP per point-view (1000 per unit) against 148 SMs x 16 SFU lanes x clock.
 e2e_call_site   the reference-facing entry point itself: 82-column tracks -> odam_b200.run_multi_view.optim_process ->
         result dict (staging, H2D, kernel, D2H, oriented boxes on the device, result objects), host buffers throughout.
+--dump-outputs DIR   what the last timed step returned (native: params, loss, status of rank 0, plus the all-gathered
+        params with several GPUs; reference: params and loss of its sample) as DIR/<name>.npy.  Inputs are seeded, so
+        two builds run with the same arguments can be compared output for output.
 Multi-GPU: the headline stays weak scaling -- every rank optimises its own scene of the named shape (objects are
 independent, no data-path collective) and the final parameters are all-gathered over NCCL inside the timed step -- and
 `strong` carries what north_star names: ONE batch (BASELINE configs 3 and 5) sharded by object across the N ranks
@@ -134,14 +137,15 @@ def workload(cfg_idx, rank, n_objects=None, device="cpu"):
 
 # ------------------------------------------------------------------------------------------------------
 def cpu_port_worker(job):
-    """One object of the reference loop on one core (module-level so that multiprocessing can pickle it)."""
+    """One object of the reference loop on one core (module-level so that multiprocessing can pickle it).
+    Returns (seconds, final parameters [9], loss of every iteration)."""
     import torch
     torch.set_num_threads(job["threads"])
     from oracle import torch_oracle
     t0 = time.perf_counter()
-    torch_oracle.run(job["translate"], job["angle"], job["dims"], job["Ms"], job["box"], job["mask"], job["prior33"],
-                     n_iters=job["iters"], representation="super_quadric", anomaly=True, record=False)
-    return time.perf_counter() - t0
+    r = torch_oracle.run(job["translate"], job["angle"], job["dims"], job["Ms"], job["box"], job["mask"], job["prior33"],
+                         n_iters=job["iters"], representation="super_quadric", anomaly=True, record=False)
+    return time.perf_counter() - t0, r["final"], r["loss"]
 
 
 def cpu_jobs(scene, tracks, prior, objs, iters, threads):
@@ -182,7 +186,7 @@ def cpu_baseline_config1(budget_s=40.0, threads=None, max_objects=None):
     threads = threads or default_threads
     done, t_total = 0, 0.0
     for i in range(scene.n if max_objects is None else min(scene.n, max_objects)):
-        t_total += cpu_port_worker(cpu_jobs(scene, tracks, prior, [i], c["n_iters"], threads)[0])
+        t_total += cpu_port_worker(cpu_jobs(scene, tracks, prior, [i], c["n_iters"], threads)[0])[0]
         done += 1
         if t_total > budget_s:
             break
@@ -207,7 +211,7 @@ def cpu_baseline_sequential(scene, tracks, prior, budget_s=15.0):
     threads = torch.get_num_threads()
     iters, done, t_total = 40, 0, 0.0
     for i in range(min(scene.n, 64)):
-        t_total += cpu_port_worker(cpu_jobs(scene, tracks, prior, [i], iters, threads)[0])
+        t_total += cpu_port_worker(cpu_jobs(scene, tracks, prior, [i], iters, threads)[0])[0]
         done += 1
         if t_total > budget_s:
             break
@@ -239,10 +243,12 @@ def run_reference(args):
     with mp.get_context("spawn").Pool(min(cores, n_obj)) as pool:
         for k in range(args.warmup + args.steps):
             t0 = time.perf_counter()
-            pool.map(cpu_port_worker, jobs, chunksize=1)
+            res = pool.map(cpu_port_worker, jobs, chunksize=1)
             dt = time.perf_counter() - t0
             if k >= args.warmup:
                 times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"params": np.stack([r[1] for r in res]), "loss": np.stack([r[2] for r in res])})
     ms = 1e3 * float(np.mean(times))
     value = units / (ms / 1e3)
     sample = (f"{n_obj} objects x {scene.V} views x {iters} iterations per step (of {scene.n} x {scene.V} x "
@@ -328,6 +334,12 @@ def run_native(args):
     ms_per_step = total_ms / args.steps
     value = world * units_rank / (ms_per_step / 1e3)
     status = out["status"].cpu().numpy()
+    # host copies now: the multi-GPU e2e steps below reuse `out` and `gath`
+    last_step = None
+    if args.dump_outputs and rank == 0:
+        last_step = {k: v.cpu().numpy() for k, v in out.items()}
+        if world > 1:
+            last_step["params_all_ranks"] = gath.cpu().numpy()
 
     # ---- e2e through the host-buffer API (H2D + kernel + D2H inside the timed region) ----
     e2e_steps = max(3, min(args.steps, 10))
@@ -466,6 +478,8 @@ def run_native(args):
         line["cpu_baseline"] = cpu_baseline_config1(args.cpu_budget * 2.5)
         line["cpu_baseline_headline_config"] = cpu_baseline_sequential(scene, tracks, prior, args.cpu_budget)
         line["cpu_baseline_1thread"] = cpu_baseline_config1(args.cpu_budget, threads=1, max_objects=3)   # SURVEY 8d: 1 thread too
+    if last_step is not None:
+        dump_outputs(args.dump_outputs, last_step)
     emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -572,6 +586,28 @@ def emit(line):
     os.write(_REAL_STDOUT if _REAL_STDOUT is not None else 1, (json.dumps(line) + "\n").encode())
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: each array as path/<name>.npy, floats as float32/float64 and integers (status flags, indices) as
+    float64, so that two builds can be compared output for output.  Beyond DUMP_LIMIT_BYTES in all, every array keeps
+    the same share of its rows, drawn with a fixed seed, and the kept row indices go to path/<name>_rows.npy."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float32 if v.dtype.kind == "f" else np.float64)
+              for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    # when sampling, the kept row indices (8 bytes a row) count too, and 1 MiB is left for the .npy headers
+    scale = (DUMP_LIMIT_BYTES - (1 << 20)) / sum(v.nbytes + 8 * (len(v) if v.ndim else 0) for v in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES and a.ndim and len(a) > 1:
+            keep = max(1, int(len(a) * scale))
+            rows = np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+            a = a[rows]
+            np.save(os.path.join(path, f"{name}_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -589,7 +625,13 @@ def main():
     ap.add_argument("--clocks", default="smi", choices=["smi", "off"], help="clock sampler (off: diagnostics only)")
     ap.add_argument("--cpu-budget", type=float, default=15.0)
     ap.add_argument("--ref-iters", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
     claim_stdout()
     if args.impl == "reference":
         run_reference(args)

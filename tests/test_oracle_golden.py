@@ -28,14 +28,6 @@ def test_c_sampler_bit_exact_vs_reference(sampler_kat):
         assert np.array_equal(o["omegas"], sampler_kat["omegas"][k]), k
 
 
-@pytest.mark.skipif(not c_oracle.have_ref_sampler(), reason="oracle/_ref not built (no /root/reference here)")
-def test_compiled_reference_sampler_matches_vectors(sampler_kat):
-    a, e = sampler_kat["a"], sampler_kat["e"]
-    for k in range(len(a)):
-        et, om = c_oracle.ref_sample_on_batch(a[k].reshape(1, 1, 3), e[k].reshape(1, 1, 2))
-        assert np.array_equal(et.ravel(), sampler_kat["etas"][k]) and np.array_equal(om.ravel(), sampler_kat["omegas"][k])
-
-
 def test_sampler_edge_semantics():
     """cos(float(pi)/2) < 0 makes the last CDF increment negative for small exponents (SURVEY H3); the centre of each
     grid is exactly 0; both grids are strictly decreasing in angle."""

@@ -3,7 +3,6 @@ precision, and that rounding to float gives the correctly rounded result on the 
 import ctypes as C
 import os
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -12,8 +11,8 @@ REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
-def m():
-    so = os.path.join(tempfile.gettempdir(), "libsq_math_host_test.so")
+def m(tmp_path_factory):
+    so = str(tmp_path_factory.mktemp("sq_math") / "libsq_math_host_test.so")
     subprocess.run(["g++", "-O2", "-ffp-contract=off", "-fPIC", "-shared", "-std=c++17", "-o", so,
                     os.path.join(REPO, "odam_b200", "csrc", "sq_math_host.cpp"), "-lm"], check=True)
     return C.CDLL(so)
