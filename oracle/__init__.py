@@ -10,5 +10,6 @@ Contents
 sq_oracle.c          plain-C fp32 restatement (sampler + forward + analytic backward + Adam)
 c_oracle.py          ctypes binding of the above (+ of oracle/_ref/libref_sampler.so)
 torch_oracle.py      op-for-op PyTorch/autograd restatement of sq_libs.py's run loop
+grad64.py            float64 restatement of one step's gradient with its discrete decisions held fixed
 Makefile             builds _build/*.so and, when /root/reference is present, _ref/
 """

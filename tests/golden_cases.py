@@ -134,3 +134,28 @@ def teacher_forced_report(api, cases, label, **kw):
           f"discrete decision differing from the reference {disagree}; violations on decision-agreeing steps "
           f"{viol_on_agree}; worst in-tolerance rel err params {worst_p:.2e}, loss {worst_l:.2e}")
     return dict(total=total, viol_p=viol_p, viol_l=viol_l, disagree=disagree, viol_on_agree=viol_on_agree)
+
+
+def edge_object(kind, seed=31):
+    """One synthetic object (views, init) with an edge of the backward pass forced: extreme shape exponents
+    (h = +-6 puts e at 1.6 and 0.2, where samples sit in the 1e-6 clamp), yaws on the axes, a view behind the camera,
+    an all-masked track, a single view."""
+    from odam_b200 import synthetic
+    from odam_b200.api import init_params
+    V = 1 if kind == "V1" else 12
+    sc = synthetic.make_scene(1, V, seed=seed)
+    init = init_params(sc.translate[0], sc.angle[0], sc.dims[0])
+    Ms = sc.P_cws[0].reshape(V, 12).astype(np.float32)
+    box, mask = sc.box[0].astype(np.float32), sc.mask[0].copy()
+    if kind.startswith("h"):
+        init[7:9] = {"h+6": (6, 6), "h-6": (-6, -6), "h+-6": (6, -6)}[kind]
+    if kind.startswith("yaw"):
+        init[3] = {"yaw0": 0.0, "yaw+pi/2": np.pi / 2, "yaw-pi/2": -np.pi / 2, "yawpi": np.pi}[kind]
+    if kind == "behind":
+        Ms[0, 8:12] = -Ms[0, 8:12]
+    if kind == "masked":
+        mask[:] = 0
+    return init, Ms, box, mask, int(sc.cls[0])
+
+
+EDGE_KINDS = ["plain", "h+6", "h-6", "h+-6", "yaw0", "yaw+pi/2", "yaw-pi/2", "yawpi", "behind", "masked", "V1"]
