@@ -136,6 +136,25 @@ int odam_sq_project_boxes(const float *params, const int32_t *view_off, const fl
 int odam_sq_project_boxes_host(const float *params, const int32_t *view_off, const float *Ms, int n,
                                float *out_box, int device);
 
+/* Differentiable ops (odam_b200/autograd.py): forward and vector-Jacobian products of the surface samples and of the
+ * projected box sides, so that the optimiser's maths can be composed with other loss terms, optimisers or schedules.
+ * Device pointers only.  Each kernel re-runs the sampler from params (nothing is saved between forward and backward);
+ * every reduction has a fixed order, so results do not depend on the batch an object is launched in.  Each object's
+ * views [view_off[i], view_off[i+1]) are clamped to [0, total_views] on the device.  The camera matrices are constants:
+ * there is no gradient with respect to Ms.
+ *
+ * odam_sq_sample_points_vjp: grad_xyz[n][1000][3] (dL/d of odam_sq_sample_points' output) -> out_grad_params[n][9].
+ * odam_sq_box_sides: constraint_2d (sq_libs.py:397-413) for every (object, view): out_pred[SV][4] = x_min, x_max, y_min,
+ *   y_max over the samples of valid ? q / (|q_z| + 1e-6) : +-1e6 with valid = q_z > 0.5 (first index on ties, NaN
+ *   propagates as in torch.min/max); out_arg[SV][4] = the winning sample, -1 when a sentinel won.
+ * odam_sq_box_sides_vjp: grad_pred[SV][4] and the arg of odam_sq_box_sides -> out_grad_params[n][9]; sides with
+ *   arg < 0 contribute nothing. */
+int odam_sq_sample_points_vjp(const float *params, const float *grad_xyz, int n, float *out_grad_params, void *stream);
+int odam_sq_box_sides(const float *params, const int32_t *view_off, const float *Ms, int n, int total_views,
+                      float *out_pred, int32_t *out_arg, void *stream);
+int odam_sq_box_sides_vjp(const float *params, const int32_t *view_off, const float *Ms, const int32_t *arg,
+                          const float *grad_pred, int n, int total_views, float *out_grad_params, void *stream);
+
 /* compute_ellipsoid_points + compute_oriented_bbox (src/scripts/run_multi_view.py:66-67, src/utils/box_utils.py:319-410):
  * params[n][9] -> out_corners[n][8][3] DOUBLE, the oriented box of each object's 1000 surface points: min-area rectangle
  * of the xy convex hull over the directions of the hull edges, upper four corners (z_max) first, then the same four at

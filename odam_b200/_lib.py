@@ -18,7 +18,8 @@ EXPORTS = ("odam_sq_abi_version", "odam_sq_error_string", "odam_sq_last_cuda_err
            "odam_sq_project_boxes", "odam_sq_project_boxes_host", "odam_sq_query_launch",
            "odam_sq_sample_on_batch_host", "odam_sq_fma_peak", "odam_sq_selftest", "odam_sq_oriented_boxes",
            "odam_sq_oriented_boxes_host", "odam_sq_oriented_boxes_of_points_host", "odam_sq_merge_cost_host",
-           "odam_sq_cluster_capacity", "odam_sq_stage_tracks_host")
+           "odam_sq_cluster_capacity", "odam_sq_stage_tracks_host", "odam_sq_sample_points_vjp", "odam_sq_box_sides",
+           "odam_sq_box_sides_vjp")
 
 
 class Options(C.Structure):
@@ -69,6 +70,9 @@ def load():
         L.odam_sq_query_launch.argtypes = [vp, ci, C.POINTER(Options)] + [C.POINTER(ci)] * 6
         L.odam_sq_cluster_capacity.argtypes = [ci, ci, C.POINTER(ci)]
         L.odam_sq_stage_tracks_host.argtypes = [vp, vp, ci, ci, vp, ci, ci, ci] + [vp] * 9
+        L.odam_sq_sample_points_vjp.argtypes = [vp, vp, ci, vp, vp]
+        L.odam_sq_box_sides.argtypes = [vp, vp, vp, ci, ci, vp, vp, vp]
+        L.odam_sq_box_sides_vjp.argtypes = [vp, vp, vp, vp, vp, ci, ci, vp, vp]
         for f in EXPORTS:
             if getattr(L, f).restype is None:
                 pass

@@ -11,7 +11,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = [os.path.join(HERE, "csrc", "sq_kernels.cu")]
-DEPS = SRC + [os.path.join(HERE, "csrc", "sq_device.cuh"), os.path.join(HERE, "csrc", "sq_math.cuh"), os.path.join(HERE, "csrc", "sq_glibc_data.h"), os.path.join(HERE, "csrc", "sq_postproc.cuh"), os.path.join(HERE, "csrc", "sq_stage.h"), os.path.join(HERE, "..", "include", "odam_sq.h")]
+DEPS = SRC + [os.path.join(HERE, "csrc", "sq_device.cuh"), os.path.join(HERE, "csrc", "sq_math.cuh"), os.path.join(HERE, "csrc", "sq_glibc_data.h"), os.path.join(HERE, "csrc", "sq_postproc.cuh"), os.path.join(HERE, "csrc", "sq_stage.h"), os.path.join(HERE, "csrc", "sq_autograd.cuh"), os.path.join(HERE, "..", "include", "odam_sq.h")]
 OUT = os.path.join(HERE, "lib", "libodam_sq.so")
 # -regUsageLevel=10: ptxas trades registers for better code more aggressively (default 5); inside the same launch
 # bounds it is worth +0.4..1.6 % on the dense configs (profiles/r02_ptxas_regusage.txt), nothing changes numerically

@@ -501,7 +501,9 @@ __global__ void __launch_bounds__(kMaxThreads, SQ_MIN_BLOCKS(kMaxThreads, kCompa
             }
             if (arg < 0 && mk != 0.f) atomicOr(&S.status, ODAM_SQ_ST_NO_VALID_PT);
             if (arg < 0 || mk == 0.f || !(diff == diff)) continue;
-            // gradient through the arg-extreme point
+            // gradient through the arg-extreme point.  point_vjp (sq_autograd.cuh) holds the same chain rule for the
+            // differentiable ops; this copy stays inline on purpose: phase F is register-capped tuned code, and moving
+            // it onto the shared helper would need its own A/B timing.
             float c = __fmul_rn(__fmul_rn(sgnf(diff), mk), invV);
             float g_lin = __fdiv_rn(c, d);                                        // d(u)/d(q_x or q_y)
             float g_z = -__fmul_rn(__fdiv_rn(__fmul_rn(c, num), __fmul_rn(d, d)), sgnf(qz));  // d(u)/d(q_z)
@@ -681,6 +683,8 @@ __global__ void __launch_bounds__(256) sq_points_kernel(const float *params, int
         o[0] = S.px[i]; o[1] = S.py[i]; o[2] = S.pz[i];
     }
 }
+
+#include "sq_autograd.cuh"
 
 // The reference's own native entry point (sampling.hpp:5-15 sample_on_batch, B*M primitives, N=1000,
 // buffer_size=201, seed=0): a[n][3], e[n][2] -> etas[n][1000], omegas[n][1000].  One CTA (2 warps) per primitive.
@@ -1022,6 +1026,9 @@ static int ensure_init(int device)
     CU(cudaFuncSetAttribute(sq_boxes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
     CU(cudaFuncSetAttribute(sq_angles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
     CU(cudaFuncSetAttribute(sq_obb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
+    CU(cudaFuncSetAttribute(sq_points_vjp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
+    CU(cudaFuncSetAttribute(sq_sides_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSidesSmem));
+    CU(cudaFuncSetAttribute(sq_sides_vjp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
     CU(cudaStreamCreateWithFlags(&D.stream, cudaStreamNonBlocking));
     D.ready = true;
     return ODAM_SQ_OK;
@@ -1343,6 +1350,52 @@ int odam_sq_project_boxes(const float *params, const int32_t *view_off, const fl
     int rc = ensure_init(device);
     if (rc) return rc;
     sq_boxes_kernel<<<n, 256, kFwdSmem, (cudaStream_t)stream>>>(params, view_off, Ms, n, out_box);
+    CU(cudaGetLastError());
+    return ODAM_SQ_OK;
+}
+
+// ---- differentiable ops (sq_autograd.cuh): device pointers, enqueued on `stream` ----
+
+int odam_sq_sample_points_vjp(const float *params, const float *grad_xyz, int n, float *out_grad_params, void *stream)
+{
+    if (!params || !grad_xyz || !out_grad_params || n < 0) return ODAM_SQ_ERR_ARG;
+    if (n == 0) return ODAM_SQ_OK;
+    int device = 0;
+    CU(cudaGetDevice(&device));
+    int rc = ensure_init(device);
+    if (rc) return rc;
+    sq_points_vjp_kernel<<<n, kAgThreads, kFwdSmem, (cudaStream_t)stream>>>(params, grad_xyz, n, out_grad_params);
+    CU(cudaGetLastError());
+    return ODAM_SQ_OK;
+}
+
+int odam_sq_box_sides(const float *params, const int32_t *view_off, const float *Ms, int n, int total_views,
+                      float *out_pred, int32_t *out_arg, void *stream)
+{
+    if (!params || !view_off || !Ms || !out_pred || !out_arg || n < 0 || total_views < 0) return ODAM_SQ_ERR_ARG;
+    if (n == 0) return ODAM_SQ_OK;
+    int device = 0;
+    CU(cudaGetDevice(&device));
+    int rc = ensure_init(device);
+    if (rc) return rc;
+    sq_sides_kernel<<<n, kAgThreads, kSidesSmem, (cudaStream_t)stream>>>(params, view_off, Ms, n, total_views, out_pred,
+                                                                          out_arg);
+    CU(cudaGetLastError());
+    return ODAM_SQ_OK;
+}
+
+int odam_sq_box_sides_vjp(const float *params, const int32_t *view_off, const float *Ms, const int32_t *arg,
+                          const float *grad_pred, int n, int total_views, float *out_grad_params, void *stream)
+{
+    if (!params || !view_off || !Ms || !arg || !grad_pred || !out_grad_params || n < 0 || total_views < 0)
+        return ODAM_SQ_ERR_ARG;
+    if (n == 0) return ODAM_SQ_OK;
+    int device = 0;
+    CU(cudaGetDevice(&device));
+    int rc = ensure_init(device);
+    if (rc) return rc;
+    sq_sides_vjp_kernel<<<n, kAgThreads, kFwdSmem, (cudaStream_t)stream>>>(params, view_off, Ms, arg, grad_pred, n,
+                                                                            total_views, out_grad_params);
     CU(cudaGetLastError());
     return ODAM_SQ_OK;
 }
