@@ -73,10 +73,9 @@ def load():
         L.odam_sq_sample_points_vjp.argtypes = [vp, vp, ci, vp, vp]
         L.odam_sq_box_sides.argtypes = [vp, vp, vp, ci, ci, vp, vp, vp]
         L.odam_sq_box_sides_vjp.argtypes = [vp, vp, vp, vp, vp, ci, ci, vp, vp]
-        for f in EXPORTS:
-            if getattr(L, f).restype is None:
-                pass
-            getattr(L, f)
+        missing = [f for f in EXPORTS if not hasattr(L, f)]
+        if missing:
+            raise OdamSqError(f"{LIB_PATH} does not export {', '.join(missing)}")
         _lib = L
     return _lib
 

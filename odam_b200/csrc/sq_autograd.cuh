@@ -1,11 +1,10 @@
 // sq_autograd.cuh -- forward and backward kernels of the differentiable ops (odam_b200/autograd.py; C ABI
 // odam_sq_sample_points_vjp, odam_sq_box_sides, odam_sq_box_sides_vjp).  Included by sq_kernels.cu inside namespace odam,
-// after Smem, derive_param and sample_surface.
+// after Smem and sample_object.
 //
-// Every kernel runs one CTA of kAgThreads threads per object and starts like sq_points_kernel: the sampler runs from
-// the parameters, which leaves the points, the eta bucket of every sample (S.pj), both grids and the pose in shared
-// memory.  Backward kernels recompute the sampler instead of saving anything from the forward pass: it is
-// deterministic, so both passes see the same samples.
+// Every kernel runs one CTA of kAgThreads threads per object and starts with sample_object, like sq_points_kernel.
+// Backward kernels recompute the sampler instead of saving anything from the forward pass: it is deterministic, so
+// both passes see the same samples.
 //
 // Reductions are deterministic: each thread's items follow a fixed stride, then a warp butterfly, then a fixed warp
 // order.  An object's gradient is therefore the same bits from run to run and whether it is launched alone or in a
@@ -20,8 +19,8 @@ static_assert(kSidesSmem >= kSpecBytes, "the sampler's scratch must fit the dyna
 
 // Chain rule of one surface sample: d(point)/d(params) applied to the upstream gradient gp = dL/d(world point), added
 // into acc[9] (sq_libs.py:577-595 + sampling.py:598-615).  The same arithmetic as phase F of sq_optimize_kernel, which
-// keeps its own copy: phase F is register-capped tuned code, and moving it onto this helper would need its own A/B
-// timing.  Unlike phase F the shape gradient is always formed (at h = -10000 the sigmoid factor makes it 0 by itself),
+// keeps its own copy: phase F is register-capped tuned code, and on this helper it measured 0.2 % slower (config 2,
+// B200 at 1000 W).  Unlike phase F the shape gradient is always formed (at h = -10000 the sigmoid factor makes it 0 by itself),
 // and NaN or Inf in gp propagates.
 __device__ __forceinline__ void point_vjp(const Smem &S, const Pose &P, int j, int k, float gp0, float gp1, float gp2,
                                           float (&acc)[9])
@@ -46,22 +45,6 @@ __device__ __forceinline__ void point_vjp(const Smem &S, const Pose &P, int j, i
     const float ge2 = gl0 * x0 * lco + gl1 * y0 * lso;
     acc[7] += ge1 * 1.4f * P.sig[0] * (1.f - P.sig[0]);
     acc[8] += ge2 * 1.4f * P.sig[1] * (1.f - P.sig[1]);
-}
-
-// parameters -> sampler state in shared memory (the common start of every kernel here)
-__device__ __forceinline__ void ag_sample(Smem &S, const float *params, int obj, unsigned char *scratch)
-{
-    const int tid = threadIdx.x;
-    if (tid < 9) S.par[tid] = params[(size_t)obj * 9 + tid];
-    if (tid == 0) {
-        const float pi = 3.14159274101257324f, pi_2 = __fmul_rn(pi, 0.5f);
-        pool_init(S.ge, pi_2, -pi_2);
-        pool_init(S.go, pi, -pi);
-    }
-    __syncthreads();
-    if (tid < 10) derive_param(S, tid);
-    __syncthreads();
-    sample_surface<true>(S, reinterpret_cast<GridSpec *>(scratch), tid, blockDim.x, false);
 }
 
 // acc[9] of every thread -> out[9]: warp butterfly, then the warps in order.  red: 9 floats per warp.
@@ -98,7 +81,7 @@ __global__ void __launch_bounds__(kAgThreads) sq_points_vjp_kernel(const float *
     __shared__ float red[kAgThreads / 32][9];
     extern __shared__ __align__(16) unsigned char scratch_raw[];
     const int obj = blockIdx.x, tid = threadIdx.x;
-    ag_sample(S, params, obj, scratch_raw);
+    sample_object(S, params, obj, scratch_raw);
     float acc[9];
 #pragma unroll
     for (int k = 0; k < 9; k++) acc[k] = 0.f;
@@ -142,7 +125,7 @@ __global__ void __launch_bounds__(kAgThreads) sq_sides_kernel(const float *param
     __shared__ Smem S;
     extern __shared__ __align__(16) unsigned char scratch_raw[];
     const int obj = blockIdx.x, tid = threadIdx.x, T = blockDim.x;
-    ag_sample(S, params, obj, scratch_raw);
+    sample_object(S, params, obj, scratch_raw);
     int v_begin, V;
     ag_views(view_off, obj, total_views, v_begin, V);
     float(*val)[4] = reinterpret_cast<float(*)[4]>(scratch_raw);                  // [T][4]
@@ -206,7 +189,7 @@ __global__ void __launch_bounds__(kAgThreads) sq_sides_vjp_kernel(const float *p
     __shared__ float red[kAgThreads / 32][9];
     extern __shared__ __align__(16) unsigned char scratch_raw[];
     const int obj = blockIdx.x, tid = threadIdx.x;
-    ag_sample(S, params, obj, scratch_raw);
+    sample_object(S, params, obj, scratch_raw);
     int v_begin, V;
     ag_views(view_off, obj, total_views, v_begin, V);
     float acc[9];
