@@ -19,7 +19,7 @@ EXPORTS = ("odam_sq_abi_version", "odam_sq_error_string", "odam_sq_last_cuda_err
            "odam_sq_sample_on_batch_host", "odam_sq_fma_peak", "odam_sq_selftest", "odam_sq_oriented_boxes",
            "odam_sq_oriented_boxes_host", "odam_sq_oriented_boxes_of_points_host", "odam_sq_merge_cost_host",
            "odam_sq_cluster_capacity", "odam_sq_stage_tracks_host", "odam_sq_sample_points_vjp", "odam_sq_box_sides",
-           "odam_sq_box_sides_vjp")
+           "odam_sq_box_sides_vjp", "odam_sq_box_sides_vjp_cameras")
 
 
 class Options(C.Structure):
@@ -73,6 +73,7 @@ def load():
         L.odam_sq_sample_points_vjp.argtypes = [vp, vp, ci, vp, vp]
         L.odam_sq_box_sides.argtypes = [vp, vp, vp, ci, ci, vp, vp, vp]
         L.odam_sq_box_sides_vjp.argtypes = [vp, vp, vp, vp, vp, ci, ci, vp, vp]
+        L.odam_sq_box_sides_vjp_cameras.argtypes = [vp, vp, vp, vp, vp, ci, ci, vp, vp, vp]
         missing = [f for f in EXPORTS if not hasattr(L, f)]
         if missing:
             raise OdamSqError(f"{LIB_PATH} does not export {', '.join(missing)}")

@@ -5,9 +5,10 @@ pieces of that loss so that callers can build their own: add loss terms, use ano
 schedule, or backpropagate into parameters produced by other modules.
 
   surface_points(params)                  -> [n, 1000, 3]   compute_ellipsoid_points (sq_libs.py:577-595)
-  box_sides(params, view_off, Ms)         -> (pred [SV, 4], arg [SV, 4] int32)
+  box_sides(params, view_off, Ms, camera_grad=False)
+                                          -> (pred [SV, 4], arg [SV, 4] int32)
                                              the projected box sides of constraint_2d (sq_libs.py:397-413)
-  box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None) -> [n]
+  box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None, camera_grad=False) -> [n]
                                              the optimiser's per-object loss (sq_libs.py:420-430 + :463-466)
 
 params is a float32 CUDA tensor [n, 9]: translation x, y, z | yaw | scales s1, s2, s3 | shape logits h1, h2, the layout of
@@ -19,7 +20,14 @@ Forward and backward passes are CUDA kernels (csrc/sq_autograd.cuh) enqueued on 
 Backward passes recompute the surface samples from params; gradients are deterministic, bit for bit, and independent of
 the batch an object is evaluated in.  The sampler's discrete choices (which surface angles are sampled) and the
 arg-extreme sample of every side are piecewise constant in params and carry no gradient, exactly as in the reference.
-Ms is a constant: its gradient is None.  Double backward is not supported.
+Double backward is not supported.
+
+By default Ms is a constant: it is detached and its gradient stays None.  With camera_grad=True box_sides and box_loss
+also return dL/dMs, through the caller's reshape of Ms, from the same backward kernel (its second pass, one thread per
+view): joint object and camera refinement.  Rows of Ms that no object owns get 0.  Cameras shared by several objects are
+gathered per frame, Ms = P[frame_idx] (run_multi_view.stage_tracks returns frame_idx); torch's backward of that gather
+sums with atomics and is bit-reproducible only under torch.use_deterministic_algorithms(True).  dL/dMs itself is
+deterministic either way.
 """
 import ctypes as C
 
@@ -79,7 +87,7 @@ def _views(params, view_off, Ms):
         _check_cuda("view_off", view_off, params.device)
     if SV >= 2 ** 31 // 4:
         raise ValueError("too many views for int32 indexing")
-    return Ms.detach().contiguous(), view_off.to(params.device).contiguous()
+    return Ms.contiguous(), view_off.to(params.device).contiguous()
 
 
 class _SurfacePoints(torch.autograd.Function):
@@ -128,14 +136,22 @@ class _BoxSides(torch.autograd.Function):
     def backward(ctx, grad_pred, _grad_arg):
         params, view_off, Ms, arg = ctx.saved_tensors
         n, SV = params.shape[0], Ms.shape[0]
-        grad = torch.zeros_like(params)
+        cams = ctx.needs_input_grad[2]   # Ms is attached only with camera_grad=True
+        # camera-only refinement (params frozen) passes NULL: the kernel then skips the params pass
+        grad = torch.zeros_like(params) if ctx.needs_input_grad[0] or not cams else None
+        grad_Ms = torch.zeros((SV, 12), dtype=torch.float32, device=params.device) if cams else None
         if n and SV and grad_pred is not None:
             g = grad_pred.to(torch.float32).contiguous()
             L = _lib.load()
             with torch.cuda.device(params.device):
-                _lib.check(L.odam_sq_box_sides_vjp(_p(params), _p(view_off), _p(Ms), _p(arg), _p(g), n, SV, _p(grad),
-                                                   _stream(params.device)))
-        return grad, None, None
+                if cams:
+                    _lib.check(L.odam_sq_box_sides_vjp_cameras(_p(params), _p(view_off), _p(Ms), _p(arg), _p(g), n, SV,
+                                                               None if grad is None else _p(grad), _p(grad_Ms),
+                                                               _stream(params.device)))
+                else:
+                    _lib.check(L.odam_sq_box_sides_vjp(_p(params), _p(view_off), _p(Ms), _p(arg), _p(g), n, SV,
+                                                       _p(grad), _stream(params.device)))
+        return grad, None, grad_Ms
 
 
 def surface_points(params):
@@ -146,15 +162,16 @@ def surface_points(params):
     return _SurfacePoints.apply(params.contiguous())
 
 
-def box_sides(params, view_off, Ms):
+def box_sides(params, view_off, Ms, camera_grad=False):
     """Projected box sides of every (object, view): pred [SV, 4] (x_min, x_max, y_min, y_max), differentiable with
     respect to params, and arg [SV, 4] int32, the sample that attains each side (-1 where no sample is in front of the
-    camera, z > 0.5, and pred holds the reference's +-1e6 sentinel).  Ms gets no gradient."""
+    camera, z > 0.5, and pred holds the reference's +-1e6 sentinel).  Ms gets no gradient unless camera_grad is True;
+    then pred is differentiable with respect to Ms too (sides with arg -1 contribute nothing)."""
     Ms12, voff = _views(params, view_off, Ms)
-    return _BoxSides.apply(params.contiguous(), voff, Ms12)
+    return _BoxSides.apply(params.contiguous(), voff, Ms12 if camera_grad else Ms12.detach())
 
 
-def box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None):
+def box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None, camera_grad=False):
     """The optimiser's loss per object, [n] float32: the sum over the four sides of the mean over all V views of the
     object of mask * |pred - box| (NaN terms count 0), plus 20 (s0 - s)^T A (s0 - s) with A = prior[cls] when a prior
     table is given.
@@ -162,8 +179,8 @@ def box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None):
     box [SV, 4] float32 detected sides (x_min, x_max, y_min, y_max), mask [SV, 4] (nonzero = side present), prior
     [8, 9] float32 per-class matrices (api.prior_table()), cls [n] class ids 0..7, s0 [n, 3] the anchor scales (the
     reference takes the scales at the start of its run).  The sum of this loss over objects, backpropagated, gives the
-    fused optimiser's gradient."""
-    pred, _ = box_sides(params, view_off, Ms)
+    fused optimiser's gradient.  camera_grad=True also backpropagates into Ms (box_sides)."""
+    pred, _ = box_sides(params, view_off, Ms, camera_grad)
     n, SV, dev = params.shape[0], pred.shape[0], params.device
     for name, t in (("box", box), ("mask", mask)):
         if not isinstance(t, torch.Tensor) or tuple(t.shape) != (SV, 4):

@@ -1,6 +1,6 @@
 // sq_autograd.cuh -- forward and backward kernels of the differentiable ops (odam_b200/autograd.py; C ABI
-// odam_sq_sample_points_vjp, odam_sq_box_sides, odam_sq_box_sides_vjp).  Included by sq_kernels.cu inside namespace odam,
-// after Smem and sample_object.
+// odam_sq_sample_points_vjp, odam_sq_box_sides, odam_sq_box_sides_vjp, odam_sq_box_sides_vjp_cameras).  Included by
+// sq_kernels.cu inside namespace odam, after Smem and sample_object.
 //
 // Every kernel runs one CTA of kAgThreads threads per object and starts with sample_object, like sq_points_kernel.
 // Backward kernels recompute the sampler instead of saving anything from the forward pass: it is deterministic, so
@@ -178,12 +178,29 @@ __global__ void __launch_bounds__(kAgThreads) sq_sides_kernel(const float *param
     }
 }
 
+// d pred / d q and d pred / d q_z of one side, scaled by its upstream gradient c = grad_pred[o]: pred = q / d with
+// d = |q_z| + 1e-6, g_lin = c / d, g_z = -c q sign(q_z) / d^2.  Both passes of sq_sides_vjp_kernel form them here, so
+// the camera gradient uses the same scalars as the parameter gradient.
+__device__ __forceinline__ void side_scalars(float num, float qz, const float *grad_pred, size_t o, float &g_lin,
+                                             float &g_z)
+{
+    const float d = __fadd_rn(fabsf(qz), 1e-6f);
+    const float c = grad_pred[o];
+    g_lin = __fdiv_rn(c, d);
+    g_z = -__fmul_rn(__fdiv_rn(__fmul_rn(c, num), __fmul_rn(d, d)), sgnf(qz));
+}
+
 // vector-Jacobian product of sq_sides_kernel: one item per (view, side) with arg >= 0, through the arg sample.
-// pred = q / d with d = |q_z| + 1e-6: d pred / d q = 1 / d, d pred / d q_z = -q sign(q_z) / d^2, then the camera
-// rows M[:, :3]^T and the per-sample chain of point_vjp.  Ms is a constant.
+// side_scalars, then the camera rows M[:, :3]^T and the per-sample chain of point_vjp.
+// kCams = false: Ms is a constant and out_grad is required (odam_sq_box_sides_vjp).
+// kCams = true (odam_sq_box_sides_vjp_cameras): out_grad may be NULL (the params pass is skipped); then one thread per
+// view writes out_grad_Ms[gv][12] = sum over the live sides s, in the order x_min, x_max, y_min, y_max, of
+// g_lin ph into row s >> 1 and g_z ph into row 2, ph = [X, Y, Z, 1] the arg sample.  No atomics: every row has one
+// writer and a fixed order.  Rows outside every object's clamped view range are not written.
+template <bool kCams>
 __global__ void __launch_bounds__(kAgThreads) sq_sides_vjp_kernel(const float *params, const int32_t *view_off,
                                                                   const float *Ms, const int32_t *arg, const float *grad_pred,
-                                                                  int n, int total_views, float *out_grad)
+                                                                  int n, int total_views, float *out_grad, float *out_grad_Ms)
 {
     __shared__ Smem S;
     __shared__ float red[kAgThreads / 32][9];
@@ -192,31 +209,57 @@ __global__ void __launch_bounds__(kAgThreads) sq_sides_vjp_kernel(const float *p
     sample_object(S, params, obj, scratch_raw);
     int v_begin, V;
     ag_views(view_off, obj, total_views, v_begin, V);
-    float acc[9];
+    if (!kCams || out_grad) {
+        float acc[9];
 #pragma unroll
-    for (int k = 0; k < 9; k++) acc[k] = 0.f;
-    const Pose P = S.pose;
-    for (int pr = tid; pr < 4 * V; pr += blockDim.x) {
-        const size_t o = (size_t)v_begin * 4 + pr;
-        const int a = arg[o];
-        if (a < 0 || a >= kN) continue;   // a sentinel won: the side does not depend on the parameters
-        const int gv = v_begin + (pr >> 2), s = pr & 3;
-        float Mr[4], Mz[4];
+        for (int k = 0; k < 9; k++) acc[k] = 0.f;
+        const Pose P = S.pose;
+        for (int pr = tid; pr < 4 * V; pr += blockDim.x) {
+            const size_t o = (size_t)v_begin * 4 + pr;
+            const int a = arg[o];
+            if (a < 0 || a >= kN) continue;   // a sentinel won: the side does not depend on the parameters
+            const int gv = v_begin + (pr >> 2), s = pr & 3;
+            float Mr[4], Mz[4];
 #pragma unroll
-        for (int k = 0; k < 4; k++) {
-            Mr[k] = __ldg(Ms + (size_t)gv * 12 + 4 * (s >> 1) + k);
-            Mz[k] = __ldg(Ms + (size_t)gv * 12 + 8 + k);
+            for (int k = 0; k < 4; k++) {
+                Mr[k] = __ldg(Ms + (size_t)gv * 12 + 4 * (s >> 1) + k);
+                Mz[k] = __ldg(Ms + (size_t)gv * 12 + 8 + k);
+            }
+            const float X = S.px[a], Y = S.py[a], Z = S.pz[a];
+            float g_lin, g_z;
+            side_scalars(ag_row(Mr, X, Y, Z), ag_row(Mz, X, Y, Z), grad_pred, o, g_lin, g_z);
+            const float gp0 = __fmaf_rn(Mz[0], g_z, __fmul_rn(Mr[0], g_lin));
+            const float gp1 = __fmaf_rn(Mz[1], g_z, __fmul_rn(Mr[1], g_lin));
+            const float gp2 = __fmaf_rn(Mz[2], g_z, __fmul_rn(Mr[2], g_lin));
+            point_vjp(S, P, S.pj[a], g_k_omega[a], gp0, gp1, gp2, acc);
         }
-        const float X = S.px[a], Y = S.py[a], Z = S.pz[a];
-        const float num = ag_row(Mr, X, Y, Z), qz = ag_row(Mz, X, Y, Z);
-        const float d = __fadd_rn(fabsf(qz), 1e-6f);
-        const float c = grad_pred[o];
-        const float g_lin = __fdiv_rn(c, d);
-        const float g_z = -__fmul_rn(__fdiv_rn(__fmul_rn(c, num), __fmul_rn(d, d)), sgnf(qz));
-        const float gp0 = __fmaf_rn(Mz[0], g_z, __fmul_rn(Mr[0], g_lin));
-        const float gp1 = __fmaf_rn(Mz[1], g_z, __fmul_rn(Mr[1], g_lin));
-        const float gp2 = __fmaf_rn(Mz[2], g_z, __fmul_rn(Mr[2], g_lin));
-        point_vjp(S, P, S.pj[a], g_k_omega[a], gp0, gp1, gp2, acc);
+        ag_reduce9(acc, red, out_grad + (size_t)obj * 9);
     }
-    ag_reduce9(acc, red, out_grad + (size_t)obj * 9);
+    if (kCams) {
+        for (int v = tid; v < V; v += blockDim.x) {
+            const int gv = v_begin + v;
+            float M[12], g[12];
+            ag_load_M(Ms, gv, M);
+#pragma unroll
+            for (int k = 0; k < 12; k++) g[k] = 0.f;
+#pragma unroll
+            for (int s = 0; s < 4; s++) {
+                const size_t o = (size_t)gv * 4 + s;
+                const int a = arg[o];
+                if (a < 0 || a >= kN) continue;
+                const float ph[4] = {S.px[a], S.py[a], S.pz[a], 1.f};
+                const int r = s >> 1;
+                float g_lin, g_z;
+                side_scalars(ag_row(M + 4 * r, ph[0], ph[1], ph[2]), ag_row(M + 8, ph[0], ph[1], ph[2]), grad_pred, o,
+                             g_lin, g_z);
+#pragma unroll
+                for (int k = 0; k < 4; k++) {
+                    g[4 * r + k] = __fadd_rn(g[4 * r + k], __fmul_rn(g_lin, ph[k]));
+                    g[8 + k] = __fadd_rn(g[8 + k], __fmul_rn(g_z, ph[k]));
+                }
+            }
+#pragma unroll
+            for (int k = 0; k < 12; k++) out_grad_Ms[(size_t)gv * 12 + k] = g[k];
+        }
+    }
 }

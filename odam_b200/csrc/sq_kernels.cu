@@ -1024,7 +1024,8 @@ static int ensure_init(int device)
     CU(cudaFuncSetAttribute(sq_obb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
     CU(cudaFuncSetAttribute(sq_points_vjp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
     CU(cudaFuncSetAttribute(sq_sides_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSidesSmem));
-    CU(cudaFuncSetAttribute(sq_sides_vjp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
+    CU(cudaFuncSetAttribute(sq_sides_vjp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
+    CU(cudaFuncSetAttribute(sq_sides_vjp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
     CU(cudaStreamCreateWithFlags(&D.stream, cudaStreamNonBlocking));
     D.ready = true;
     return ODAM_SQ_OK;
@@ -1464,8 +1465,23 @@ int odam_sq_box_sides_vjp(const float *params, const int32_t *view_off, const fl
     if (n == 0) return ODAM_SQ_OK;
     int device, rc = init_current_device(device);
     if (rc) return rc;
-    sq_sides_vjp_kernel<<<n, kAgThreads, kFwdSmem, (cudaStream_t)stream>>>(params, view_off, Ms, arg, grad_pred, n,
-                                                                            total_views, out_grad_params);
+    sq_sides_vjp_kernel<false><<<n, kAgThreads, kFwdSmem, (cudaStream_t)stream>>>(params, view_off, Ms, arg, grad_pred, n,
+                                                                                   total_views, out_grad_params, nullptr);
+    return check_launch();
+}
+
+int odam_sq_box_sides_vjp_cameras(const float *params, const int32_t *view_off, const float *Ms, const int32_t *arg,
+                                  const float *grad_pred, int n, int total_views, float *out_grad_params,
+                                  float *out_grad_Ms, void *stream)
+{
+    if (!params || !view_off || !Ms || !arg || !grad_pred || !out_grad_Ms || n < 0 || total_views < 0)
+        return ODAM_SQ_ERR_ARG;
+    if (n == 0) return ODAM_SQ_OK;
+    int device, rc = init_current_device(device);
+    if (rc) return rc;
+    sq_sides_vjp_kernel<true><<<n, kAgThreads, kFwdSmem, (cudaStream_t)stream>>>(params, view_off, Ms, arg, grad_pred, n,
+                                                                                  total_views, out_grad_params,
+                                                                                  out_grad_Ms);
     return check_launch();
 }
 

@@ -8,6 +8,7 @@ times, per call:
   points fwd+bwd    surface_points, then backward of a fixed upstream gradient
   sides fwd         box_sides(params, view_off, Ms)
   sides fwd+bwd     box_sides, then backward of a fixed upstream gradient of pred (the two kernels alone)
+  sides fwd+bwd, cameras   the same with camera_grad=True, backward into params and Ms (one launch for both)
   loss fwd+bwd      box_loss(...).sum().backward()               (box_sides and its VJP + the torch ops of the loss)
   fused 1 step      api.optimize_device(n_iters=1)               (the fused optimiser: sampler, sides, gradient, Adam)
 Every shape is warmed up first; each figure is the median over 5 timed windows of at least 100 ms.  The working sets
@@ -93,6 +94,12 @@ def main():
             params.grad = None
             torch.autograd.backward(AG.box_sides(params, voff, Ms)[0], Gs)
 
+        Ms_leaf = Ms.clone().requires_grad_(True)
+
+        def sides_fwd_bwd_cams():
+            params.grad = Ms_leaf.grad = None
+            torch.autograd.backward(AG.box_sides(params, voff, Ms_leaf, camera_grad=True)[0], Gs)
+
         def loss_fwd_bwd():
             params.grad = None
             AG.box_loss(params, voff, Ms, box, mask, **kw).sum().backward()
@@ -102,10 +109,11 @@ def main():
 
         print(f"config {idx}: {cfg['name']} ({tracks.n} objects, {tracks.total_views} views, prior {use_prior})")
         for name, fn in (("points fwd", points_fwd), ("points fwd+bwd", points_fwd_bwd), ("sides fwd", sides_fwd),
-                         ("sides fwd+bwd", sides_fwd_bwd), ("loss fwd+bwd", loss_fwd_bwd), ("fused 1 step", fused)):
+                         ("sides fwd+bwd", sides_fwd_bwd), ("sides fwd+bwd, cameras", sides_fwd_bwd_cams),
+                         ("loss fwd+bwd", loss_fwd_bwd), ("fused 1 step", fused)):
             ms, reps = per_call_ms(fn)
-            print(f"  {name:15s} {ms * 1e3:10.1f} us/call  ({reps} calls per window)")
-        del dt, params, G
+            print(f"  {name:22s} {ms * 1e3:10.1f} us/call  ({reps} calls per window)")
+        del dt, params, G, Ms_leaf
         torch.cuda.empty_cache()
 
 
