@@ -13,14 +13,6 @@ REPR = {"super_quadric": 0, "cube": 1, "quadric": 2}
 ST_NONFINITE, ST_SAMPLER, ST_NO_VALID_PT = 1, 2, 4
 N_SAMPLES, GRID = 1000, 201
 
-EXPORTS = ("odam_sq_abi_version", "odam_sq_error_string", "odam_sq_last_cuda_error", "odam_sq_init",
-           "odam_sq_optimize", "odam_sq_optimize_host", "odam_sq_sample_points", "odam_sq_sample_points_host",
-           "odam_sq_project_boxes", "odam_sq_project_boxes_host", "odam_sq_query_launch",
-           "odam_sq_sample_on_batch_host", "odam_sq_fma_peak", "odam_sq_selftest", "odam_sq_oriented_boxes",
-           "odam_sq_oriented_boxes_host", "odam_sq_oriented_boxes_of_points_host", "odam_sq_merge_cost_host",
-           "odam_sq_cluster_capacity", "odam_sq_stage_tracks_host", "odam_sq_sample_points_vjp", "odam_sq_box_sides",
-           "odam_sq_box_sides_vjp", "odam_sq_box_sides_vjp_cameras")
-
 
 class Options(C.Structure):
     """odam_sq_options (include/odam_sq.h)."""
@@ -37,6 +29,37 @@ class OdamSqError(RuntimeError):
     pass
 
 
+_vp, _ci, _cf = C.c_void_p, C.c_int, C.c_float
+_OPT = [_vp] * 7 + [_ci, _ci, _ci, _cf, _cf] + [_vp] * 3 + [C.POINTER(Options)]
+# every entry of include/odam_sq.h -> its argtypes
+ARGTYPES = {
+    "odam_sq_abi_version": [],
+    "odam_sq_error_string": [_ci],
+    "odam_sq_last_cuda_error": [],
+    "odam_sq_init": [_ci],
+    "odam_sq_optimize": _OPT + [_vp],
+    "odam_sq_optimize_host": _OPT + [_ci],
+    "odam_sq_sample_points": [_vp, _ci, _vp, _vp],
+    "odam_sq_sample_points_host": [_vp, _ci, _vp, _ci],
+    "odam_sq_project_boxes": [_vp, _vp, _vp, _ci, _vp, _vp],
+    "odam_sq_project_boxes_host": [_vp, _vp, _vp, _ci, _vp, _ci],
+    "odam_sq_query_launch": [_vp, _ci, C.POINTER(Options)] + [C.POINTER(_ci)] * 6,
+    "odam_sq_sample_on_batch_host": [_vp] * 4 + [_ci] * 6,
+    "odam_sq_fma_peak": [_ci, C.POINTER(C.c_double)],
+    "odam_sq_selftest": [_ci, C.c_uint32, C.c_longlong, C.POINTER(C.c_longlong)],
+    "odam_sq_oriented_boxes": [_vp, _ci, _vp, _vp, _vp, _vp],
+    "odam_sq_oriented_boxes_host": [_vp, _ci, _vp, _vp, _vp, _ci],
+    "odam_sq_oriented_boxes_of_points_host": [_vp, _ci, _ci, _vp, _vp, _ci],
+    "odam_sq_merge_cost_host": [_vp, _vp, _ci, _vp, _vp, _vp, _ci],
+    "odam_sq_cluster_capacity": [_ci, _ci, C.POINTER(_ci)],
+    "odam_sq_stage_tracks_host": [_vp, _vp, _ci, _ci, _vp, _ci, _ci, _ci] + [_vp] * 9,
+    "odam_sq_sample_points_vjp": [_vp, _vp, _ci, _vp, _vp],
+    "odam_sq_box_sides": [_vp, _vp, _vp, _ci, _ci, _vp, _vp, _vp],
+    "odam_sq_box_sides_vjp": [_vp, _vp, _vp, _vp, _vp, _ci, _ci, _vp, _vp],
+    "odam_sq_box_sides_vjp_cameras": [_vp, _vp, _vp, _vp, _vp, _ci, _ci, _vp, _vp, _vp],
+}
+EXPORTS = tuple(ARGTYPES)
+
 _lib = None
 
 
@@ -47,36 +70,13 @@ def load():
             raise OdamSqError(f"{LIB_PATH} is missing: build it with `python -m odam_b200.build` "
                               "(there is no CPU fallback)")
         L = C.CDLL(LIB_PATH)
-        vp, ci, cf = C.c_void_p, C.c_int, C.c_float
-        L.odam_sq_abi_version.restype = ci
-        L.odam_sq_error_string.restype = C.c_char_p
-        L.odam_sq_error_string.argtypes = [ci]
-        L.odam_sq_last_cuda_error.restype = C.c_char_p
-        L.odam_sq_init.argtypes = [ci]
-        opt_args = [vp] * 7 + [ci, ci, ci, cf, cf] + [vp] * 3 + [C.POINTER(Options)]
-        L.odam_sq_optimize.argtypes = opt_args + [vp]
-        L.odam_sq_optimize_host.argtypes = opt_args + [ci]
-        L.odam_sq_sample_points.argtypes = [vp, ci, vp, vp]
-        L.odam_sq_sample_points_host.argtypes = [vp, ci, vp, ci]
-        L.odam_sq_project_boxes.argtypes = [vp, vp, vp, ci, vp, vp]
-        L.odam_sq_project_boxes_host.argtypes = [vp, vp, vp, ci, vp, ci]
-        L.odam_sq_sample_on_batch_host.argtypes = [vp] * 4 + [ci] * 6
-        L.odam_sq_oriented_boxes.argtypes = [vp, ci, vp, vp, vp, vp]
-        L.odam_sq_oriented_boxes_host.argtypes = [vp, ci, vp, vp, vp, ci]
-        L.odam_sq_oriented_boxes_of_points_host.argtypes = [vp, ci, ci, vp, vp, ci]
-        L.odam_sq_merge_cost_host.argtypes = [vp, vp, ci, vp, vp, vp, ci]
-        L.odam_sq_fma_peak.argtypes = [ci, C.POINTER(C.c_double)]
-        L.odam_sq_selftest.argtypes = [ci, C.c_uint32, C.c_longlong, C.POINTER(C.c_longlong)]
-        L.odam_sq_query_launch.argtypes = [vp, ci, C.POINTER(Options)] + [C.POINTER(ci)] * 6
-        L.odam_sq_cluster_capacity.argtypes = [ci, ci, C.POINTER(ci)]
-        L.odam_sq_stage_tracks_host.argtypes = [vp, vp, ci, ci, vp, ci, ci, ci] + [vp] * 9
-        L.odam_sq_sample_points_vjp.argtypes = [vp, vp, ci, vp, vp]
-        L.odam_sq_box_sides.argtypes = [vp, vp, vp, ci, ci, vp, vp, vp]
-        L.odam_sq_box_sides_vjp.argtypes = [vp, vp, vp, vp, vp, ci, ci, vp, vp]
-        L.odam_sq_box_sides_vjp_cameras.argtypes = [vp, vp, vp, vp, vp, ci, ci, vp, vp, vp]
         missing = [f for f in EXPORTS if not hasattr(L, f)]
         if missing:
             raise OdamSqError(f"{LIB_PATH} does not export {', '.join(missing)}")
+        for name, argtypes in ARGTYPES.items():
+            getattr(L, name).argtypes = argtypes
+        L.odam_sq_error_string.restype = C.c_char_p
+        L.odam_sq_last_cuda_error.restype = C.c_char_p
         _lib = L
     return _lib
 

@@ -945,23 +945,90 @@ struct DeviceState {
 static DeviceState g_dev[64];
 static std::mutex g_mu;
 
+static void fill_adam_tab(std::vector<float> &tab, int n_iters, int step0, double lr, double lr_shape)
+{
+    tab.resize((size_t)n_iters * 4);
+    for (int it = 0; it < n_iters; it++) {
+        double step = (double)(step0 + it + 1);
+        double bc1 = 1.0 - pow(0.9, step), bc2 = 1.0 - pow(0.999, step);
+        tab[it * 4 + 0] = (float)(-(lr / bc1));
+        tab[it * 4 + 1] = (float)(-(lr_shape / bc1));
+        tab[it * 4 + 2] = (float)pow(bc2, 0.5);
+        tab[it * 4 + 3] = 0.f;
+    }
+}
+
+// Device copy of the Adam bias-correction table for a launch on `st` (host doubles, as torch computes them in Python
+// floats); one cached table per (stream, schedule), so launches on different streams never share -- or overwrite --
+// each other's table
+static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, float lr, float lr_shape,
+                      const float *&dev)
+{
+    std::lock_guard<std::mutex> lk(g_mu);
+    dev = nullptr;
+    for (const AdamTab &t : D.tabs)
+        if (t.stream == st && t.iters == n_iters && t.step0 == step0 && t.lr == (double)lr && t.lrs == (double)lr_shape)
+            dev = t.dev;
+    if (dev) return ODAM_SQ_OK;
+    AdamTab *slot = nullptr;
+    for (AdamTab &t : D.tabs)
+        if (t.stream == st) slot = &t;                    // this stream's previous schedule: reuse its buffer
+    if (!slot && D.tabs.size() >= 16) slot = &D.tabs[0];  // bounded cache: recycle the oldest entry
+    if (slot) {
+        CU(cudaStreamSynchronize(slot->stream));          // its last launch may still read the table
+        if (slot->cap < n_iters) { cudaFree(slot->dev); slot->dev = nullptr; slot->cap = 0; }
+    } else {
+        D.tabs.push_back(AdamTab{st, 0, 0, 0, 0, nullptr, 0});
+        slot = &D.tabs.back();
+    }
+    if (!slot->dev) {
+        CU(cudaMalloc(&slot->dev, sizeof(float) * 4 * n_iters));
+        slot->cap = n_iters;
+    }
+    std::vector<float> tab;
+    fill_adam_tab(tab, n_iters, step0, (double)lr, (double)lr_shape);
+    // pageable source: the copy has left the host vector when the call returns
+    CU(cudaMemcpyAsync(slot->dev, tab.data(), sizeof(float) * tab.size(), cudaMemcpyHostToDevice, st));
+    slot->stream = st; slot->iters = n_iters; slot->step0 = step0; slot->lr = (double)lr; slot->lrs = (double)lr_shape;
+    dev = slot->dev;
+    return ODAM_SQ_OK;
+}
+
 using OptKernel = void (*)(OptArgs);
 
-// every instantiation is capped at 64 registers/thread (1024 resident threads per SM worth of registers); the compact
-// layout only exists for CTAs of up to 256 threads (it is for many small CTAs per SM)
-static OptKernel pick_kernel(int threads, int compact, int solo = 0, int prof = 0)
+// The builds of sq_optimize_kernel, each with its cycle-mark twin (prof), in ascending CTA size within each layout.
+// Their register budget follows from __launch_bounds__: SQ_MIN_BLOCKS CTAs of `threads` share the 64K registers.
+// The compact layout only exists for CTAs of up to 256 threads (it is for many small CTAs per SM).
+struct OptBuild { int threads; bool compact, solo, prof; OptKernel kern; };
+static const OptBuild kOptBuilds[] = {
+    {256, false, false, false, sq_optimize_kernel<256, false, false, false>},
+    {512, false, false, false, sq_optimize_kernel<512, false, false, false>},
+    {1024, false, false, false, sq_optimize_kernel<1024, false, false, false>},
+    {256, true, false, false, sq_optimize_kernel<256, true, false, false>},
+    {512, false, true, false, sq_optimize_kernel<512, false, true, false>},
+    {256, false, false, true, sq_optimize_kernel<256, false, false, true>},
+    {512, false, false, true, sq_optimize_kernel<512, false, false, true>},
+    {1024, false, false, true, sq_optimize_kernel<1024, false, false, true>},
+    {256, true, false, true, sq_optimize_kernel<256, true, false, true>},
+    {512, false, true, true, sq_optimize_kernel<512, false, true, true>},
+};
+
+// the smallest build of the layout that fits `threads` CTA threads; the solo build when every CTA has an SM to itself
+// and it fits, else the shared one; NULL: no such build
+static const OptBuild *pick_build(int threads, bool compact, bool solo, bool prof)
 {
-    if (prof) {   // the same builds with the cycle marks compiled in
-        if (solo && !compact && threads <= 512) return sq_optimize_kernel<512, false, true, true>;
-        if (compact) return threads <= 256 ? sq_optimize_kernel<256, true, false, true> : nullptr;
-        return threads <= 256 ? sq_optimize_kernel<256, false, false, true>
-                              : (threads <= 512 ? sq_optimize_kernel<512, false, false, true> : sq_optimize_kernel<1024, false, false, true>);
-    }
-    if (solo && !compact && threads <= 512) return sq_optimize_kernel<512, false, true>;   // one CTA per SM: 128 registers
-    if (compact) return threads <= 256 ? sq_optimize_kernel<256, true> : nullptr;
-    return threads <= 256 ? sq_optimize_kernel<256, false>
-                          : (threads <= 512 ? sq_optimize_kernel<512, false> : sq_optimize_kernel<1024, false>);
+    for (int want_solo = solo && !compact; want_solo >= 0; want_solo--)
+        for (const OptBuild &B : kOptBuilds)
+            if (B.compact == compact && B.solo == (bool)want_solo && B.prof == prof && threads <= B.threads) return &B;
+    return nullptr;
 }
+
+static int opt_regs(const OptBuild &B) { return 65536 / (B.threads * SQ_MIN_BLOCKS(B.threads, B.compact, B.solo)); }
+
+// Dynamic shared memory of each per-object kernel: its launcher asks for this much and ensure_init() sets the kernel's
+// attribute to it (sq_sides_kernel's kSidesSmem is in sq_autograd.cuh)
+constexpr size_t kPointsSmem = kFwdSmem, kObbSmem = kFwdSmem, kBoxesSmem = kFwdSmem, kAnglesSmem = kFwdSmem;
+constexpr size_t kPointsVjpSmem = kFwdSmem, kSidesVjpSmem = kFwdSmem;
 
 static int ensure_init(int device)
 {
@@ -994,13 +1061,9 @@ static int ensure_init(int device)
         std::copy(one.begin(), one.end(), tab.begin() + kTabSize);
         CU(cudaMemcpyToSymbol(g_logtab, tab.data(), sizeof(double2) * 2 * kTabSize));
     }
-    for (int compact = 0; compact < 2; compact++)
-        for (int threads : {256, 512, 1024})
-            for (int prof = 0; prof < 2; prof++)
-                if (auto kern = pick_kernel(threads, compact, 0, prof))
-                    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, D.max_smem_optin - (int)sizeof(Smem)));
-    for (int prof = 0; prof < 2; prof++)
-        CU(cudaFuncSetAttribute(pick_kernel(512, 0, 1, prof), cudaFuncAttributeMaxDynamicSharedMemorySize, D.max_smem_optin - (int)sizeof(Smem)));
+    for (const OptBuild &B : kOptBuilds)
+        CU(cudaFuncSetAttribute(B.kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                D.max_smem_optin - (int)sizeof(Smem)));
     // How many view-tiled clusters can have every CTA on an SM of its own?  A cluster must fit one GPC, and the GPCs
     // of a 148-SM B200 do not hold a whole number of 3- or 4-CTA clusters: measured, 45 x 3 and 32 x 4 CTAs run one
     // per SM while 46 x 3 or 34 x 4 put two CTAs on some SMs and are 10..19 % slower than the next smaller cluster.
@@ -1015,33 +1078,110 @@ static int ensure_init(int device)
         attr.val.clusterDim.x = c; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
         cfg.attrs = &attr; cfg.numAttrs = 1;
         int num = 0;
-        if (cudaOccupancyMaxActiveClusters(&num, sq_optimize_kernel<512, false>, &cfg) == cudaSuccess) D.excl_clusters[c] = num;
+        if (cudaOccupancyMaxActiveClusters(&num, pick_build(512, false, false, false)->kern, &cfg) == cudaSuccess)
+            D.excl_clusters[c] = num;
         else cudaGetLastError();
     }
-    CU(cudaFuncSetAttribute(sq_points_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
-    CU(cudaFuncSetAttribute(sq_boxes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
-    CU(cudaFuncSetAttribute(sq_angles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
-    CU(cudaFuncSetAttribute(sq_obb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
-    CU(cudaFuncSetAttribute(sq_points_vjp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
-    CU(cudaFuncSetAttribute(sq_sides_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSidesSmem));
-    CU(cudaFuncSetAttribute(sq_sides_vjp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
-    CU(cudaFuncSetAttribute(sq_sides_vjp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFwdSmem));
+    const struct { const void *kern; size_t smem; } per_object[] = {
+        {(const void *)sq_points_kernel, kPointsSmem},
+        {(const void *)sq_boxes_kernel, kBoxesSmem},
+        {(const void *)sq_angles_kernel, kAnglesSmem},
+        {(const void *)sq_obb_kernel, kObbSmem},
+        {(const void *)sq_points_vjp_kernel, kPointsVjpSmem},
+        {(const void *)sq_sides_kernel, kSidesSmem},
+        {(const void *)sq_sides_vjp_kernel<false>, kSidesVjpSmem},
+        {(const void *)sq_sides_vjp_kernel<true>, kSidesVjpSmem},
+    };
+    for (const auto &k : per_object)
+        CU(cudaFuncSetAttribute(k.kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem));
     CU(cudaStreamCreateWithFlags(&D.stream, cudaStreamNonBlocking));
     D.ready = true;
     return ODAM_SQ_OK;
-}
-
-// the device-pointer entries run on the caller's current device
-static int init_current_device(int &device)
-{
-    CU(cudaGetDevice(&device));
-    return ensure_init(device);
 }
 
 static int check_launch()
 {
     CU(cudaGetLastError());
     return ODAM_SQ_OK;
+}
+
+// body(D) of a device-pointer entry with validated arguments: nothing for n == 0, else on the caller's current device
+template <class F>
+static int on_current_device(int n, F &&body)
+{
+    if (n == 0) return ODAM_SQ_OK;
+    int device;
+    CU(cudaGetDevice(&device));
+    int rc = ensure_init(device);
+    if (rc) return rc;
+    return body(g_dev[device]);
+}
+
+// One launcher per kernel: the only place that names its grid and CTA size, with the dynamic shared memory declared
+// above ensure_init().  One CTA per object unless stated.
+static int launch_points(const float *params, int n, float *xyz, cudaStream_t st)
+{
+    sq_points_kernel<<<n, 256, kPointsSmem, st>>>(params, n, xyz);
+    return check_launch();
+}
+
+static int launch_obb(const float *params, int n, double *corners, int32_t *flag, float *xyz, cudaStream_t st)
+{
+    sq_obb_kernel<<<n, 256, kObbSmem, st>>>(params, n, corners, flag, xyz);
+    return check_launch();
+}
+
+static int launch_boxes(const float *params, const int32_t *view_off, const float *Ms, int n, float *box,
+                        cudaStream_t st)
+{
+    sq_boxes_kernel<<<n, 256, kBoxesSmem, st>>>(params, view_off, Ms, n, box);
+    return check_launch();
+}
+
+static int launch_points_vjp(const float *params, const float *grad_xyz, int n, float *grad_params, cudaStream_t st)
+{
+    sq_points_vjp_kernel<<<n, kAgThreads, kPointsVjpSmem, st>>>(params, grad_xyz, n, grad_params);
+    return check_launch();
+}
+
+static int launch_sides(const float *params, const int32_t *view_off, const float *Ms, int n, int total_views,
+                        float *pred, int32_t *arg, cudaStream_t st)
+{
+    sq_sides_kernel<<<n, kAgThreads, kSidesSmem, st>>>(params, view_off, Ms, n, total_views, pred, arg);
+    return check_launch();
+}
+
+template <bool kCams>
+static int launch_sides_vjp(const float *params, const int32_t *view_off, const float *Ms, const int32_t *arg,
+                            const float *grad_pred, int n, int total_views, float *grad_params, float *grad_Ms,
+                            cudaStream_t st)
+{
+    sq_sides_vjp_kernel<kCams><<<n, kAgThreads, kSidesVjpSmem, st>>>(params, view_off, Ms, arg, grad_pred, n,
+                                                                      total_views, grad_params, grad_Ms);
+    return check_launch();
+}
+
+static int launch_obb_points(const float *points, int n, int n_pts, double *corners, int32_t *flag, cudaStream_t st)
+{
+    sq_obb_points_kernel<<<n, 256, 0, st>>>(points, n, n_pts, corners, flag);
+    return check_launch();
+}
+
+// grid-stride over the n x n pairs, at most 16 CTAs per SM
+static int launch_merge_cost(const double *boxes, const int32_t *cls, int n, double *cost, double *iou3d, double *iou2d,
+                             int sm_count, cudaStream_t st)
+{
+    const int threads = 128;
+    const int blocks = (int)std::min<size_t>(((size_t)n * n + threads - 1) / threads, (size_t)sm_count * 16);
+    sq_merge_cost_kernel<<<blocks, threads, 0, st>>>(boxes, cls, n, cost, iou3d, iou2d);
+    return check_launch();
+}
+
+static int launch_angles(const float *shapes, const float *epsilons, int n, float *etas, float *omegas,
+                         const float *u_eta, const uint8_t *k_omega, cudaStream_t st)
+{
+    sq_angles_kernel<<<n, 64, kAnglesSmem, st>>>(shapes, epsilons, n, etas, omegas, u_eta, k_omega);
+    return check_launch();
 }
 
 constexpr double kCompactMaxViews = 40;  // mean views per CTA up to which the compact layout wins (measured)
@@ -1087,7 +1227,6 @@ static int choose_launch(int max_views, double mean_views, int n, const odam_sq_
     if (layout < 0 || layout > 2) return ODAM_SQ_ERR_ARG;
     if (layout == 0)
         layout = (dense && mean_views <= kCompactMaxViews && (threads == 0 ? !two_wide : threads <= 256)) ? 2 : 1;
-    if (layout == 2 && threads > 256) return ODAM_SQ_ERR_ARG;
     if (threads == 0) {
         // measured on B200 (DESIGN.md section 5): in the throughput regime (several CTAs per SM) 256 threads, 320 for
         // long tracks; in the latency regime (fewer CTAs than SMs) a wide CTA with many point slices per view
@@ -1102,6 +1241,9 @@ static int choose_launch(int max_views, double mean_views, int n, const odam_sq_
         }
     }
     if (threads % 32 || threads < 64 || threads > 1024) return ODAM_SQ_ERR_ARG;  // two warps share the sampler's tail
+    // a layout with no build of this CTA size (the compact one above 256 threads, also when it was asked for with
+    // threads chosen here): every configuration this returns has a build, and pick_build() relies on it
+    if (!pick_build(threads, layout == 2, !dense, false)) return ODAM_SQ_ERR_ARG;
     long items = std::max(threads, max_views);  // V * min(max_slices, threads / V) <= threads when V <= threads
     long red_offset = std::max<long>(items * 4 * 8, (long)kSpecBytes);  // phase-E results alias the B0 scratch
     long smem = red_offset + (threads / 32) * (kRed + 3) * 4;            // + cross-warp reduction rows
@@ -1123,20 +1265,7 @@ static int choose_launch(int max_views, double mean_views, int n, const odam_sq_
     return ODAM_SQ_OK;
 }
 
-static void fill_adam_tab(std::vector<float> &tab, int n_iters, int step0, double lr, double lr_shape)
-{
-    tab.resize((size_t)n_iters * 4);
-    for (int it = 0; it < n_iters; it++) {
-        double step = (double)(step0 + it + 1);
-        double bc1 = 1.0 - pow(0.9, step), bc2 = 1.0 - pow(0.999, step);
-        tab[it * 4 + 0] = (float)(-(lr / bc1));
-        tab[it * 4 + 1] = (float)(-(lr_shape / bc1));
-        tab[it * 4 + 2] = (float)pow(bc2, 0.5);
-        tab[it * 4 + 3] = 0.f;
-    }
-}
-
-static int launch_optimize(DeviceState &D, const OptArgs &A0, const LaunchCfg &L, cudaStream_t st)
+static int launch_optimize(const OptArgs &A0, const LaunchCfg &L, cudaStream_t st)
 {
     OptArgs A = A0;
     A.max_slices = L.max_slices;
@@ -1145,7 +1274,7 @@ static int launch_optimize(DeviceState &D, const OptArgs &A0, const LaunchCfg &L
     A.red_offset = L.red_offset;
     A.stage_offset = L.stage_offset; A.stage_views = L.stage_views;
     if (A.out_status) CU(cudaMemsetAsync(A.out_status, 0, sizeof(int32_t) * A.n, st));  // CTAs OR their flags in
-    OptKernel kern = pick_kernel(L.threads, L.compact, L.solo, A.out_cycles != nullptr);
+    OptKernel kern = pick_build(L.threads, L.compact, L.solo, A.out_cycles != nullptr)->kern;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof cfg);
 #ifndef SQ_EXTRA_SMEM
@@ -1234,16 +1363,49 @@ class Staging {
     }
 };
 
+// most views of an object, from view offsets in host memory; *ordered: whether the offsets never decrease
+static int most_views(const int32_t *view_off, int n, bool *ordered = nullptr)
+{
+    int maxv = 0;
+    bool ok = true;
+    for (int i = 0; i < n; i++) {
+        ok = ok && view_off[i + 1] >= view_off[i];
+        maxv = std::max(maxv, view_off[i + 1] - view_off[i]);
+    }
+    if (ordered) *ordered = ok;
+    return maxv;
+}
+
 // host view offsets: start at 0 and never decrease (so they index the staged arrays); maxv = most views of an object
 static int check_view_off(const int32_t *view_off, int n, int &maxv)
 {
-    if (view_off[0] != 0) return ODAM_SQ_ERR_ARG;
-    maxv = 0;
-    for (int i = 0; i < n; i++) {
-        if (view_off[i + 1] < view_off[i]) return ODAM_SQ_ERR_ARG;
-        maxv = std::max(maxv, view_off[i + 1] - view_off[i]);
-    }
-    return ODAM_SQ_OK;
+    bool ordered;
+    maxv = most_views(view_off, n, &ordered);
+    return view_off[0] == 0 && ordered ? ODAM_SQ_OK : ODAM_SQ_ERR_ARG;
+}
+
+// the checks shared by the device- and host-pointer entry of each operation
+static int check_sample_points(const float *params, int n, const float *xyz)
+{
+    return !params || !xyz || n < 0 ? ODAM_SQ_ERR_ARG : ODAM_SQ_OK;
+}
+
+static int check_project_boxes(const float *params, const int32_t *view_off, const float *Ms, int n, const float *box)
+{
+    return !params || !view_off || !Ms || !box || n < 0 ? ODAM_SQ_ERR_ARG : ODAM_SQ_OK;
+}
+
+static int check_oriented_boxes(const float *params, int n, const double *corners)
+{
+    return !params || !corners || n < 0 ? ODAM_SQ_ERR_ARG : ODAM_SQ_OK;
+}
+
+// odam_sq_box_sides_vjp(_cameras): `out` is the gradient the entry must write
+static int check_sides_vjp(const float *params, const int32_t *view_off, const float *Ms, const int32_t *arg,
+                           const float *grad_pred, int n, int total_views, const float *out)
+{
+    return !params || !view_off || !Ms || !arg || !grad_pred || !out || n < 0 || total_views < 0 ? ODAM_SQ_ERR_ARG
+                                                                                                  : ODAM_SQ_OK;
 }
 
 // the arguments of odam_sq_optimize(_host); the launch fields and adam_tab are set later
@@ -1312,8 +1474,7 @@ int odam_sq_query_launch(const int32_t *view_off, int n, const odam_sq_options *
                          int *ctas_per_sm, int *cluster, int *code_layout, int *max_slices)
 {
     if (!view_off || n <= 0) return ODAM_SQ_ERR_ARG;
-    int maxv = 0;
-    for (int i = 0; i < n; i++) maxv = std::max(maxv, view_off[i + 1] - view_off[i]);
+    const int maxv = most_views(view_off, n);
     LaunchCfg L;
     int sm_count = 148, smem_optin = 232448;   // B200; the current device's own numbers once it is initialised
     const int *excl = nullptr;
@@ -1335,7 +1496,7 @@ int odam_sq_query_launch(const int32_t *view_off, int n, const odam_sq_options *
     if (max_slices) *max_slices = L.max_slices;
     if (smem_bytes) *smem_bytes = L.smem;
     if (smem_bytes) *smem_bytes += (int)sizeof(Smem);
-    const int regs = (L.solo && !L.compact && L.threads <= 512) ? 128 : 64;   // the build pick_kernel() selects
+    const int regs = opt_regs(*pick_build(L.threads, L.compact, L.solo, false));
     if (ctas_per_sm) *ctas_per_sm = std::min({32, 2048 / L.threads, 65536 / (regs * L.threads), (233472 - 1024) / (L.smem + (int)sizeof(Smem) + 1024)});
     return ODAM_SQ_OK;
 }
@@ -1349,88 +1510,46 @@ int odam_sq_optimize(const float *init, const int32_t *cls, const int32_t *view_
 {
     OptArgs A = opt_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
                          out_status, opt);
-    int device = 0, rc = check_opt_args(A, representation);
-    if (rc || n == 0 || n_iters == 0) return rc;
-    rc = init_current_device(device);
-    if (rc) return rc;
-    DeviceState &D = g_dev[device];
-    cudaStream_t st = (cudaStream_t)stream;
-    int maxv = opt ? opt->max_views : 0;
-    double meanv = maxv;
-    if (!(opt && opt->threads && maxv > 0)) {
-        std::vector<int32_t> voff(n + 1);
-        CU(cudaMemcpyAsync(voff.data(), view_off, sizeof(int32_t) * (n + 1), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        maxv = 0;
-        for (int i = 0; i < n; i++) {
-            if (voff[i + 1] < voff[i]) return ODAM_SQ_ERR_ARG;
-            maxv = std::max(maxv, voff[i + 1] - voff[i]);
+    int rc = check_opt_args(A, representation);
+    if (rc || n_iters == 0) return rc;
+    return on_current_device(n, [&](DeviceState &D) {
+        cudaStream_t st = (cudaStream_t)stream;
+        int maxv = opt ? opt->max_views : 0;
+        double meanv = maxv;
+        if (!(opt && opt->threads && maxv > 0)) {
+            std::vector<int32_t> voff(n + 1);
+            CU(cudaMemcpyAsync(voff.data(), view_off, sizeof(int32_t) * (n + 1), cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            bool ordered;
+            maxv = most_views(voff.data(), n, &ordered);
+            if (!ordered) return ODAM_SQ_ERR_ARG;
+            meanv = (double)(voff[n] - voff[0]) / n;
         }
-        meanv = (double)(voff[n] - voff[0]) / n;
-    }
-    LaunchCfg L;
-    rc = choose_launch(maxv, meanv, n, opt, D.sm_count, D.max_smem_optin, D.excl_clusters, L);
-    if (rc) return rc;
-    // Adam bias-correction table (host doubles, as torch computes them in Python floats); one cached table per
-    // (stream, schedule), so launches on different streams never share -- or overwrite -- each other's table
-    {
-        std::lock_guard<std::mutex> lk(g_mu);
-        const int step0 = opt ? opt->step0 : 0;
-        for (const AdamTab &t : D.tabs)
-            if (t.stream == st && t.iters == n_iters && t.step0 == step0 && t.lr == (double)lr && t.lrs == (double)lr_shape)
-                A.adam_tab = t.dev;
-        if (!A.adam_tab) {
-            AdamTab *slot = nullptr;
-            for (AdamTab &t : D.tabs)
-                if (t.stream == st) slot = &t;                    // this stream's previous schedule: reuse its buffer
-            if (!slot && D.tabs.size() >= 16) slot = &D.tabs[0];  // bounded cache: recycle the oldest entry
-            if (slot) {
-                CU(cudaStreamSynchronize(slot->stream));          // its last launch may still read the table
-                if (slot->cap < n_iters) { cudaFree(slot->dev); slot->dev = nullptr; slot->cap = 0; }
-            } else {
-                D.tabs.push_back(AdamTab{st, 0, 0, 0, 0, nullptr, 0});
-                slot = &D.tabs.back();
-            }
-            if (!slot->dev) {
-                CU(cudaMalloc(&slot->dev, sizeof(float) * 4 * n_iters));
-                slot->cap = n_iters;
-            }
-            std::vector<float> tab;
-            fill_adam_tab(tab, n_iters, step0, (double)lr, (double)lr_shape);
-            // pageable source: the copy has left the host vector when the call returns
-            CU(cudaMemcpyAsync(slot->dev, tab.data(), sizeof(float) * tab.size(), cudaMemcpyHostToDevice, st));
-            slot->stream = st; slot->iters = n_iters; slot->step0 = step0; slot->lr = (double)lr; slot->lrs = (double)lr_shape;
-            A.adam_tab = slot->dev;
-        }
-    }
-    rc = launch_optimize(D, A, L, st);
-    if (rc) return rc;
-    if (opt && opt->out_corners) {   // run_multi_view.py:66-67 right behind the optimiser, same stream
-        sq_obb_kernel<<<n, 256, kFwdSmem, st>>>(out_params, n, opt->out_corners, opt->out_box_flag, nullptr);
-        return check_launch();
-    }
-    return ODAM_SQ_OK;
+        LaunchCfg L;
+        rc = choose_launch(maxv, meanv, n, opt, D.sm_count, D.max_smem_optin, D.excl_clusters, L);
+        if (rc) return rc;
+        rc = adam_table(D, st, n_iters, opt ? opt->step0 : 0, lr, lr_shape, A.adam_tab);
+        if (rc) return rc;
+        rc = launch_optimize(A, L, st);
+        if (rc || !(opt && opt->out_corners)) return rc;
+        // run_multi_view.py:66-67 right behind the optimiser, same stream
+        return launch_obb(out_params, n, opt->out_corners, opt->out_box_flag, nullptr, st);
+    });
 }
 
 int odam_sq_sample_points(const float *params, int n, float *out_xyz, void *stream)
 {
-    if (!params || !out_xyz || n < 0) return ODAM_SQ_ERR_ARG;
-    if (n == 0) return ODAM_SQ_OK;
-    int device, rc = init_current_device(device);
-    if (rc) return rc;
-    sq_points_kernel<<<n, 256, kFwdSmem, (cudaStream_t)stream>>>(params, n, out_xyz);
-    return check_launch();
+    if (int rc = check_sample_points(params, n, out_xyz)) return rc;
+    return on_current_device(n, [&](DeviceState &) { return launch_points(params, n, out_xyz, (cudaStream_t)stream); });
 }
 
 int odam_sq_project_boxes(const float *params, const int32_t *view_off, const float *Ms, int n, float *out_box,
                           void *stream)
 {
-    if (!params || !view_off || !Ms || !out_box || n < 0) return ODAM_SQ_ERR_ARG;
-    if (n == 0) return ODAM_SQ_OK;
-    int device, rc = init_current_device(device);
-    if (rc) return rc;
-    sq_boxes_kernel<<<n, 256, kFwdSmem, (cudaStream_t)stream>>>(params, view_off, Ms, n, out_box);
-    return check_launch();
+    if (int rc = check_project_boxes(params, view_off, Ms, n, out_box)) return rc;
+    return on_current_device(n, [&](DeviceState &) {
+        return launch_boxes(params, view_off, Ms, n, out_box, (cudaStream_t)stream);
+    });
 }
 
 // ---- differentiable ops (sq_autograd.cuh): device pointers, enqueued on `stream` ----
@@ -1438,51 +1557,39 @@ int odam_sq_project_boxes(const float *params, const int32_t *view_off, const fl
 int odam_sq_sample_points_vjp(const float *params, const float *grad_xyz, int n, float *out_grad_params, void *stream)
 {
     if (!params || !grad_xyz || !out_grad_params || n < 0) return ODAM_SQ_ERR_ARG;
-    if (n == 0) return ODAM_SQ_OK;
-    int device, rc = init_current_device(device);
-    if (rc) return rc;
-    sq_points_vjp_kernel<<<n, kAgThreads, kFwdSmem, (cudaStream_t)stream>>>(params, grad_xyz, n, out_grad_params);
-    return check_launch();
+    return on_current_device(n, [&](DeviceState &) {
+        return launch_points_vjp(params, grad_xyz, n, out_grad_params, (cudaStream_t)stream);
+    });
 }
 
 int odam_sq_box_sides(const float *params, const int32_t *view_off, const float *Ms, int n, int total_views,
                       float *out_pred, int32_t *out_arg, void *stream)
 {
     if (!params || !view_off || !Ms || !out_pred || !out_arg || n < 0 || total_views < 0) return ODAM_SQ_ERR_ARG;
-    if (n == 0) return ODAM_SQ_OK;
-    int device, rc = init_current_device(device);
-    if (rc) return rc;
-    sq_sides_kernel<<<n, kAgThreads, kSidesSmem, (cudaStream_t)stream>>>(params, view_off, Ms, n, total_views, out_pred,
-                                                                          out_arg);
-    return check_launch();
+    return on_current_device(n, [&](DeviceState &) {
+        return launch_sides(params, view_off, Ms, n, total_views, out_pred, out_arg, (cudaStream_t)stream);
+    });
 }
 
 int odam_sq_box_sides_vjp(const float *params, const int32_t *view_off, const float *Ms, const int32_t *arg,
                           const float *grad_pred, int n, int total_views, float *out_grad_params, void *stream)
 {
-    if (!params || !view_off || !Ms || !arg || !grad_pred || !out_grad_params || n < 0 || total_views < 0)
-        return ODAM_SQ_ERR_ARG;
-    if (n == 0) return ODAM_SQ_OK;
-    int device, rc = init_current_device(device);
-    if (rc) return rc;
-    sq_sides_vjp_kernel<false><<<n, kAgThreads, kFwdSmem, (cudaStream_t)stream>>>(params, view_off, Ms, arg, grad_pred, n,
-                                                                                   total_views, out_grad_params, nullptr);
-    return check_launch();
+    if (int rc = check_sides_vjp(params, view_off, Ms, arg, grad_pred, n, total_views, out_grad_params)) return rc;
+    return on_current_device(n, [&](DeviceState &) {
+        return launch_sides_vjp<false>(params, view_off, Ms, arg, grad_pred, n, total_views, out_grad_params, nullptr,
+                                       (cudaStream_t)stream);
+    });
 }
 
 int odam_sq_box_sides_vjp_cameras(const float *params, const int32_t *view_off, const float *Ms, const int32_t *arg,
                                   const float *grad_pred, int n, int total_views, float *out_grad_params,
                                   float *out_grad_Ms, void *stream)
 {
-    if (!params || !view_off || !Ms || !arg || !grad_pred || !out_grad_Ms || n < 0 || total_views < 0)
-        return ODAM_SQ_ERR_ARG;
-    if (n == 0) return ODAM_SQ_OK;
-    int device, rc = init_current_device(device);
-    if (rc) return rc;
-    sq_sides_vjp_kernel<true><<<n, kAgThreads, kFwdSmem, (cudaStream_t)stream>>>(params, view_off, Ms, arg, grad_pred, n,
-                                                                                  total_views, out_grad_params,
-                                                                                  out_grad_Ms);
-    return check_launch();
+    if (int rc = check_sides_vjp(params, view_off, Ms, arg, grad_pred, n, total_views, out_grad_Ms)) return rc;
+    return on_current_device(n, [&](DeviceState &) {
+        return launch_sides_vjp<true>(params, view_off, Ms, arg, grad_pred, n, total_views, out_grad_params,
+                                      out_grad_Ms, (cudaStream_t)stream);
+    });
 }
 
 // ---- host-pointer entry points: one Staging round trip on the library's own stream ----
@@ -1524,31 +1631,27 @@ int odam_sq_optimize_host(const float *init, const int32_t *cls, const int32_t *
     S.out(A.out_eta_idx, (size_t)n * kN); S.out(A.out_grids, (size_t)n * 2 * kG);
     S.out(A.out_param_hist, n9 * n_iters); S.out(corners, (size_t)n * 24); S.out(box_flag, n);
     return S.run(device, [&](cudaStream_t st) {
-        rc = launch_optimize(g_dev[device], A, L, st);
+        rc = launch_optimize(A, L, st);
         if (rc || !corners) return rc;
         // run_multi_view.py:66-67 right behind the optimiser: no second call, copy or sync
-        sq_obb_kernel<<<n, 256, kFwdSmem, st>>>(A.out_params, n, corners, box_flag, nullptr);
-        return check_launch();
+        return launch_obb(A.out_params, n, corners, box_flag, nullptr, st);
     });
 }
 
 int odam_sq_sample_points_host(const float *params, int n, float *out_xyz, int device)
 {
-    if (!params || !out_xyz || n < 0) return ODAM_SQ_ERR_ARG;
+    if (int rc = check_sample_points(params, n, out_xyz)) return rc;
     if (n == 0) return ODAM_SQ_OK;
     Staging S;
     S.in(params, (size_t)n * 9);
     S.out(out_xyz, (size_t)n * kN * 3);
-    return S.run(device, [&](cudaStream_t st) {
-        sq_points_kernel<<<n, 256, kFwdSmem, st>>>(params, n, out_xyz);
-        return check_launch();
-    });
+    return S.run(device, [&](cudaStream_t st) { return launch_points(params, n, out_xyz, st); });
 }
 
 int odam_sq_project_boxes_host(const float *params, const int32_t *view_off, const float *Ms, int n, float *out_box,
                                int device)
 {
-    if (!params || !view_off || !Ms || !out_box || n < 0) return ODAM_SQ_ERR_ARG;
+    if (int rc = check_project_boxes(params, view_off, Ms, n, out_box)) return rc;
     if (n == 0) return ODAM_SQ_OK;
     int maxv, rc = check_view_off(view_off, n, maxv);
     if (rc) return rc;
@@ -1556,35 +1659,27 @@ int odam_sq_project_boxes_host(const float *params, const int32_t *view_off, con
     Staging S;
     S.in(params, (size_t)n * 9); S.in(view_off, n + 1); S.in(Ms, SV * 12);
     S.out(out_box, SV * 4);
-    return S.run(device, [&](cudaStream_t st) {
-        sq_boxes_kernel<<<n, 256, kFwdSmem, st>>>(params, view_off, Ms, n, out_box);
-        return check_launch();
-    });
+    return S.run(device, [&](cudaStream_t st) { return launch_boxes(params, view_off, Ms, n, out_box, st); });
 }
 
 int odam_sq_oriented_boxes_host(const float *params, int n, double *out_corners, int32_t *out_flag, float *out_xyz,
                                 int device)
 {
-    if (!params || !out_corners || n < 0) return ODAM_SQ_ERR_ARG;
+    if (int rc = check_oriented_boxes(params, n, out_corners)) return rc;
     if (n == 0) return ODAM_SQ_OK;
     Staging S;
     S.in(params, (size_t)n * 9);
     S.out(out_corners, (size_t)n * 24); S.out(out_flag, n); S.out(out_xyz, (size_t)n * kN * 3);
-    return S.run(device, [&](cudaStream_t st) {
-        sq_obb_kernel<<<n, 256, kFwdSmem, st>>>(params, n, out_corners, out_flag, out_xyz);
-        return check_launch();
-    });
+    return S.run(device, [&](cudaStream_t st) { return launch_obb(params, n, out_corners, out_flag, out_xyz, st); });
 }
 
 int odam_sq_oriented_boxes(const float *params, int n, double *out_corners, int32_t *out_flag, float *out_xyz,
                            void *stream)
 {
-    if (!params || !out_corners || n < 0) return ODAM_SQ_ERR_ARG;
-    if (n == 0) return ODAM_SQ_OK;
-    int device, rc = init_current_device(device);
-    if (rc) return rc;
-    sq_obb_kernel<<<n, 256, kFwdSmem, (cudaStream_t)stream>>>(params, n, out_corners, out_flag, out_xyz);
-    return check_launch();
+    if (int rc = check_oriented_boxes(params, n, out_corners)) return rc;
+    return on_current_device(n, [&](DeviceState &) {
+        return launch_obb(params, n, out_corners, out_flag, out_xyz, (cudaStream_t)stream);
+    });
 }
 
 int odam_sq_oriented_boxes_of_points_host(const float *points, int n, int n_pts, double *out_corners, int32_t *out_flag,
@@ -1596,8 +1691,7 @@ int odam_sq_oriented_boxes_of_points_host(const float *points, int n, int n_pts,
     S.in(points, (size_t)n * n_pts * 3);
     S.out(out_corners, (size_t)n * 24); S.out(out_flag, n);
     return S.run(device, [&](cudaStream_t st) {
-        sq_obb_points_kernel<<<n, 256, 0, st>>>(points, n, n_pts, out_corners, out_flag);
-        return check_launch();
+        return launch_obb_points(points, n, n_pts, out_corners, out_flag, st);
     });
 }
 
@@ -1611,10 +1705,7 @@ int odam_sq_merge_cost_host(const double *boxes, const int32_t *cls, int n, doub
     S.in(boxes, (size_t)n * 24); S.in(cls, n);
     S.out(out_cost, nn); S.out(out_iou3d, nn); S.out(out_iou2d, nn);
     return S.run(device, [&](cudaStream_t st) {
-        const int threads = 128;
-        const int blocks = (int)std::min<size_t>((nn + threads - 1) / threads, (size_t)g_dev[device].sm_count * 16);
-        sq_merge_cost_kernel<<<blocks, threads, 0, st>>>(boxes, cls, n, out_cost, out_iou3d, out_iou2d);
-        return check_launch();
+        return launch_merge_cost(boxes, cls, n, out_cost, out_iou3d, out_iou2d, g_dev[device].sm_count, st);
     });
 }
 
@@ -1647,8 +1738,7 @@ int odam_sq_sample_on_batch_host(const float *shapes, const float *epsilons, flo
     S.in(shapes, (size_t)n * 3); S.in(epsilons, (size_t)n * 2); S.in(u_ptr, u_eta.size()); S.in(k_ptr, k_omega.size());
     S.out(etas, (size_t)n * kN); S.out(omegas, (size_t)n * kN);
     return S.run(device, [&](cudaStream_t st) {
-        sq_angles_kernel<<<n, 64, kFwdSmem, st>>>(shapes, epsilons, n, etas, omegas, u_ptr, k_ptr);
-        return check_launch();
+        return launch_angles(shapes, epsilons, n, etas, omegas, u_ptr, k_ptr, st);
     });
 }
 

@@ -100,6 +100,35 @@ def test_argument_validation_without_gpu(lib):
     assert lay.value == 2 and th.value == 256
 
 
+@pytest.mark.parametrize("n, views, threads, ctas_per_sm", [
+    (50, 20, 512, 1),      # latency regime, the solo build: 128 registers per thread
+    (4, 3000, 768, 1),     # latency regime, wider than the solo build: the 1024-thread build
+    (160, 20, 512, 2),     # dense, two wide CTAs per SM
+    (300, 300, 320, 3),    # dense, long tracks
+    (1000, 20, 256, 4),    # dense, the compact build
+])
+def test_query_launch_ctas_per_sm(lib, n, views, threads, ctas_per_sm):
+    """The resident CTAs per SM that odam_sq_query_launch reports (bench.py's launch record) follow the register budget
+    of the build the optimiser launches."""
+    from odam_b200 import api
+    q = api.query_launch(np.arange(0, views * (n + 1), views, dtype=np.int32))
+    assert (q["threads"], q["ctas_per_sm"]) == (threads, ctas_per_sm)
+
+
+@pytest.mark.parametrize("n, views", [(50, 20), (160, 20), (300, 300)])
+def test_compact_layout_wider_than_its_builds_is_rejected(lib, n, views):
+    """The compact layout has builds of up to 256 threads.  Forced onto a batch for which the library picks wider CTAs
+    (latency regime, two wide CTAs per SM, long dense tracks), it is an invalid argument, as it is with the wide CTA
+    size given -- not a configuration without a kernel."""
+    from odam_b200 import _lib, api
+    voff = np.arange(0, views * (n + 1), views, dtype=np.int32)
+    for threads in (0, 512):
+        with pytest.raises(_lib.OdamSqError, match="invalid argument"):
+            api.query_launch(voff, threads=threads, code_layout=2)
+    q = api.query_launch(voff, threads=256, code_layout=2)
+    assert (q["threads"], q["code_layout"]) == (256, 2)
+
+
 def test_no_gpu_means_loud_failure_not_fallback(lib):
     import torch
     if torch.cuda.is_available():
