@@ -93,3 +93,34 @@ def check(rc):
 def ptr(a):
     """numpy array -> void* (None passes NULL)."""
     return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def host_array(name, a, dtype, shape):
+    """A caller's array as a C-contiguous numpy array of `dtype` and `shape` (numpy's reshape rules), None for None.
+    The C entries size their copies from n and the view offsets, not from the arrays, so an array of another size
+    is a ValueError here rather than a read or write past its end."""
+    if a is None:
+        return None
+    a = np.ascontiguousarray(a, dtype)
+    try:
+        return a.reshape(shape)
+    except ValueError:
+        raise ValueError(f"{name} must have shape {list(shape)}, got {list(a.shape)}") from None
+
+
+def check_tensor(name, t, dtype, shape, device):
+    """ValueError unless t is a contiguous `dtype` tensor of exactly `shape` on `device`."""
+    if tuple(t.shape) != tuple(shape) or t.dtype != dtype or not t.is_contiguous() or t.device != device:
+        raise ValueError(f"{name} must be a contiguous {dtype} tensor of shape {list(shape)} on {device}, got "
+                         f"{t.dtype} {list(t.shape)} on {t.device} (contiguous: {t.is_contiguous()})")
+
+
+def tensor_ptr(t):
+    """torch tensor -> void* (None passes NULL)."""
+    return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def current_stream(device):
+    """torch's current stream on `device` as the cudaStream_t the C entries take."""
+    import torch
+    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)

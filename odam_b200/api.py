@@ -46,13 +46,15 @@ class PackedTracks:
 
 
 def init_params(translate, angle, dims, representation="super_quadric"):
-    """What SuperQuadricOptimizer.__init__ builds (reference sq_libs.py:353-369): [t3, yaw, sqrt(dims/2), h2]."""
+    """What SuperQuadricOptimizer.__init__ builds (reference sq_libs.py:353-369): [t3, yaw, sqrt(dims/2), h2].
+    translate [..., 3], angle [...], dims [..., 3] -> [..., 9] float32 (one object's values give [9])."""
     assert representation in ("cube", "super_quadric", "quadric")
-    p = np.empty(9, np.float32)
-    p[0:3] = np.asarray(translate, np.float64)
-    p[3] = np.float64(angle)
-    p[4:7] = np.sqrt(np.asarray(dims, np.float64) / 2)
-    p[7:9] = -10000.0 if representation == "cube" else -0.0
+    angle = np.asarray(angle, np.float64)
+    p = np.empty(angle.shape + (9,), np.float32)
+    p[..., 0:3] = np.asarray(translate, np.float64)
+    p[..., 3] = angle
+    p[..., 4:7] = np.sqrt(np.asarray(dims, np.float64) / 2)
+    p[..., 7:9] = -10000.0 if representation == "cube" else -0.0
     return p
 
 
@@ -70,10 +72,17 @@ def pack_lines(gt_lines):
     return box, mask
 
 
+def unpack_lines(box, mask):
+    """The inverse of pack_lines: (box[V,4], mask[V,4]) -> the reference's list[V] of {side: line}, with the float64
+    lines [1, 0, -x] and [0, 1, -y] of quadric_helper.py:69-109 for the sides the mask keeps."""
+    return [{name: np.array([1, 0, -float(v)] if name[0] == "x" else [0, 1, -float(v)])
+             for name, v, keep in zip(SIDES, b, m) if keep} for b, m in zip(box, mask)]
+
+
 def pack_scene(scene, representation="super_quadric"):
     """odam_b200.synthetic.Scene -> PackedTracks."""
     n, V = scene.n, scene.V
-    init = np.stack([init_params(scene.translate[i], scene.angle[i], scene.dims[i], representation) for i in range(n)])
+    init = init_params(scene.translate, scene.angle, scene.dims, representation)
     return PackedTracks(init=init, cls=scene.cls.astype(np.int32),
                         view_off=(np.arange(n + 1) * V).astype(np.int32),
                         Ms=np.ascontiguousarray(scene.P_cws.reshape(n * V, 12), np.float32),
@@ -133,22 +142,34 @@ def cluster_capacity(device=0):
     return out
 
 
-def _options(n, SV, n_iters, threads, max_slices, m0, v0, step0, s0, extras, alloc, cluster=0, code_layout=0):
-    o = _lib.Options()
-    o.threads, o.max_slices, o.step0, o.cluster = int(threads), int(max_slices), int(step0), int(cluster)
-    o.code_layout = int(code_layout)
-    keep = {}
-    for name, arr, shape in (("m0", m0, (n, 9)), ("v0", v0, (n, 9)), ("s0", s0, (n, 3))):
-        if arr is not None:
-            keep[name] = alloc(arr, shape)
-    shapes = dict(out_m=((n, 9), np.float32), out_v=((n, 9), np.float32), out_grad=((n, 9), np.float32),
-                  out_pred=((SV, 4), np.float32), out_arg=((SV, 4), np.int32),
-                  out_eta_idx=((n, _lib.N_SAMPLES), np.uint8), out_grids=((n, 2, _lib.GRID), np.float32),
-                  out_param_hist=((n, n_iters, 9), np.float32),
-                  out_corners=((n, 8, 3), np.float64), out_box_flag=(n, np.int32))
-    for name in extras:
-        keep[name] = alloc(None, *shapes[name])
-    return o, keep
+def check_classes(cls):
+    """KeyError for the first class id outside 0..7: with the prior on, the reference's CLASS_MAPPER lookup
+    (sq_libs.py:464) fails the same way."""
+    cls = np.asarray(cls)
+    bad = cls[(cls < 0) | (cls > 7)]
+    if bad.size:
+        raise KeyError(int(bad[0]))
+
+
+def check_finite(status, objects=None):
+    """RuntimeError naming the objects whose status has ST_NONFINITE (the reference raises from torch anomaly mode at
+    the offending step).  objects[i] is the caller's index of row i (default: i)."""
+    bad = np.nonzero(status & _lib.ST_NONFINITE)[0]
+    if bad.size:
+        raise RuntimeError(f"superquadric optimisation produced NaN/Inf for object(s) "
+                           f"{(bad if objects is None else np.asarray(objects)[bad]).tolist()} "
+                           "(the reference raises from torch anomaly mode, sq_libs.py:456)")
+
+
+def _track_arrays(tracks):
+    """(init, cls, view_off, Ms, box, mask) of PackedTracks as the optimiser entries read them, each checked against
+    n and view_off[-1]."""
+    n, a = tracks.n, _lib.host_array
+    voff = a("view_off", tracks.view_off, np.int32, (n + 1,))
+    SV = int(voff[-1])
+    return (a("init", tracks.init, np.float32, (n, 9)), a("cls", tracks.cls, np.int32, (n,)), voff,
+            a("Ms", tracks.Ms, np.float32, (SV, 12)), a("box", tracks.box, np.float32, (SV, 4)),
+            a("mask", tracks.mask, np.uint8, (SV, 4)))
 
 
 def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric", lr=0.01, lr_shape=0.1,
@@ -162,23 +183,24 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
             objects, computed by a second launch fused behind the optimiser inside the same call).
     """
     L = _lib.load()
-    n, SV = tracks.n, tracks.total_views
-    f32c = lambda a, shape: np.ascontiguousarray(a, np.float32).reshape(shape)
-
-    def alloc(arr, shape, dtype=np.float32):
-        return np.zeros(shape, dtype) if arr is None else np.ascontiguousarray(arr, dtype).reshape(shape)
-
-    o, keep = _options(n, SV, n_iters, threads, max_slices, m0, v0, step0, s0, extras, alloc, cluster, code_layout)
+    init, cls, voff, Ms, box, mask = _track_arrays(tracks)
+    n, SV = len(init), int(voff[-1])
+    pr = _lib.host_array("prior", prior, np.float32, (8, 9))
+    if pr is not None:
+        check_classes(cls)
+    o = _lib.Options()
+    o.threads, o.max_slices, o.step0, o.cluster = int(threads), int(max_slices), int(step0), int(cluster)
+    o.code_layout = int(code_layout)
+    keep = dict(m0=_lib.host_array("m0", m0, np.float32, (n, 9)), v0=_lib.host_array("v0", v0, np.float32, (n, 9)),
+                s0=_lib.host_array("s0", s0, np.float32, (n, 3)))
+    shapes = dict(out_m=((n, 9), np.float32), out_v=((n, 9), np.float32), out_grad=((n, 9), np.float32),
+                  out_pred=((SV, 4), np.float32), out_arg=((SV, 4), np.int32),
+                  out_eta_idx=((n, _lib.N_SAMPLES), np.uint8), out_grids=((n, 2, _lib.GRID), np.float32),
+                  out_param_hist=((n, n_iters, 9), np.float32),
+                  out_corners=((n, 8, 3), np.float64), out_box_flag=(n, np.int32))
+    keep.update((name, np.zeros(*shapes[name])) for name in extras)
     for name, arr in keep.items():
         setattr(o, name, _lib.ptr(arr))
-    init = f32c(tracks.init, (n, 9))
-    cls = np.ascontiguousarray(tracks.cls, np.int32)
-    voff = np.ascontiguousarray(tracks.view_off, np.int32)
-    Ms, box = f32c(tracks.Ms, (SV, 12)), f32c(tracks.box, (SV, 4))
-    mask = np.ascontiguousarray(tracks.mask, np.uint8).reshape(SV, 4)
-    pr = None if prior is None else f32c(prior, (8, 9))
-    if pr is not None and n and (cls.min() < 0 or cls.max() > 7):
-        raise KeyError(int(cls[(cls < 0) | (cls > 7)][0]))  # the reference's CLASS_MAPPER lookup fails the same way
     out = dict(params=np.zeros((n, 9), np.float32), loss=np.zeros((n, n_iters), np.float32),
                status=np.zeros(n, np.int32))
     rc = L.odam_sq_optimize_host(_lib.ptr(init), _lib.ptr(cls), _lib.ptr(voff), _lib.ptr(Ms), _lib.ptr(box),
@@ -186,17 +208,16 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
                                  lr, lr_shape, _lib.ptr(out["params"]), _lib.ptr(out["loss"]),
                                  _lib.ptr(out["status"]), C.byref(o), device)
     _lib.check(rc)
-    for name in extras:
-        out[name] = keep[name]
+    out.update((name, keep[name]) for name in extras)
     return out
 
 
 def sample_points_host(params, device=0):
     """compute_ellipsoid_points for [n,9] parameter rows -> [n,1000,3] float32 world points."""
     L = _lib.load()
-    p = np.ascontiguousarray(params, np.float32).reshape(-1, 9)
-    out = np.zeros((p.shape[0], _lib.N_SAMPLES, 3), np.float32)
-    _lib.check(L.odam_sq_sample_points_host(_lib.ptr(p), p.shape[0], _lib.ptr(out), device))
+    p = _lib.host_array("params", params, np.float32, (-1, 9))
+    out = np.zeros((len(p), _lib.N_SAMPLES, 3), np.float32)
+    _lib.check(L.odam_sq_sample_points_host(_lib.ptr(p), len(p), _lib.ptr(out), device))
     return out
 
 
@@ -204,9 +225,9 @@ def sample_on_batch(shapes, epsilons, n_samples=1000, device=0):
     """Drop-in for learnable_primitives.fast_sampler.fast_sample_on_batch (reference _sampler.pyx:413-441):
     shapes [B,M,3], epsilons [B,M,2] float32 -> (etas, omegas) [B,M,N] float32."""
     L = _lib.load()
-    a = np.ascontiguousarray(shapes, np.float32)
-    e = np.ascontiguousarray(epsilons, np.float32)
-    B, M = a.shape[0], a.shape[1]
+    B, M = np.shape(shapes)[:2]
+    a = _lib.host_array("shapes", shapes, np.float32, (B, M, 3))
+    e = _lib.host_array("epsilons", epsilons, np.float32, (B, M, 2))
     etas = np.zeros((B, M, n_samples), np.float32)
     omegas = np.zeros((B, M, n_samples), np.float32)
     _lib.check(L.odam_sq_sample_on_batch_host(_lib.ptr(a), _lib.ptr(e), _lib.ptr(etas), _lib.ptr(omegas), B, M,
@@ -217,11 +238,12 @@ def sample_on_batch(shapes, epsilons, n_samples=1000, device=0):
 def project_boxes_host(params, view_off, Ms, device=0):
     """get_bbox for every (object, view): [SV,4] = x_min,x_max,y_min,y_max."""
     L = _lib.load()
-    p = np.ascontiguousarray(params, np.float32).reshape(-1, 9)
-    voff = np.ascontiguousarray(view_off, np.int32)
-    M = np.ascontiguousarray(Ms, np.float32).reshape(-1, 12)
-    out = np.zeros((M.shape[0], 4), np.float32)
-    _lib.check(L.odam_sq_project_boxes_host(_lib.ptr(p), _lib.ptr(voff), _lib.ptr(M), p.shape[0], _lib.ptr(out), device))
+    p = _lib.host_array("params", params, np.float32, (-1, 9))
+    voff = _lib.host_array("view_off", view_off, np.int32, (len(p) + 1,))
+    SV = int(voff[-1])
+    M = _lib.host_array("Ms", Ms, np.float32, (SV, 12))
+    out = np.zeros((max(SV, 0), 4), np.float32)   # offsets that do not start at 0 or decrease are the entry's ERR_ARG
+    _lib.check(L.odam_sq_project_boxes_host(_lib.ptr(p), _lib.ptr(voff), _lib.ptr(M), len(p), _lib.ptr(out), device))
     return out
 
 
@@ -229,8 +251,8 @@ def oriented_boxes_host(params, device=0, want_points=False):
     """compute_ellipsoid_points + compute_oriented_bbox for [n,9] parameter rows in ONE launch (odam_sq_oriented_boxes_host):
     returns corners [n,8,3] float64 (upper four first), flags [n] int32 and, when asked, the points [n,1000,3] float32."""
     L = _lib.load()
-    p = np.ascontiguousarray(params, np.float32).reshape(-1, 9)
-    n = p.shape[0]
+    p = _lib.host_array("params", params, np.float32, (-1, 9))
+    n = len(p)
     corners = np.zeros((n, 8, 3), np.float64)
     flags = np.zeros(n, np.int32)
     pts = np.zeros((n, _lib.N_SAMPLES, 3), np.float32) if want_points else None
@@ -239,12 +261,12 @@ def oriented_boxes_host(params, device=0, want_points=False):
 
 
 def oriented_boxes_of_points_host(points, device=0):
-    """compute_oriented_bbox (reference box_utils.py:319-410) of point sets [n, n_pts, 3] (n_pts <= 1024)."""
+    """compute_oriented_bbox (reference box_utils.py:319-410) of point sets [n, n_pts, 3] (n_pts <= 1024); one set may
+    be given as [n_pts, 3]."""
     L = _lib.load()
-    pts = np.ascontiguousarray(points, np.float32)
-    if pts.ndim == 2:
-        pts = pts[None]
-    n, n_pts = pts.shape[0], pts.shape[1]
+    shape = np.shape(points)
+    n, n_pts = ((1,) + shape if len(shape) == 2 else shape)[:2]
+    pts = _lib.host_array("points", points, np.float32, (n, n_pts, 3))
     corners = np.zeros((n, 8, 3), np.float64)
     flags = np.zeros(n, np.int32)
     _lib.check(L.odam_sq_oriented_boxes_of_points_host(_lib.ptr(pts), n, n_pts, _lib.ptr(corners), _lib.ptr(flags), device))
@@ -256,9 +278,9 @@ def merge_cost_host(boxes, cls=None, device=0, want_iou=False):
     ids or None -> cost [n,n] float64 (1 - IoU3D where the classes allow a merge, else 1; symmetric, zero diagonal).
     want_iou: also the raw (iou3d, iou2d) matrices for i < j."""
     L = _lib.load()
-    b = np.ascontiguousarray(boxes, np.float64).reshape(-1, 8, 3)
-    n = b.shape[0]
-    c = None if cls is None else np.ascontiguousarray(cls, np.int32).reshape(n)
+    b = _lib.host_array("boxes", boxes, np.float64, (-1, 8, 3))
+    n = len(b)
+    c = _lib.host_array("cls", cls, np.int32, (n,))
     cost = np.zeros((n, n), np.float64)
     i3 = np.zeros((n, n), np.float64) if want_iou else None
     i2 = np.zeros((n, n), np.float64) if want_iou else None
@@ -273,26 +295,34 @@ class DeviceTracks:
         import torch
         self.torch = torch
         self.device = torch.device(device)
-        t = lambda a, dt: torch.from_numpy(np.ascontiguousarray(a, dt)).to(self.device)
+        init, cls, self.view_off_host, Ms, box, mask = _track_arrays(tracks)
+        prior = _lib.host_array("prior", prior, np.float32, (8, 9))
+        t = lambda a: None if a is None else torch.from_numpy(a).to(self.device)
         self.n, self.total_views = tracks.n, tracks.total_views
-        self.view_off_host = np.ascontiguousarray(tracks.view_off, np.int32)
-        self.init, self.cls = t(tracks.init, np.float32), t(tracks.cls, np.int32)
-        self.view_off, self.Ms = t(tracks.view_off, np.int32), t(tracks.Ms, np.float32)
-        self.box, self.mask = t(tracks.box, np.float32), t(tracks.mask, np.uint8)
-        self.prior = None if prior is None else t(prior, np.float32)
+        self.init, self.cls, self.view_off, self.Ms = t(init), t(cls), t(self.view_off_host), t(Ms)
+        self.box, self.mask, self.prior = t(box), t(mask), t(prior)
 
 
 def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr_shape=0.1, threads=0,
                     max_slices=0, out=None, cycles=None, cluster=0, code_layout=0, corners=None):
     """Enqueue one fused launch on torch's current stream; returns dict of CUDA tensors (no sync).
+    out: the dict of a previous call with the same n and n_iters, to be written again.
+    cycles: optional int64 CUDA tensor [n, 16], per-phase SM cycles (diagnostics; slot names in tools/prof_run.py).
     corners: optional float64 CUDA tensor [n, 8, 3] -- the oriented boxes of the optimised objects, from a second launch
     enqueued right behind the optimiser (odam_sq_options.out_corners)."""
     torch = dt.torch
-    L = _lib.load()
+    dev = dt.init.device   # the tracks' device, with its index
+    shapes = dict(params=(torch.float32, (dt.n, 9)), loss=(torch.float32, (dt.n, n_iters)), status=(torch.int32, (dt.n,)))
     if out is None:
-        out = dict(params=torch.empty((dt.n, 9), dtype=torch.float32, device=dt.device),
-                   loss=torch.empty((dt.n, n_iters), dtype=torch.float32, device=dt.device),
-                   status=torch.empty((dt.n,), dtype=torch.int32, device=dt.device))
+        out = {k: torch.empty(shape, dtype=dtype, device=dev) for k, (dtype, shape) in shapes.items()}
+    else:
+        for k, (dtype, shape) in shapes.items():
+            _lib.check_tensor(f"out[{k!r}]", out[k], dtype, shape, dev)
+    if cycles is not None:
+        _lib.check_tensor("cycles", cycles, torch.int64, (dt.n, 16), dev)
+    if corners is not None:
+        _lib.check_tensor("corners", corners, torch.float64, (dt.n, 8, 3), dev)
+        out["corners"] = corners
     o = _lib.Options()
     if threads == 0 or cluster == 0 or code_layout == 0:
         # choose on the host from the host copy of view_off (avoids the library's D2H read-back)
@@ -300,23 +330,13 @@ def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr
         threads, cluster, code_layout, max_slices = q["threads"], q["cluster"], q["code_layout"], q["max_slices"]
     o.threads, o.max_slices, o.cluster, o.code_layout = int(threads), int(max_slices), int(cluster), int(code_layout)
     o.max_views = int(np.diff(dt.view_off_host).max()) if dt.n else 0
-    if cycles is not None:  # int64 CUDA tensor [n, 16]: per-phase SM cycles (diagnostics; slot names in tools/prof_run.py)
-        if tuple(cycles.shape) != (dt.n, 16) or cycles.dtype != torch.int64 or not cycles.is_contiguous() \
-                or cycles.device != dt.device:
-            raise ValueError("cycles must be a contiguous int64 CUDA tensor of shape [n, 16] on the tracks' device")
-        o.out_cycles = cycles.data_ptr()
-    if corners is not None:
-        if tuple(corners.shape) != (dt.n, 8, 3) or corners.dtype != torch.float64 or not corners.is_contiguous() \
-                or corners.device != dt.device:
-            raise ValueError("corners must be a contiguous float64 CUDA tensor of shape [n, 8, 3] on the tracks' device")
-        o.out_corners = corners.data_ptr()
-        out["corners"] = corners
-    p = lambda x: None if x is None else C.c_void_p(x.data_ptr())
-    with torch.cuda.device(dt.device):
-        stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        rc = L.odam_sq_optimize(p(dt.init), p(dt.cls), p(dt.view_off), p(dt.Ms), p(dt.box), p(dt.mask), p(dt.prior),
-                                dt.n, n_iters, _lib.REPR[representation], lr, lr_shape,
-                                p(out["params"]), p(out["loss"]), p(out["status"]), C.byref(o), stream)
+    p = _lib.tensor_ptr
+    o.out_cycles, o.out_corners = p(cycles), p(corners)
+    with torch.cuda.device(dev):
+        rc = _lib.load().odam_sq_optimize(p(dt.init), p(dt.cls), p(dt.view_off), p(dt.Ms), p(dt.box), p(dt.mask),
+                                          p(dt.prior), dt.n, n_iters, _lib.REPR[representation], lr, lr_shape,
+                                          p(out["params"]), p(out["loss"]), p(out["status"]), C.byref(o),
+                                          _lib.current_stream(dev))
     _lib.check(rc)
     return out
 

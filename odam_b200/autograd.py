@@ -29,22 +29,13 @@ gathered per frame, Ms = P[frame_idx] (run_multi_view.stage_tracks returns frame
 sums with atomics and is bit-reproducible only under torch.use_deterministic_algorithms(True).  dL/dMs itself is
 deterministic either way.
 """
-import ctypes as C
-
 import torch
 from torch.autograd.function import once_differentiable
 
 from . import _lib
 
 N_SAMPLES = _lib.N_SAMPLES
-
-
-def _stream(device):
-    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-
-
-def _p(t):
-    return C.c_void_p(t.data_ptr())
+_p, _stream = _lib.tensor_ptr, _lib.current_stream
 
 
 def _check_params(params):
@@ -146,7 +137,7 @@ class _BoxSides(torch.autograd.Function):
             with torch.cuda.device(params.device):
                 if cams:
                     _lib.check(L.odam_sq_box_sides_vjp_cameras(_p(params), _p(view_off), _p(Ms), _p(arg), _p(g), n, SV,
-                                                               None if grad is None else _p(grad), _p(grad_Ms),
+                                                               _p(grad), _p(grad_Ms),
                                                                _stream(params.device)))
                 else:
                     _lib.check(L.odam_sq_box_sides_vjp(_p(params), _p(view_off), _p(Ms), _p(arg), _p(g), n, SV,

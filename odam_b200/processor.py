@@ -15,16 +15,16 @@ from . import api
 
 
 def track_quadric_params(tracks):
-    """[n, 9] C-ABI parameters (t3, yaw, sqrt(dim/2) x3, h2 = 0) of the mean-pose quadric of every track
+    """[n, 9] C-ABI parameters (api.init_params, shape logits 0) of the mean-pose quadric of every track
     (processor.py:191-196); tracks = list of [rows, 82] arrays, columns 6:9 dims, 9:12 centre, 12 yaw."""
-    P = np.zeros((len(tracks), 9), np.float32)
-    for i, track in enumerate(tracks):
+    n = len(tracks)
+    t_wo, azi_wo, dimensions = np.zeros((n, 3)), np.zeros(n), np.zeros((n, 3))
+    for i, track in enumerate(tracks):   # the reference's own per-track np.mean calls, for its float64 rounding
         track = np.asarray(track)
-        azi_wo = np.mean(track[:, 12], axis=0)
-        t_wo = np.mean(track[:, 9: 12], axis=0)
-        dimensions = np.clip(np.mean(track[:, 6: 9], axis=0), a_min=0.05, a_max=np.inf)
-        P[i] = api.init_params(t_wo, azi_wo, dimensions)   # float64 -> float32 as SuperQuadric.__init__ does (torch.tensor)
-    return P
+        azi_wo[i] = np.mean(track[:, 12], axis=0)
+        t_wo[i] = np.mean(track[:, 9: 12], axis=0)
+        dimensions[i] = np.clip(np.mean(track[:, 6: 9], axis=0), a_min=0.05, a_max=np.inf)
+    return api.init_params(t_wo, azi_wo, dimensions)   # float64 -> float32 as SuperQuadric.__init__ does (torch.tensor)
 
 
 def project_points_reference_way(pts, T_wc, K):

@@ -26,19 +26,6 @@ from .sq_libs import SuperQuadric
 EDGE_THRESHOLD = 20  # tracking_gt_utils.py:199
 
 
-def bbox_to_lines(bbox, img_size, edge_threshold=EDGE_THRESHOLD):
-    """{side: homogeneous line} for the sides farther than edge_threshold from the image border
-    (reference src/super_quadric/quadric_helper.py:69-109).  bbox = [[x_min, y_min], [x_max, y_max]]."""
-    img_h, img_w = img_size
-    (x_min, y_min), (x_max, y_max) = bbox
-    lines = {}
-    for name, value, hi in (("x_min", x_min, img_w), ("y_min", y_min, img_h), ("x_max", x_max, img_w),
-                            ("y_max", y_max, img_h)):
-        if edge_threshold < value < hi - edge_threshold:
-            lines[name] = np.array([1, 0, -value]) if name[0] == "x" else np.array([0, 1, -value])
-    return lines
-
-
 def mean_yaw(yaw):
     """Chordal L2 mean of rotations about z -- what ``averaging_T_wos`` (tracking_gt_utils.py:59-66) gets from scipy's
     ``Rotation.from_matrix(...).mean()`` followed by ``as_euler("zxy")[0]`` (run_multi_view.py:57): for quaternions
@@ -146,9 +133,7 @@ def stage_tracks_numpy(tracks, frame_ids, img_h, img_w):
 
 def lines_of(stage):
     """The reference's list-of-dicts form of a staged object's boxes (for SuperQuadricOptimizer.run)."""
-    names = ("x_min", "x_max", "y_min", "y_max")
-    return [{n: (np.array([1, 0, -float(b[k])]) if n[0] == "x" else np.array([0, 1, -float(b[k])]))
-             for k, n in enumerate(names) if m[k]} for b, m in zip(stage["box"], stage["mask"])]
+    return api.unpack_lines(stage["box"], stage["mask"])
 
 
 def boxes_3d(dims, yaw, centre):
@@ -168,22 +153,16 @@ def optim_process(tracks, img_names, T_wcs, P_cws, img_h, img_w, K, representati
     compatibility (the optimiser only needs P_cws = K @ inv(T_wc)[:3, :], processor.py:311).
     devices: optional list of CUDA device indices -- the eligible objects are then sharded by object across them
     (contiguous blocks balanced by views, odam_b200.sharding), one host thread per device."""
-    assert representation in ("cube", "super_quadric", "quadric")
     n = len(tracks)
     st = stage_tracks(tracks, img_names, img_h, img_w)
     bboxes_dl = boxes_3d(st["dims"], st["yaw"], st["t_wo"])
-    init = np.empty((n, 9), np.float32)
-    init[:, 0:3] = st["t_wo"]
-    init[:, 3] = st["yaw"]
-    init[:, 4:7] = np.sqrt(st["dims"] / 2)
-    init[:, 7:9] = -10000.0 if representation == "cube" else -0.0
+    init = api.init_params(st["t_wo"], st["yaw"], st["dims"], representation)
     views = np.diff(st["view_off"])
     run = np.nonzero(views >= n_views)[0]                       # :59-62 eligibility
     params = init.copy()
     bboxes_qc = bboxes_dl.copy()
-    if prior and n and (st["cls"].min() < 0 or st["cls"].max() > 7):
-        bad = st["cls"][(st["cls"] < 0) | (st["cls"] > 7)][0]
-        raise KeyError(int(bad))                                # the reference's CLASS_MAPPER lookup fails the same way
+    if prior:
+        api.check_classes(st["cls"])                            # every track's, eligible or not
     if run.size:
         sel = np.nonzero(np.repeat(views >= n_views, views))[0]        # the packed views of the eligible objects
         P32 = np.ascontiguousarray(np.asarray(P_cws, np.float64).reshape(-1, 12)[st["frame_idx"][sel]], np.float32)
@@ -197,10 +176,7 @@ def optim_process(tracks, img_names, T_wcs, P_cws, img_h, img_w, K, representati
         else:
             out = api.optimize_host(packed, prior=table, n_iters=n_iters, representation=representation, device=device,
                                     extras=("out_corners", "out_box_flag"))   # :66-67 fused behind the optimiser
-        bad = np.nonzero(out["status"] & _lib.ST_NONFINITE)[0]
-        if bad.size:
-            raise RuntimeError(f"superquadric optimisation produced NaN/Inf for object(s) {run[bad].tolist()} "
-                               "(the reference raises from torch anomaly mode, sq_libs.py:456)")
+        api.check_finite(out["status"], run)
         params[run] = out["params"]
         corners = out.get("out_corners")
         if corners is None:   # sharded over several devices: one more launch for all surfaces + oriented boxes

@@ -51,7 +51,7 @@ class SuperQuadric:
         p = np.empty(9, np.float32)
         p[0:3] = np.asarray(translate, np.float64)
         p[3] = np.float64(angle)
-        p[4:7] = np.asarray(scales, np.float64)      # sqrt(dim / 2)
+        p[4:7] = np.asarray(scales, np.float64)      # the scales of api.init_params
         p[7:9] = np.asarray(shapes, np.float64)
         self.__dict__["_p"] = p
         self.__dict__["_t"] = {}
@@ -183,12 +183,9 @@ class SuperQuadricOptimizer:
 
     def __init__(self, translate, quat, scales, obj_class, representation, prior):
         # `quat` is the yaw angle (reference run_multi_view.py:57); `scales` are box dimensions (sq_libs.py:361)
-        scales = np.sqrt(np.asarray(scales, np.float64) / 2)
         self.use_prior = prior
-        assert representation in ["cube", "super_quadric", "quadric"]
         self.representation = representation
-        shapes = np.array([-10000., -10000.]) if representation == "cube" else np.array([-0., -0.])
-        self.Q_init = SuperQuadric(translate, quat, scales, shapes=shapes)
+        self.Q_init = SuperQuadric.from_params(api.init_params(translate, quat, scales, representation))
         self.Q_init.obj_class = obj_class
         self.optimizer = _AdamState(representation == "super_quadric")
         # reference sq_libs.py:388-392: ./src/super_quadric/scale_prior relative to the cwd; the packaged export of
@@ -207,15 +204,6 @@ class SuperQuadricOptimizer:
         if len(box) != Ms.shape[0]:
             raise ValueError("one projection matrix per set of lines expected")
         return Ms, box, mask
-
-    def _prior_table(self):
-        if not self.use_prior:
-            return None
-        cls = self.Q_init.obj_class
-        key = CLASS_MAPPER[cls]  # KeyError for an unknown class, as in the reference (sq_libs.py:464)
-        tab = np.zeros((8, 9), np.float32)
-        tab[cls] = self.scale_prior[key].numpy().reshape(9)
-        return tab
 
     def run(self, gt_lines, gt_planes, Ms, n_iters=200):
         """One launch, n_iters Adam steps; returns self.Q_init (same instance, tensors updated in place)."""
@@ -250,8 +238,9 @@ def optimize_batch(optimizers, gt_lines_list, Ms_list, n_iters=200, device=None,
     prior = None
     if o0.use_prior:
         prior = np.zeros((8, 9), np.float32)
-        for o in optimizers:
-            prior[o.Q_init.obj_class] = o._prior_table()[o.Q_init.obj_class]
+        for o in optimizers:   # KeyError for an unknown class, as in the reference (sq_libs.py:464)
+            c = o.Q_init.obj_class
+            prior[c] = o.scale_prior[CLASS_MAPPER[c]].numpy().reshape(9)
     tracks = api.PackedTracks(init=np.stack([o.Q_init.params() for o in optimizers]),
                               cls=np.array([o.Q_init.obj_class if o.use_prior else 0 for o in optimizers], np.int32),
                               view_off=np.array(off, np.int32), Ms=np.concatenate(Ms), box=np.concatenate(box),
@@ -264,13 +253,10 @@ def optimize_batch(optimizers, gt_lines_list, Ms_list, n_iters=200, device=None,
         m0=np.stack([o.optimizer.exp_avg for o in optimizers]) if continuing else None,
         v0=np.stack([o.optimizer.exp_avg_sq for o in optimizers]) if continuing else None,
         step0=o0.optimizer.step, extras=("out_m", "out_v") + (("out_param_hist",) if want_history else ()))
-    bad = np.nonzero(out["status"] & _lib.ST_NONFINITE)[0]
     for i, o in enumerate(optimizers):
         o.Q_init._set_params(out["params"][i])
         o.optimizer.exp_avg, o.optimizer.exp_avg_sq = out["out_m"][i].copy(), out["out_v"][i].copy()
         o.optimizer.step += n_iters
         o.loss_log.extend_values(out["loss"][i])   # read back as a list of 1-element [tensor] lists, as :471
-    if bad.size:
-        raise RuntimeError(f"superquadric optimisation produced NaN/Inf for object(s) {bad.tolist()} "
-                           "(the reference raises from torch anomaly mode, sq_libs.py:456)")
+    api.check_finite(out["status"])
     return [out["out_param_hist"][i] for i in range(len(optimizers))] if want_history else []

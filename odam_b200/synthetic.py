@@ -20,10 +20,11 @@ from dataclasses import dataclass
 import numpy as np
 import torch
 
+from .api import SIDES, unpack_lines  # noqa: F401  (SIDES: the order of the last axis of box and mask)
+
 IMG_W, IMG_H = 1296, 968
 K = np.array([[1170.0, 0.0, 648.0], [0.0, 1170.0, 484.0], [0.0, 0.0, 1.0]])
 EDGE = 20.0
-SIDES = ("x_min", "x_max", "y_min", "y_max")
 
 
 @dataclass
@@ -31,7 +32,7 @@ class Scene:
     """n objects x V views each, in the layout the C-ABI takes (include/odam_sq.h)."""
     translate: np.ndarray   # [n,3] f64  initial centre (averaged detector output)
     angle: np.ndarray       # [n]   f64  initial yaw
-    dims: np.ndarray        # [n,3] f64  initial 3-D box dimensions (NOT sqrt(dim/2))
+    dims: np.ndarray        # [n,3] f64  initial 3-D box dimensions (NOT api.init_params' scales)
     cls: np.ndarray         # [n]   i32  class id 0..7
     P_cws: np.ndarray       # [n,V,3,4] f64 projection matrices
     box: np.ndarray         # [n,V,4] f64 detected sides in SIDES order, pixels
@@ -48,15 +49,7 @@ class Scene:
 
     def gt_lines(self, i):
         """Object i's detections in the reference's list-of-dicts form (quadric_helper.py:69-109)."""
-        out = []
-        for v in range(self.V):
-            d = {}
-            for s, name in enumerate(SIDES):
-                if self.mask[i, v, s]:
-                    val = self.box[i, v, s]
-                    d[name] = np.array([1, 0, -val]) if name[0] == "x" else np.array([0, 1, -val])
-            out.append(d)
-        return out
+        return unpack_lines(self.box[i], self.mask[i])
 
 
 def _lattice(n_eta=48, n_omega=96):

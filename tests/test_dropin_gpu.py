@@ -14,9 +14,8 @@ pytestmark = pytest.mark.gpu
 
 
 def _lines(box, mask):
-    names = ("x_min", "x_max", "y_min", "y_max")
-    return [{n: (np.array([1, 0, -float(box[v, s])]) if n[0] == "x" else np.array([0, 1, -float(box[v, s])]))
-             for s, n in enumerate(names) if mask[v, s]} for v in range(len(box))]
+    from odam_b200.api import unpack_lines
+    return unpack_lines(box, mask)
 
 
 def test_run_matches_reference_first_iterations(golden_runs):
