@@ -6,7 +6,8 @@ import os
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# ODAM_SQ_LIB selects another build of the same library (A/B timing of kernel variants, tools/ab_build.sh)
+# ODAM_SQ_LIB selects another build of the same library (A/B timing of source trees: each built with
+# `python -m odam_b200.build --force --out odam_b200/lib/ab/libodam_sq_<name>.so`, then tools/ab_run.sh <name>...)
 LIB_PATH = os.environ.get("ODAM_SQ_LIB") or os.path.join(HERE, "lib", "libodam_sq.so")
 
 REPR = {"super_quadric": 0, "cube": 1, "quadric": 2}

@@ -1,10 +1,13 @@
 """Build odam_b200/lib/libodam_sq.so (hand-written sm_100a CUDA + the C ABI of include/odam_sq.h).
 
-    python -m odam_b200.build [--force] [--verbose]
+    python -m odam_b200.build [--force] [--verbose] [--out PATH]
 
+--out writes the library elsewhere with the same flags, e.g. one build per source tree for A/B timing
+(odam_b200/lib/ab/libodam_sq_<name>.so, run by tools/ab_run.sh <name>).
 nvcc cross-compiles without a GPU.  -fmad=false: the sampler restates the reference's fp32 rounding
 sequence, so every fused multiply-add in the kernels is written explicitly (__fmaf_rn).
 """
+import argparse
 import os
 import subprocess
 import sys
@@ -19,26 +22,31 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
               "-Xptxas", "-regUsageLevel=10", "-Xcompiler", "-fPIC", "-shared"]
 
 
-def needs_build():
-    if not os.path.exists(OUT):
+def needs_build(out=OUT):
+    if not os.path.exists(out):
         return True
-    t = os.path.getmtime(OUT)
+    t = os.path.getmtime(out)
     return any(os.path.getmtime(d) > t for d in DEPS)
 
 
-def build(force=False, verbose=False):
-    if not force and not needs_build():
-        return OUT
-    os.makedirs(os.path.dirname(OUT), exist_ok=True)
+def build(force=False, verbose=False, out=OUT):
+    if not force and not needs_build(out):
+        return out
+    os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", OUT] + SRC
+    cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", out] + SRC
     r = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or r.returncode:
         sys.stderr.write(r.stdout + r.stderr)
     if r.returncode:
-        raise RuntimeError("nvcc failed building libodam_sq.so")
-    return OUT
+        raise RuntimeError(f"nvcc failed building {out}")
+    return out
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv))
+    ap = argparse.ArgumentParser(prog="python -m odam_b200.build")
+    ap.add_argument("--force", action="store_true", help="rebuild even when the library is newer than its sources")
+    ap.add_argument("--verbose", action="store_true", help="print nvcc's output, with ptxas resource usage")
+    ap.add_argument("--out", default=OUT, help="library to write (default: %(default)s)")
+    a = ap.parse_args()
+    print(build(force=a.force, verbose=a.verbose, out=a.out))

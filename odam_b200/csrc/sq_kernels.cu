@@ -25,9 +25,6 @@
 
 #include "../../include/odam_sq.h"
 
-#ifndef SQ_FFMA2
-#define SQ_FFMA2 1   // phase E on packed fp32 pairs (FFMA2/FMUL2); 0 = scalar FFMA build for A/B timing
-#endif
 #include "sq_device.cuh"
 #include "sq_postproc.cuh"
 #include "sq_stage.h"
@@ -286,15 +283,8 @@ __device__ __forceinline__ void scan_item(const Smem &S, const float (&M)[12], i
 #pragma unroll
             for (int h = 0; h < kGroup / 4; h++) {
                 float4 x = xs[h], y = ys[h], z = zs[h];
-#if SQ_FFMA2
                 project_uv2<kCheck>(M, x.x, x.y, y.x, y.y, z.x, z.y, u[4 * h + 0], u[4 * h + 1], w[4 * h + 0], w[4 * h + 1]);
                 project_uv2<kCheck>(M, x.z, x.w, y.z, y.w, z.z, z.w, u[4 * h + 2], u[4 * h + 3], w[4 * h + 2], w[4 * h + 3]);
-#else
-                project_uv<kCheck>(M, x.x, y.x, z.x, u[4 * h + 0], w[4 * h + 0]);
-                project_uv<kCheck>(M, x.y, y.y, z.y, u[4 * h + 1], w[4 * h + 1]);
-                project_uv<kCheck>(M, x.z, y.z, z.z, u[4 * h + 2], w[4 * h + 2]);
-                project_uv<kCheck>(M, x.w, y.w, z.w, u[4 * h + 3], w[4 * h + 3]);
-#endif
             }
 #pragma unroll
             for (int h = 0; h < kGroup; h += 2) {
@@ -324,8 +314,9 @@ __device__ __forceinline__ void load_M2(const float *Ms, int gv, int row, float 
     Mz[0] = z.x; Mz[1] = z.y; Mz[2] = z.z; Mz[3] = z.w;
 }
 
-// first point of chunk `c` whose projected coordinate (the same operations as project_uv<true>, for the one image
-// axis this side lives on) equals the extremum `best`
+// first point of chunk `c` whose projected coordinate equals the extremum `best`: one half of project_uv2<true>'s
+// sequence, for the one image axis this side lives on: FMA chains for q and q_z with the 1e-6 folded into M[11]
+// (Mz[3] here), MUFU.RCP of q_z, NaN unless q_z > 0.500001, one rounded product
 __device__ __forceinline__ int resolve_arg(const Smem &S, const float (&Mr)[4], const float (&Mz)[4], int c, float best)
 {
     // Every thread searches its own chunk, so at the same step neighbouring lanes would read addresses 16 words apart
@@ -348,14 +339,11 @@ __device__ __forceinline__ int resolve_arg(const Smem &S, const float (&Mr)[4], 
     return found < kNPad ? found : -1;
 }
 
-#ifndef SQ_COMPACT_BLOCKS
-#define SQ_COMPACT_BLOCKS 4
-#endif
 // Resident CTAs per SM the register allocation aims at: the compact build 4 x 256 threads, the straight-line build 1024
 // threads' worth (64 registers each) -- except kSolo, the build for launches where every CTA has an SM to itself (the
 // latency regime): one 512-thread CTA may then use 128 registers per thread, which removes every spill and most of
 // the rematerialised address arithmetic from the serial phases (+3..6 % there, bit-identical results).
-#define SQ_MIN_BLOCKS(threads, compact, solo) ((compact) ? SQ_COMPACT_BLOCKS : ((solo) ? 1 : 1024 / (threads)))
+constexpr int min_blocks(int threads, bool compact, bool solo) { return compact ? 4 : (solo ? 1 : 1024 / threads); }
 // phase-E work item -> view << 16 | first chunk << 8 | end chunk: item = slice * V + view, the 63 chunks split evenly
 __device__ __forceinline__ unsigned item_code(int item, int V, int slices)
 {
@@ -368,16 +356,12 @@ __device__ __forceinline__ unsigned item_code(int item, int V, int slices)
 // compiled out of the production kernels: a predicate test, a branch and a volatile clock read at 15 places cost
 // 2.6 % (config 2) to 4.8 % (config 5) of the throughput even when no count is taken.
 template <int kMaxThreads, bool kCompact, bool kSolo = false, bool kProf = false>
-__global__ void __launch_bounds__(kMaxThreads, SQ_MIN_BLOCKS(kMaxThreads, kCompact, kSolo)) sq_optimize_kernel(OptArgs A)
+__global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact, kSolo)) sq_optimize_kernel(OptArgs A)
 {
     // fixed state in static shared memory (compile-time addresses), per-launch scratch in dynamic shared memory
     __shared__ Smem S;
     extern __shared__ __align__(16) unsigned char scratch_raw[];
-#ifdef SQ_E_GROUP
-    constexpr int kGroup = SQ_E_GROUP;
-#else
     constexpr int kGroup = kCompact ? 4 : kChunk;
-#endif
     const int tid = threadIdx.x, T = blockDim.x;
     const int warp = tid >> 5, lane = tid & 31, nwarps = T >> 5;
     constexpr bool prof = kProf;
@@ -460,7 +444,7 @@ __global__ void __launch_bounds__(kMaxThreads, SQ_MIN_BLOCKS(kMaxThreads, kCompa
             const int v = code >> 16, c0 = (code >> 8) & 0xff, c1 = code & 0xff;
             float M[12];
             if (staged) load_M<true>(Msrc, v, M); else load_M<false>(Msrc, v, M);
-            M[11] = __fadd_rn(M[11], 1e-6f);  // the reference's |z| + 1e-6, folded (see project_uv)
+            M[11] = __fadd_rn(M[11], 1e-6f);  // the reference's |z| + 1e-6, folded (see project_uv2)
             float best[4];
             int cid[4];
             if (view_all_valid(M, S.pose)) scan_item<false, kGroup>(S, M, c0, c1, best, cid);
@@ -997,7 +981,7 @@ static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, f
 using OptKernel = void (*)(OptArgs);
 
 // The builds of sq_optimize_kernel, each with its cycle-mark twin (prof), in ascending CTA size within each layout.
-// Their register budget follows from __launch_bounds__: SQ_MIN_BLOCKS CTAs of `threads` share the 64K registers.
+// Their register budget follows from __launch_bounds__: min_blocks() CTAs of `threads` share the 64K registers.
 // The compact layout only exists for CTAs of up to 256 threads (it is for many small CTAs per SM).
 struct OptBuild { int threads; bool compact, solo, prof; OptKernel kern; };
 static const OptBuild kOptBuilds[] = {
@@ -1023,7 +1007,7 @@ static const OptBuild *pick_build(int threads, bool compact, bool solo, bool pro
     return nullptr;
 }
 
-static int opt_regs(const OptBuild &B) { return 65536 / (B.threads * SQ_MIN_BLOCKS(B.threads, B.compact, B.solo)); }
+static int opt_regs(const OptBuild &B) { return 65536 / (B.threads * min_blocks(B.threads, B.compact, B.solo)); }
 
 // Dynamic shared memory of each per-object kernel: its launcher asks for this much and ensure_init() sets the kernel's
 // attribute to it (sq_sides_kernel's kSidesSmem is in sq_autograd.cuh)
@@ -1277,10 +1261,7 @@ static int launch_optimize(const OptArgs &A0, const LaunchCfg &L, cudaStream_t s
     OptKernel kern = pick_build(L.threads, L.compact, L.solo, A.out_cycles != nullptr)->kern;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof cfg);
-#ifndef SQ_EXTRA_SMEM
-#define SQ_EXTRA_SMEM 0   // diagnostics: unused dynamic shared memory per CTA, to lower the number of resident CTAs
-#endif
-    cfg.gridDim = dim3(A.n * L.cluster); cfg.blockDim = dim3(L.threads); cfg.dynamicSmemBytes = L.smem + SQ_EXTRA_SMEM; cfg.stream = st;
+    cfg.gridDim = dim3(A.n * L.cluster); cfg.blockDim = dim3(L.threads); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
     cudaLaunchAttribute attr;
     attr.id = cudaLaunchAttributeClusterDimension;
     attr.val.clusterDim.x = L.cluster; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;

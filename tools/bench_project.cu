@@ -5,6 +5,15 @@
 #include "sq_device.cuh"
 using namespace odam;
 
+__device__ __forceinline__ void proj_valid(const float (&M)[12], float X, float Y, float Z, float &u, float &w)
+{
+    float qx = __fmaf_rn(X, M[0], __fmaf_rn(Y, M[1], __fmaf_rn(Z, M[2], M[3])));
+    float qy = __fmaf_rn(X, M[4], __fmaf_rn(Y, M[5], __fmaf_rn(Z, M[6], M[7])));
+    float qz = __fmaf_rn(X, M[8], __fmaf_rn(Y, M[9], __fmaf_rn(Z, M[10], M[11])));
+    float r = rcp_approx(__fadd_rn(fabsf(qz), 1e-6f));
+    r = qz > 0.5f ? r : __int_as_float(0x7fc00000);
+    u = __fmul_rn(qx, r); w = __fmul_rn(qy, r);
+}
 __device__ __forceinline__ void proj_novalid(const float (&M)[12], float X, float Y, float Z, float &u, float &w)
 {
     float qx = __fmaf_rn(X, M[0], __fmaf_rn(Y, M[1], __fmaf_rn(Z, M[2], M[3])));
@@ -50,7 +59,7 @@ __global__ void __launch_bounds__(512, 2) k(const float *Ms, float *out, int rep
                 float4 x = reinterpret_cast<const float4 *>(px + c * CH)[h], y = reinterpret_cast<const float4 *>(py + c * CH)[h],
                        z = reinterpret_cast<const float4 *>(pz + c * CH)[h];
 #define P(a, i)                                                                     \
-    if (VAR == 0) project_uv(M, x.a, y.a, z.a, u[4 * h + i], w[4 * h + i]);          \
+    if (VAR == 0) proj_valid(M, x.a, y.a, z.a, u[4 * h + i], w[4 * h + i]);          \
     else if (VAR == 1) proj_novalid(M, x.a, y.a, z.a, u[4 * h + i], w[4 * h + i]);   \
     else if (VAR == 5) proj_folded_valid(M, x.a, y.a, z.a, u[4 * h + i], w[4 * h + i]); \
     else proj_folded(M, x.a, y.a, z.a, u[4 * h + i], w[4 * h + i]);
@@ -80,7 +89,7 @@ int main()
     for (int v = 0; v < 50; v++) { float m[12] = {1170, 0, 648, 100 + v, 0, 1170, 484, 50, 0, 0, 1, 3.0f + 0.01f * v}; for (int k2 = 0; k2 < 12; k2++) hM[v * 12 + k2] = m[k2]; }
     float *dM, *out; cudaMalloc(&dM, sizeof hM); cudaMalloc(&out, 4 * 148 * 4 * 512); cudaMemcpy(dM, hM, sizeof hM, cudaMemcpyHostToDevice);
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
-    const char *names[] = {"V0 current", "V1 no validity", "V2 no validity + folded eps", "V3 = V2 with 2-input min/max", "V4 = V2 with 16-point chunks", "V5 folded eps + validity"};
+    const char *names[] = {"V0 validity", "V1 no validity", "V2 no validity + folded eps", "V3 = V2 with 2-input min/max", "V4 = V2 with 16-point chunks", "V5 folded eps + validity"};
     for (int threads = 256; threads <= 512; threads *= 2)
     for (int var = 0; var < 6; var++) {
         int reps = 20, blocks = 148 * (1024 / threads);

@@ -7,6 +7,17 @@
 #include "sq_device.cuh"
 using namespace odam;
 
+// scalar FFMA form of project_uv2<false>, one point per call
+__device__ __forceinline__ void project_scalar(const float (&M)[12], float X, float Y, float Z, float &u, float &w)
+{
+    float qx = __fmaf_rn(X, M[0], __fmaf_rn(Y, M[1], __fmaf_rn(Z, M[2], M[3])));
+    float qy = __fmaf_rn(X, M[4], __fmaf_rn(Y, M[5], __fmaf_rn(Z, M[6], M[7])));
+    float qz = __fmaf_rn(X, M[8], __fmaf_rn(Y, M[9], __fmaf_rn(Z, M[10], M[11])));
+    float r = rcp_approx(qz);
+    u = __fmul_rn(qx, r);
+    w = __fmul_rn(qy, r);
+}
+
 template <bool PACKED>
 __device__ __forceinline__ void proj4(const float (&M)[12], const float4 x, const float4 y, const float4 z, float (&u)[4], float (&w)[4])
 {
@@ -14,10 +25,10 @@ __device__ __forceinline__ void proj4(const float (&M)[12], const float4 x, cons
         project_uv2<false>(M, x.x, x.y, y.x, y.y, z.x, z.y, u[0], u[1], w[0], w[1]);
         project_uv2<false>(M, x.z, x.w, y.z, y.w, z.z, z.w, u[2], u[3], w[2], w[3]);
     } else {
-        project_uv<false>(M, x.x, y.x, z.x, u[0], w[0]);
-        project_uv<false>(M, x.y, y.y, z.y, u[1], w[1]);
-        project_uv<false>(M, x.z, y.z, z.z, u[2], w[2]);
-        project_uv<false>(M, x.w, y.w, z.w, u[3], w[3]);
+        project_scalar(M, x.x, y.x, z.x, u[0], w[0]);
+        project_scalar(M, x.y, y.y, z.y, u[1], w[1]);
+        project_scalar(M, x.z, y.z, z.z, u[2], w[2]);
+        project_scalar(M, x.w, y.w, z.w, u[3], w[3]);
     }
 }
 
