@@ -12,9 +12,10 @@ import numpy as np
 import pytest
 
 from golden_cases import EDGE_KINDS, FLOOR, TOL_LOSS, TOL_PARAM, all_cases, edge_object, rel_loss, rel_param, wide_cases
+from launch_checks import EXTRAS, TAU_KERNEL, check_decisions, pack
 from oracle import grad64 as G64
 from surface_vjp64 import surface_vjp64
-from test_backward_gpu import EXTRAS, TAU_KERNEL, _check_decisions, _pack, _ragged_tracks
+from test_backward_gpu import _ragged_tracks
 
 pytestmark = pytest.mark.gpu
 
@@ -60,7 +61,7 @@ def _with_repr(tracks, representation):
 
 
 def _edge_tracks(representation="super_quadric"):
-    return _with_repr(_pack([edge_object(k) for k in EDGE_KINDS]), representation)
+    return _with_repr(pack([edge_object(k) for k in EDGE_KINDS]), representation)
 
 
 def _long_tracks(api, V):
@@ -133,7 +134,7 @@ def test_box_sides_decisions(api, AG, batch):
     for i in range(tr.n):
         a, b = int(tr.view_off[i]), int(tr.view_off[i + 1])
         etas, omegas = G64.angles(o["out_grids"][i], o["out_eta_idx"][i])
-        _check_decisions(tr.init[i], etas, omegas, tr.Ms[a:b], pred[a:b], arg[a:b], (batch, i))
+        check_decisions(tr.init[i], etas, omegas, tr.Ms[a:b], pred[a:b], arg[a:b], (batch, i))
         _check_sentinels(tr.init[i], etas, omegas, tr.Ms[a:b], pred[a:b], arg[a:b], (batch, i))
     print(f"  box_sides {batch}: {tr.total_views} views, {int((arg < 0).sum())} sentinel sides, decisions legitimate")
 

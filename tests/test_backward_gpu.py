@@ -17,15 +17,10 @@ import numpy as np
 import pytest
 
 from golden_cases import EDGE_KINDS, all_cases, edge_object, wide_cases
+from launch_checks import EXTRAS, TAU_KERNEL, check_launch, pack
 from oracle import grad64 as G64
 
 pytestmark = pytest.mark.gpu
-
-# About 10x the reference's own measured error (5.4e-7, tests/test_backward_ref.py) and ~34 eps32: the kernel sums the
-# same terms in another order (warp butterfly, warps, cluster ranks).
-TAU_KERNEL = 4e-6
-EXTRAS = ("out_grad", "out_m", "out_v", "out_grids", "out_eta_idx", "out_arg", "out_pred", "out_param_hist")
-BBOX_RTOL, BBOX_ATOL = 2e-6, 2e-3   # test_get_bbox_csr_many_objects: float64 get_bbox of the kernel's own points
 
 
 @pytest.fixture(scope="module")
@@ -39,58 +34,6 @@ def _wall_time():
     t0 = time.time()
     yield
     print(f"\ntests/test_backward_gpu.py wall time {time.time() - t0:.1f} s")
-
-
-def _pack(objs):
-    """[(init, Ms, box, mask, cls)] -> PackedTracks."""
-    from odam_b200.api import PackedTracks
-    off = np.concatenate([[0], np.cumsum([len(o[1]) for o in objs])]).astype(np.int32)
-    return PackedTracks(np.stack([o[0] for o in objs]).astype(np.float32), np.array([o[4] for o in objs], np.int32), off,
-                        np.concatenate([o[1] for o in objs]).astype(np.float32),
-                        np.concatenate([o[2] for o in objs]).astype(np.float32),
-                        np.concatenate([o[3] for o in objs]).astype(np.uint8))
-
-
-def _check_decisions(state, etas, omegas, Ms, pred, arg, label):
-    """pred = float64 projection of the arg point = float64 extremum over every valid point (up to near-ties)."""
-    u, w, valid = G64.project(state, etas, omegas, Ms)
-    V = len(Ms)
-    tol = lambda x: BBOX_ATOL + BBOX_RTOL * np.abs(x)
-    for sd in range(4):
-        c = u if sd < 2 else w
-        big = np.where(valid, c, np.inf if sd % 2 == 0 else -np.inf)
-        ext = big.min(1) if sd % 2 == 0 else big.max(1)
-        has = arg[:, sd] >= 0
-        at = c[np.arange(V), np.maximum(arg[:, sd], 0)]
-        assert (np.abs(pred[has, sd] - at[has]) <= tol(at[has])).all(), (label, sd, "pred != projection of arg point")
-        assert valid[np.arange(V), np.maximum(arg[:, sd], 0)][has].all(), (label, sd, "arg point not valid")
-        assert (np.abs(pred[has, sd] - ext[has]) <= tol(ext[has])).all(), (label, sd, "arg point is not the extremum")
-        assert (np.abs(pred[~has, sd]) == 1e6).all(), (label, sd, "no valid point but no sentinel")
-
-
-def _check_launch(api, tracks, prior=None, n_iters=1, representation="super_quadric", label="", **kw):
-    """One launch with every diagnostic output; the last iteration's gradient of every object against float64 under
-    the kernel's own decisions; prints the worst ratio per component."""
-    o = api.optimize_host(tracks, prior=prior, n_iters=n_iters, representation=representation, extras=EXTRAS, **kw)
-    opt = representation == "super_quadric"
-    nc = 9 if opt else 7
-    worst = np.zeros(9)
-    for i in range(tracks.n):
-        a, b = int(tracks.view_off[i]), int(tracks.view_off[i + 1])
-        state = tracks.init[i] if n_iters == 1 else o["out_param_hist"][i, -2]
-        etas, omegas = G64.angles(o["out_grids"][i], o["out_eta_idx"][i])
-        Ms, box, mask = tracks.Ms[a:b], tracks.box[a:b], tracks.mask[a:b]
-        pred, arg = o["out_pred"][a:b], o["out_arg"][a:b]
-        if b > a:
-            _check_decisions(state, etas, omegas, Ms, pred, arg, (label, i))
-        p33 = None if prior is None else prior[tracks.cls[i]].reshape(3, 3)
-        g, sc = G64.grad64(state, Ms, box, mask, etas, omegas, arg, np.sign(pred - box), p33, tracks.init[i][4:7], opt)
-        r = G64.ratio(o["out_grad"][i][:nc], g[:nc], sc[:nc])
-        assert (r <= TAU_KERNEL).all(), (label, i, b - a, r, o["out_grad"][i], g)
-        if not opt:
-            assert (o["out_grad"][i][7:9] == 0).all(), (label, i)
-        worst[:nc] = np.maximum(worst[:nc], r)
-    print(f"  {label}: worst |g - g64| / scale " + " ".join(f"{x:.1e}" for x in worst))
 
 
 def _ragged_tracks(api):
@@ -109,7 +52,7 @@ def _ragged_tracks(api):
         if i == 7:
             m[:] = 0
         objs.append((init_params(scene.translate[i], scene.angle[i], scene.dims[i]), M, scene.box[i][:V], m, scene.cls[i]))
-    return _pack(objs)
+    return pack(objs)
 
 
 @pytest.mark.parametrize("n_iters", [1, 5])
@@ -118,7 +61,7 @@ def test_gradient_ragged_batch_every_cta_size(api, n_iters):
     tracks, prior = _ragged_tracks(api), api.prior_table()
     for threads in (64, 128, 256, 512, 1024):
         for layout in ((1, 2) if threads <= 256 else (1,)):
-            _check_launch(api, tracks, prior, n_iters, label=f"ragged threads={threads} layout={layout} iters={n_iters}",
+            check_launch(api, tracks, prior, n_iters, label=f"ragged threads={threads} layout={layout} iters={n_iters}",
                           threads=threads, code_layout=layout)
 
 
@@ -128,10 +71,10 @@ def test_gradient_view_tiled_clusters(api):
     from odam_b200.api import init_params
     Vs = [50, 37, 3, 2, 64]
     sc = synthetic.make_scene(len(Vs), 64, seed=13)
-    tracks = _pack([(init_params(sc.translate[i], sc.angle[i], sc.dims[i]), sc.P_cws[i][:V].reshape(V, 12),
+    tracks = pack([(init_params(sc.translate[i], sc.angle[i], sc.dims[i]), sc.P_cws[i][:V].reshape(V, 12),
                      sc.box[i][:V], sc.mask[i][:V], sc.cls[i]) for i, V in enumerate(Vs)])
     for c in (1, 2, 3, 4):
-        _check_launch(api, tracks, api.prior_table(), 4, label=f"cluster={c}", cluster=c)
+        check_launch(api, tracks, api.prior_table(), 4, label=f"cluster={c}", cluster=c)
 
 
 def test_gradient_long_tracks(api):
@@ -140,7 +83,7 @@ def test_gradient_long_tracks(api):
     for V in (1500, 2500):
         tracks = api.pack_scene(synthetic.make_scene(2, V, seed=21))
         for cluster in (0, 1):
-            _check_launch(api, tracks, api.prior_table(), 2, label=f"V={V} cluster={cluster}", cluster=cluster)
+            check_launch(api, tracks, api.prior_table(), 2, label=f"V={V} cluster={cluster}", cluster=cluster)
 
 
 @pytest.mark.parametrize("representation", ["cube", "quadric", "super_quadric"])
@@ -155,10 +98,10 @@ def test_gradient_edge_objects(api, representation):
         elif representation == "quadric":
             init[7:9] = 0.0
         objs.append((init, Ms, box, mask, cls))
-    tracks = _pack(objs)
+    tracks = pack(objs)
     for prior in (api.prior_table(), None):
         for n_iters in (1, 3):
-            _check_launch(api, tracks, prior, n_iters, representation,
+            check_launch(api, tracks, prior, n_iters, representation,
                           label=f"edge objects {representation} prior={prior is not None} iters={n_iters}")
 
 
@@ -167,7 +110,7 @@ def test_gradient_after_200_free_iterations(api):
     iteration's gradient of every object against float64."""
     from odam_b200 import synthetic
     tracks = api.pack_scene(synthetic.make_config(2))
-    _check_launch(api, tracks, api.prior_table(), 200, label="config 2, iteration 200")
+    check_launch(api, tracks, api.prior_table(), 200, label="config 2, iteration 200")
 
 
 def test_gradient_and_moments_vs_reference_records(api, golden_runs, golden_wide):
