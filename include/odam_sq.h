@@ -111,6 +111,31 @@ const char *odam_sq_last_cuda_error(void);
  * onto `device` and sizes the kernels' shared memory.  Idempotent; called lazily by every entry point. */
 int odam_sq_init(int device);
 
+/* Opt-in objective of odam_sq_optimize_objective[_host], for detections noisier than the reference assumes.  Object i
+ * with V views (all of them, as the reference divides) minimises
+ *     sum over sides s and views v of  w[v][s] * mask[v][s] * rho(pred[v][s] - box[v][s]) / V   (+ the prior, unchanged)
+ * with rho one of
+ *     ODAM_SQ_LOSS_L1         |r|  (the reference)
+ *     ODAM_SQ_LOSS_SMOOTH_L1  0.5 r^2 / beta if |r| < beta, else |r| - 0.5 beta  (torch's smooth_l1_loss), beta = loss_scale
+ *     ODAM_SQ_LOSS_CAUCHY     0.5 c^2 log1p((r / c)^2), rho' = r / (1 + (r / c)^2), c = loss_scale
+ * A NaN residual contributes nothing.  Weights are finite and >= 0 and multiply the mask: a side whose w * mask is 0
+ * contributes nothing to the loss or the gradient and never raises ODAM_SQ_ST_NO_VALID_PT, exactly as a masked-out side.
+ * lr_scale[it] (it = 0 .. n_iters-1 of the call) multiplies both learning rates of iteration it, as a torch scheduler
+ * that sets group["lr"] = lr * lr_scale[it]; the bias corrections continue from step0 as before.
+ * The kernel build with weights and robust kinds runs only when side_weight != NULL or loss != L1; a schedule alone runs
+ * the builds of odam_sq_optimize.  The new build has no cycle-mark twin: out_cycles with it is ODAM_SQ_ERR_ARG. */
+#define ODAM_SQ_LOSS_L1 0
+#define ODAM_SQ_LOSS_SMOOTH_L1 1
+#define ODAM_SQ_LOSS_CAUCHY 2
+typedef struct odam_sq_objective {
+    const float *side_weight;  /* [SV][4] per-side weights; NULL = 1.  DEVICE memory for odam_sq_optimize_objective,
+                                  which does not validate them (as for cls); HOST memory for the _host entry, which
+                                  rejects negative or non-finite weights                                          */
+    int loss;                  /* ODAM_SQ_LOSS_*                                                                    */
+    float loss_scale;          /* beta / c in pixels, finite and > 0 for the robust kinds; ignored for L1           */
+    const float *lr_scale;     /* HOST [n_iters] finite, >= 0 multipliers of both learning rates; NULL = constant   */
+} odam_sq_objective;
+
 /* SuperQuadricOptimizer.run for n objects at once (sq_libs.py:432-475).  Device pointers. */
 int odam_sq_optimize(const float *init, const int32_t *cls, const int32_t *view_off,
                      const float *Ms, const float *box, const uint8_t *mask, const float *prior,
@@ -124,6 +149,21 @@ int odam_sq_optimize_host(const float *init, const int32_t *cls, const int32_t *
                           int n, int n_iters, int representation, float lr, float lr_shape,
                           float *out_params, float *out_loss, int32_t *out_status,
                           const odam_sq_options *opt, int device);
+
+/* odam_sq_optimize[_host] with the objective above; obj == NULL is exactly the entry without it.  Besides the checks of
+ * odam_sq_optimize[_host], ODAM_SQ_ERR_ARG (before any CUDA call) for an unknown loss, a robust kind without a finite
+ * loss_scale > 0, a negative or non-finite lr_scale entry, opt->out_cycles with the weighted/robust build, and at the
+ * _host entry a negative or non-finite weight. */
+int odam_sq_optimize_objective(const float *init, const int32_t *cls, const int32_t *view_off,
+                               const float *Ms, const float *box, const uint8_t *mask, const float *prior,
+                               int n, int n_iters, int representation, float lr, float lr_shape,
+                               float *out_params, float *out_loss, int32_t *out_status,
+                               const odam_sq_objective *obj, const odam_sq_options *opt, void *stream);
+int odam_sq_optimize_objective_host(const float *init, const int32_t *cls, const int32_t *view_off,
+                                    const float *Ms, const float *box, const uint8_t *mask, const float *prior,
+                                    int n, int n_iters, int representation, float lr, float lr_shape,
+                                    float *out_params, float *out_loss, int32_t *out_status,
+                                    const odam_sq_objective *obj, const odam_sq_options *opt, int device);
 
 /* compute_ellipsoid_points (sq_libs.py:577-595): params[n][9] -> xyz[n][1000][3] world points. */
 int odam_sq_sample_points(const float *params, int n, float *out_xyz, void *stream);

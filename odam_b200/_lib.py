@@ -26,6 +26,14 @@ class Options(C.Structure):
                 ("out_corners", C.c_void_p), ("out_box_flag", C.c_void_p)]
 
 
+LOSS = {"l1": 0, "smooth_l1": 1, "cauchy": 2}   # ODAM_SQ_LOSS_*
+
+
+class Objective(C.Structure):
+    """odam_sq_objective (include/odam_sq.h)."""
+    _fields_ = [("side_weight", C.c_void_p), ("loss", C.c_int), ("loss_scale", C.c_float), ("lr_scale", C.c_void_p)]
+
+
 class OdamSqError(RuntimeError):
     pass
 
@@ -40,6 +48,8 @@ ARGTYPES = {
     "odam_sq_init": [_ci],
     "odam_sq_optimize": _OPT + [_vp],
     "odam_sq_optimize_host": _OPT + [_ci],
+    "odam_sq_optimize_objective": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Options), _vp],
+    "odam_sq_optimize_objective_host": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Options), _ci],
     "odam_sq_sample_points": [_vp, _ci, _vp, _vp],
     "odam_sq_sample_points_host": [_vp, _ci, _vp, _ci],
     "odam_sq_project_boxes": [_vp, _vp, _vp, _ci, _vp, _vp],

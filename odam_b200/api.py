@@ -172,19 +172,44 @@ def _track_arrays(tracks):
             a("mask", tracks.mask, np.uint8, (SV, 4)))
 
 
+def _objective(side_weight, loss, loss_scale, lr_scale, n_iters):
+    """(odam_sq_objective, the schedule array it points into) of the optimiser's objective keywords, or (None, None)
+    when all are at their defaults: then the entry without an objective runs.  side_weight: the pointer the entry
+    reads (host or device memory) or None.  Values are checked by the library (negative or non-finite weights,
+    schedule entries and scales are its ODAM_SQ_ERR_ARG)."""
+    if loss not in _lib.LOSS:
+        raise ValueError(f"loss must be one of {', '.join(_lib.LOSS)}, got {loss!r}")
+    if loss != "l1" and loss_scale is None:
+        raise ValueError(f"loss={loss!r} needs loss_scale (beta or c, in pixels)")
+    sched = _lib.host_array("lr_scale", lr_scale, np.float32, (n_iters,))
+    if side_weight is None and loss == "l1" and sched is None:
+        return None, None
+    obj = _lib.Objective()
+    obj.side_weight, obj.loss, obj.lr_scale = side_weight, _lib.LOSS[loss], _lib.ptr(sched)
+    obj.loss_scale = 0.0 if loss == "l1" else float(loss_scale)
+    return obj, sched
+
+
 def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric", lr=0.01, lr_shape=0.1,
                   device=0, threads=0, max_slices=0, m0=None, v0=None, step0=0, s0=None, extras=(), cluster=0,
-                  code_layout=0):
+                  code_layout=0, side_weight=None, loss="l1", loss_scale=None, lr_scale=None):
     """Run the fused optimiser on packed host arrays.  Returns dict(params[n,9], loss[n,n_iters], status[n], ...extras).
 
     prior: None (no prior term) or an [8,9] float32 table (see prior_table()).
     extras: names of optional outputs of odam_sq_options (out_m, out_v, out_grad, out_pred, out_arg,
             out_eta_idx, out_grids, out_param_hist; out_corners (+ out_box_flag): the oriented boxes of the optimised
             objects, computed by a second launch fused behind the optimiser inside the same call).
+    The objective (odam_sq_objective; all defaults = the reference's masked L1 at a constant step size):
+      side_weight: [SV,4] finite weights >= 0 that multiply the mask (e.g. detector confidences), or None = 1;
+      loss: "l1", "smooth_l1" (torch's smooth_l1_loss, beta = loss_scale) or "cauchy" (0.5 c^2 log1p((r/c)^2),
+            c = loss_scale), loss_scale in pixels;
+      lr_scale: [n_iters] multipliers of both learning rates, one per iteration of this call (a schedule).
     """
     L = _lib.load()
     init, cls, voff, Ms, box, mask = _track_arrays(tracks)
     n, SV = len(init), int(voff[-1])
+    w = _lib.host_array("side_weight", side_weight, np.float32, (SV, 4))
+    obj, _sched = _objective(_lib.ptr(w), loss, loss_scale, lr_scale, n_iters)
     pr = _lib.host_array("prior", prior, np.float32, (8, 9))
     if pr is not None:
         check_classes(cls)
@@ -203,10 +228,13 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
         setattr(o, name, _lib.ptr(arr))
     out = dict(params=np.zeros((n, 9), np.float32), loss=np.zeros((n, n_iters), np.float32),
                status=np.zeros(n, np.int32))
-    rc = L.odam_sq_optimize_host(_lib.ptr(init), _lib.ptr(cls), _lib.ptr(voff), _lib.ptr(Ms), _lib.ptr(box),
-                                 _lib.ptr(mask), _lib.ptr(pr), n, n_iters, _lib.REPR[representation],
-                                 lr, lr_shape, _lib.ptr(out["params"]), _lib.ptr(out["loss"]),
-                                 _lib.ptr(out["status"]), C.byref(o), device)
+    args = (_lib.ptr(init), _lib.ptr(cls), _lib.ptr(voff), _lib.ptr(Ms), _lib.ptr(box), _lib.ptr(mask), _lib.ptr(pr),
+            n, n_iters, _lib.REPR[representation], lr, lr_shape, _lib.ptr(out["params"]), _lib.ptr(out["loss"]),
+            _lib.ptr(out["status"]))
+    if obj is None:
+        rc = L.odam_sq_optimize_host(*args, C.byref(o), device)
+    else:
+        rc = L.odam_sq_optimize_objective_host(*args, C.byref(obj), C.byref(o), device)
     _lib.check(rc)
     out.update((name, keep[name]) for name in extras)
     return out
@@ -304,14 +332,21 @@ class DeviceTracks:
 
 
 def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr_shape=0.1, threads=0,
-                    max_slices=0, out=None, cycles=None, cluster=0, code_layout=0, corners=None):
+                    max_slices=0, out=None, cycles=None, cluster=0, code_layout=0, corners=None, side_weight=None,
+                    loss="l1", loss_scale=None, lr_scale=None):
     """Enqueue one fused launch on torch's current stream; returns dict of CUDA tensors (no sync).
     out: the dict of a previous call with the same n and n_iters, to be written again.
     cycles: optional int64 CUDA tensor [n, 16], per-phase SM cycles (diagnostics; slot names in tools/prof_run.py).
     corners: optional float64 CUDA tensor [n, 8, 3] -- the oriented boxes of the optimised objects, from a second launch
-    enqueued right behind the optimiser (odam_sq_options.out_corners)."""
+    enqueued right behind the optimiser (odam_sq_options.out_corners).
+    side_weight, loss, loss_scale, lr_scale: the objective of optimize_host; side_weight is a float32 CUDA tensor
+    [SV, 4] on the tracks' device, read in place and not validated (negative or non-finite weights are the caller's to
+    exclude); lr_scale is a host array [n_iters]."""
     torch = dt.torch
     dev = dt.init.device   # the tracks' device, with its index
+    if side_weight is not None:
+        _lib.check_tensor("side_weight", side_weight, torch.float32, (dt.total_views, 4), dev)
+    obj, _sched = _objective(_lib.tensor_ptr(side_weight), loss, loss_scale, lr_scale, n_iters)
     shapes = dict(params=(torch.float32, (dt.n, 9)), loss=(torch.float32, (dt.n, n_iters)), status=(torch.int32, (dt.n,)))
     if out is None:
         out = {k: torch.empty(shape, dtype=dtype, device=dev) for k, (dtype, shape) in shapes.items()}
@@ -332,11 +367,14 @@ def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr
     o.max_views = int(np.diff(dt.view_off_host).max()) if dt.n else 0
     p = _lib.tensor_ptr
     o.out_cycles, o.out_corners = p(cycles), p(corners)
+    args = (p(dt.init), p(dt.cls), p(dt.view_off), p(dt.Ms), p(dt.box), p(dt.mask), p(dt.prior), dt.n, n_iters,
+            _lib.REPR[representation], lr, lr_shape, p(out["params"]), p(out["loss"]), p(out["status"]))
+    L = _lib.load()
     with torch.cuda.device(dev):
-        rc = _lib.load().odam_sq_optimize(p(dt.init), p(dt.cls), p(dt.view_off), p(dt.Ms), p(dt.box), p(dt.mask),
-                                          p(dt.prior), dt.n, n_iters, _lib.REPR[representation], lr, lr_shape,
-                                          p(out["params"]), p(out["loss"]), p(out["status"]), C.byref(o),
-                                          _lib.current_stream(dev))
+        if obj is None:
+            rc = L.odam_sq_optimize(*args, C.byref(o), _lib.current_stream(dev))
+        else:
+            rc = L.odam_sq_optimize_objective(*args, C.byref(obj), C.byref(o), _lib.current_stream(dev))
     _lib.check(rc)
     return out
 

@@ -8,8 +8,10 @@ schedule, or backpropagate into parameters produced by other modules.
   box_sides(params, view_off, Ms, camera_grad=False)
                                           -> (pred [SV, 4], arg [SV, 4] int32)
                                              the projected box sides of constraint_2d (sq_libs.py:397-413)
-  box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None, camera_grad=False) -> [n]
-                                             the optimiser's per-object loss (sq_libs.py:420-430 + :463-466)
+  box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None, camera_grad=False, weight=None, loss="l1",
+           loss_scale=None) -> [n]
+                                             the optimiser's per-object loss (sq_libs.py:420-430 + :463-466), or the
+                                             weighted robust objective of api.optimize_host(side_weight=, loss=, ...)
 
 params is a float32 CUDA tensor [n, 9]: translation x, y, z | yaw | scales s1, s2, s3 | shape logits h1, h2, the layout of
 include/odam_sq.h.  Object i owns the views view_off[i] .. view_off[i+1]-1 of Ms ([SV, 12] or [SV, 3, 4] float32 camera
@@ -29,6 +31,8 @@ gathered per frame, Ms = P[frame_idx] (run_multi_view.stage_tracks returns frame
 sums with atomics and is bit-reproducible only under torch.use_deterministic_algorithms(True).  dL/dMs itself is
 deterministic either way.
 """
+import math
+
 import torch
 from torch.autograd.function import once_differentiable
 
@@ -162,7 +166,8 @@ def box_sides(params, view_off, Ms, camera_grad=False):
     return _BoxSides.apply(params.contiguous(), voff, Ms12 if camera_grad else Ms12.detach())
 
 
-def box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None, camera_grad=False):
+def box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None, camera_grad=False, weight=None, loss="l1",
+             loss_scale=None):
     """The optimiser's loss per object, [n] float32: the sum over the four sides of the mean over all V views of the
     object of mask * |pred - box| (NaN terms count 0), plus 20 (s0 - s)^T A (s0 - s) with A = prior[cls] when a prior
     table is given.
@@ -170,15 +175,26 @@ def box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None, cam
     box [SV, 4] float32 detected sides (x_min, x_max, y_min, y_max), mask [SV, 4] (nonzero = side present), prior
     [8, 9] float32 per-class matrices (api.prior_table()), cls [n] class ids 0..7, s0 [n, 3] the anchor scales (the
     reference takes the scales at the start of its run).  The sum of this loss over objects, backpropagated, gives the
-    fused optimiser's gradient.  camera_grad=True also backpropagates into Ms (box_sides)."""
+    fused optimiser's gradient.  camera_grad=True also backpropagates into Ms (box_sides).
+
+    weight, loss, loss_scale: the objective of api.optimize_host(side_weight=, loss=, loss_scale=) in torch ops, each
+    term weight * mask * rho(pred - box) with rho = |r| ("l1", the default), torch's smooth_l1_loss with beta =
+    loss_scale ("smooth_l1") or 0.5 c^2 log1p((r / c)^2) with c = loss_scale ("cauchy"); weight [SV, 4] float32 on
+    params' device, finite and >= 0 (not checked), or None = 1.  With the defaults this is the reference's loss."""
     pred, _ = box_sides(params, view_off, Ms, camera_grad)
     n, SV, dev = params.shape[0], pred.shape[0], params.device
-    for name, t in (("box", box), ("mask", mask)):
+    for name, t in (("box", box), ("mask", mask)) + ((("weight", weight),) if weight is not None else ()):
         if not isinstance(t, torch.Tensor) or tuple(t.shape) != (SV, 4):
             raise ValueError(f"{name} must be a tensor of shape [SV, 4] = [{SV}, 4]")
         _check_cuda(name, t, dev)
     if box.dtype != torch.float32:
         raise ValueError("box must be float32")
+    if weight is not None and weight.dtype != torch.float32:
+        raise ValueError("weight must be float32")
+    if loss not in _lib.LOSS:
+        raise ValueError(f"loss must be one of {', '.join(_lib.LOSS)}, got {loss!r}")
+    if loss != "l1" and not (loss_scale is not None and math.isfinite(loss_scale) and loss_scale > 0):
+        raise ValueError(f"loss={loss!r} needs a finite loss_scale > 0, got {loss_scale!r}")
     if prior is not None:
         if cls is None or s0 is None:
             raise ValueError("a prior needs cls and s0 (the anchor scales, [n, 3])")
@@ -192,8 +208,15 @@ def box_loss(params, view_off, Ms, box, mask, prior=None, cls=None, s0=None, cam
             _check_cuda(name, t, dev)
     # clamped into [0, SV] and made monotone without a host round trip: device offsets are not checked on the host
     voff = torch.cummax(view_off.to(dev, torch.int64).clamp(0, SV), 0).values
-    l =torch.abs(pred - box)
-    l = torch.where(torch.isnan(l), torch.zeros_like(l), l) * mask.to(torch.float32)
+    if loss == "l1":
+        l =torch.abs(pred - box)
+    elif loss == "smooth_l1":
+        l = torch.nn.functional.smooth_l1_loss(pred, box, reduction="none", beta=loss_scale)
+    else:
+        t = (pred - box) / loss_scale
+        l = 0.5 * loss_scale * loss_scale * torch.log1p(t * t)
+    w = mask.to(torch.float32) if weight is None else mask.to(torch.float32) * weight
+    l = torch.where(torch.isnan(l), torch.zeros_like(l), l) * w
     per_side = torch.segment_reduce(l, "sum", offsets=voff, axis=0, unsafe=True)          # [n, 4]
     V = (voff[1:] - voff[:-1]).to(torch.float32)
     loss = (per_side / V[:, None]).sum(1)

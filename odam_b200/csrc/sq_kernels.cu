@@ -20,6 +20,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <mutex>
 #include <vector>
 
@@ -79,6 +80,10 @@ struct OptArgs {
     float *out_m, *out_v, *out_grad, *out_pred; int32_t *out_arg; uint8_t *out_eta_idx; float *out_grids;
     float *out_param_hist;
     long long *out_cycles;
+    // the objective build only (odam_sq_objective); appended so that the other builds' parameter offsets stay put
+    const float *side_weight;   // [SV][4] or NULL = 1
+    int loss_kind;              // ODAM_SQ_LOSS_*
+    float loss_scale;           // beta / c of the robust kinds
 };
 
 // phase A: what the sampler and the surface need of parameter `k` (one lane per parameter), plus the per-iteration
@@ -351,11 +356,32 @@ __device__ __forceinline__ unsigned item_code(int item, int V, int slices)
     return ((unsigned)v << 16) | (unsigned)(((sl * kNChunks) / slices) << 8) | (unsigned)(((sl + 1) * kNChunks) / slices);
 }
 
+// rho(r) and rho'(r) of a side's residual r under odam_sq_objective::loss; s = loss_scale (beta or c).  IEEE division
+// and libdevice's log1pf: the library builds with -fmad=false, and the oracle is torch's fp32 smooth_l1_loss / log1p.
+__device__ __forceinline__ void residual_loss(int kind, float s, float r, float &rho, float &drho)
+{
+    const float z = fabsf(r);
+    if (kind == ODAM_SQ_LOSS_SMOOTH_L1) {   // torch.nn.functional.smooth_l1_loss(beta=s)
+        const bool quad = z < s;
+        rho = quad ? __fdiv_rn(__fmul_rn(__fmul_rn(0.5f, z), z), s) : __fsub_rn(z, __fmul_rn(0.5f, s));
+        drho = quad ? __fdiv_rn(r, s) : sgnf(r);
+    } else if (kind == ODAM_SQ_LOSS_CAUCHY) {   // 0.5 c^2 log1p((r/c)^2)
+        const float t = __fdiv_rn(r, s), t2 = __fmul_rn(t, t);
+        rho = __fmul_rn(__fmul_rn(__fmul_rn(0.5f, s), s), log1pf(t2));
+        drho = __fdiv_rn(r, __fadd_rn(1.f, t2));
+    } else {
+        rho = z;
+        drho = sgnf(r);
+    }
+}
+
 // kCompact selects the small-instruction-footprint build (odam_sq_options::code_layout): same arithmetic either way.
 // kProf: the instantiation that accumulates the per-phase cycle counts (odam_sq_options::out_cycles).  The marks are
 // compiled out of the production kernels: a predicate test, a branch and a volatile clock read at 15 places cost
 // 2.6 % (config 2) to 4.8 % (config 5) of the throughput even when no count is taken.
-template <int kMaxThreads, bool kCompact, bool kSolo = false, bool kProf = false>
+// kObjective: the build of odam_sq_optimize_objective with per-side weights and a robust residual loss (phase F only);
+// the other builds form the reference's masked L1.
+template <int kMaxThreads, bool kCompact, bool kSolo = false, bool kProf = false, bool kObjective = false>
 __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact, kSolo)) sq_optimize_kernel(OptArgs A)
 {
     // fixed state in static shared memory (compile-time addresses), per-launch scratch in dynamic shared memory
@@ -479,6 +505,9 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
             int gv = v_begin + v;
             float target = Bsrc[v * 4 + sd];
             float mk = Ksrc[v * 4 + sd] ? 1.f : 0.f;
+            // the objective build's effective weight mask * w: a side of weight 0 is a masked-out side in every respect
+            if constexpr (kObjective)
+                if (mk != 0.f && A.side_weight) mk = A.side_weight[(size_t)gv * 4 + sd];
             // Only two rows of the camera matrix matter to this side: Mr = the x row (sides 0,1) or the y row (2,3), Mz.
             // The scan ranks points with a 1-ulp reciprocal; the winner's coordinate is now re-evaluated with the
             // reference's own rounding sequence (k-ordered FMA chain of the CPU GEMM, IEEE division) so that the
@@ -499,7 +528,8 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
             }
             SQ_MARK(S, tid, 5);
             float diff = __fsub_rn(best, target);
-            float l = fabsf(diff);
+            float l = fabsf(diff), dl = 0.f;
+            if constexpr (kObjective) residual_loss(A.loss_kind, A.loss_scale, diff, l, dl);
             if (!(l == l)) l = 0.f;  // sq_libs.py:426-427
             lside = __fadd_rn(lside, __fmul_rn(l, mk));
             if (last) {
@@ -511,7 +541,7 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
             // gradient through the arg-extreme point.  point_vjp (sq_autograd.cuh) holds the same chain rule for the
             // differentiable ops; this copy stays inline on purpose: phase F is register-capped tuned code, and on the
             // shared helper it measured 0.2 % slower (config 2, B200 at 1000 W).
-            float c = __fmul_rn(__fmul_rn(sgnf(diff), mk), invV);
+            float c = __fmul_rn(__fmul_rn(kObjective ? dl : sgnf(diff), mk), invV);   // (rho' w) / V
             float g_lin = __fdiv_rn(c, d);                                        // d(u)/d(q_x or q_y)
             float g_z = -__fmul_rn(__fdiv_rn(__fmul_rn(c, num), __fmul_rn(d, d)), sgnf(qz));  // d(u)/d(q_z)
             float gp0 = __fmaf_rn(Mz[0], g_z, __fmul_rn(Mr[0], g_lin));
@@ -911,6 +941,7 @@ struct DeviceGuard {
 
 struct AdamTab {   // bias-correction table of one (stream, schedule): kept until evicted, never shared across streams
     cudaStream_t stream; int iters, step0; double lr, lrs; float *dev; int cap;
+    std::vector<float> lr_scale;   // odam_sq_objective::lr_scale of the table (empty = constant)
 };
 
 struct DeviceState {
@@ -929,14 +960,17 @@ struct DeviceState {
 static DeviceState g_dev[64];
 static std::mutex g_mu;
 
-static void fill_adam_tab(std::vector<float> &tab, int n_iters, int step0, double lr, double lr_shape)
+// lr_scale (NULL = constant): group["lr"] = lr * lr_scale[it] of a torch scheduler, in double as Python computes it
+static void fill_adam_tab(std::vector<float> &tab, int n_iters, int step0, double lr, double lr_shape,
+                          const float *lr_scale = nullptr)
 {
     tab.resize((size_t)n_iters * 4);
     for (int it = 0; it < n_iters; it++) {
         double step = (double)(step0 + it + 1);
         double bc1 = 1.0 - pow(0.9, step), bc2 = 1.0 - pow(0.999, step);
-        tab[it * 4 + 0] = (float)(-(lr / bc1));
-        tab[it * 4 + 1] = (float)(-(lr_shape / bc1));
+        const double sc = lr_scale ? (double)lr_scale[it] : 1.0;
+        tab[it * 4 + 0] = (float)(-((lr * sc) / bc1));
+        tab[it * 4 + 1] = (float)(-((lr_shape * sc) / bc1));
         tab[it * 4 + 2] = (float)pow(bc2, 0.5);
         tab[it * 4 + 3] = 0.f;
     }
@@ -946,12 +980,14 @@ static void fill_adam_tab(std::vector<float> &tab, int n_iters, int step0, doubl
 // floats); one cached table per (stream, schedule), so launches on different streams never share -- or overwrite --
 // each other's table
 static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, float lr, float lr_shape,
-                      const float *&dev)
+                      const float *lr_scale, const float *&dev)
 {
     std::lock_guard<std::mutex> lk(g_mu);
     dev = nullptr;
+    const std::vector<float> sched = lr_scale ? std::vector<float>(lr_scale, lr_scale + n_iters) : std::vector<float>();
     for (const AdamTab &t : D.tabs)
-        if (t.stream == st && t.iters == n_iters && t.step0 == step0 && t.lr == (double)lr && t.lrs == (double)lr_shape)
+        if (t.stream == st && t.iters == n_iters && t.step0 == step0 && t.lr == (double)lr && t.lrs == (double)lr_shape &&
+            t.lr_scale == sched)
             dev = t.dev;
     if (dev) return ODAM_SQ_OK;
     AdamTab *slot = nullptr;
@@ -962,7 +998,7 @@ static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, f
         CU(cudaStreamSynchronize(slot->stream));          // its last launch may still read the table
         if (slot->cap < n_iters) { cudaFree(slot->dev); slot->dev = nullptr; slot->cap = 0; }
     } else {
-        D.tabs.push_back(AdamTab{st, 0, 0, 0, 0, nullptr, 0});
+        D.tabs.push_back(AdamTab{st, 0, 0, 0, 0, nullptr, 0, {}});
         slot = &D.tabs.back();
     }
     if (!slot->dev) {
@@ -970,42 +1006,54 @@ static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, f
         slot->cap = n_iters;
     }
     std::vector<float> tab;
-    fill_adam_tab(tab, n_iters, step0, (double)lr, (double)lr_shape);
+    fill_adam_tab(tab, n_iters, step0, (double)lr, (double)lr_shape, lr_scale);
     // pageable source: the copy has left the host vector when the call returns
     CU(cudaMemcpyAsync(slot->dev, tab.data(), sizeof(float) * tab.size(), cudaMemcpyHostToDevice, st));
     slot->stream = st; slot->iters = n_iters; slot->step0 = step0; slot->lr = (double)lr; slot->lrs = (double)lr_shape;
+    slot->lr_scale = sched;
     dev = slot->dev;
     return ODAM_SQ_OK;
 }
 
 using OptKernel = void (*)(OptArgs);
 
-// The builds of sq_optimize_kernel, each with its cycle-mark twin (prof), in ascending CTA size within each layout.
+// The builds of sq_optimize_kernel, each with its cycle-mark twin (prof), in ascending CTA size within each layout;
+// then the objective builds (weights and robust losses, odam_sq_optimize_objective), which have no twin.
 // Their register budget follows from __launch_bounds__: min_blocks() CTAs of `threads` share the 64K registers.
 // The compact layout only exists for CTAs of up to 256 threads (it is for many small CTAs per SM).
-struct OptBuild { int threads; bool compact, solo, prof; OptKernel kern; };
+struct OptBuild { int threads; bool compact, solo, prof, objective; OptKernel kern; };
 static const OptBuild kOptBuilds[] = {
-    {256, false, false, false, sq_optimize_kernel<256, false, false, false>},
-    {512, false, false, false, sq_optimize_kernel<512, false, false, false>},
-    {1024, false, false, false, sq_optimize_kernel<1024, false, false, false>},
-    {256, true, false, false, sq_optimize_kernel<256, true, false, false>},
-    {512, false, true, false, sq_optimize_kernel<512, false, true, false>},
-    {256, false, false, true, sq_optimize_kernel<256, false, false, true>},
-    {512, false, false, true, sq_optimize_kernel<512, false, false, true>},
-    {1024, false, false, true, sq_optimize_kernel<1024, false, false, true>},
-    {256, true, false, true, sq_optimize_kernel<256, true, false, true>},
-    {512, false, true, true, sq_optimize_kernel<512, false, true, true>},
+    {256, false, false, false, false, sq_optimize_kernel<256, false, false, false>},
+    {512, false, false, false, false, sq_optimize_kernel<512, false, false, false>},
+    {1024, false, false, false, false, sq_optimize_kernel<1024, false, false, false>},
+    {256, true, false, false, false, sq_optimize_kernel<256, true, false, false>},
+    {512, false, true, false, false, sq_optimize_kernel<512, false, true, false>},
+    {256, false, false, true, false, sq_optimize_kernel<256, false, false, true>},
+    {512, false, false, true, false, sq_optimize_kernel<512, false, false, true>},
+    {1024, false, false, true, false, sq_optimize_kernel<1024, false, false, true>},
+    {256, true, false, true, false, sq_optimize_kernel<256, true, false, true>},
+    {512, false, true, true, false, sq_optimize_kernel<512, false, true, true>},
+    {256, false, false, false, true, sq_optimize_kernel<256, false, false, false, true>},
+    {512, false, false, false, true, sq_optimize_kernel<512, false, false, false, true>},
+    {1024, false, false, false, true, sq_optimize_kernel<1024, false, false, false, true>},
+    {256, true, false, false, true, sq_optimize_kernel<256, true, false, false, true>},
+    {512, false, true, false, true, sq_optimize_kernel<512, false, true, false, true>},
 };
 
 // the smallest build of the layout that fits `threads` CTA threads; the solo build when every CTA has an SM to itself
 // and it fits, else the shared one; NULL: no such build
-static const OptBuild *pick_build(int threads, bool compact, bool solo, bool prof)
+static const OptBuild *pick_build(int threads, bool compact, bool solo, bool prof, bool objective = false)
 {
     for (int want_solo = solo && !compact; want_solo >= 0; want_solo--)
         for (const OptBuild &B : kOptBuilds)
-            if (B.compact == compact && B.solo == (bool)want_solo && B.prof == prof && threads <= B.threads) return &B;
+            if (B.compact == compact && B.solo == (bool)want_solo && B.prof == prof && B.objective == objective &&
+                threads <= B.threads)
+                return &B;
     return nullptr;
 }
+
+// whether a launch with these arguments runs an objective build
+static bool objective_build(const OptArgs &A) { return A.side_weight || A.loss_kind != ODAM_SQ_LOSS_L1; }
 
 static int opt_regs(const OptBuild &B) { return 65536 / (B.threads * min_blocks(B.threads, B.compact, B.solo)); }
 
@@ -1258,7 +1306,7 @@ static int launch_optimize(const OptArgs &A0, const LaunchCfg &L, cudaStream_t s
     A.red_offset = L.red_offset;
     A.stage_offset = L.stage_offset; A.stage_views = L.stage_views;
     if (A.out_status) CU(cudaMemsetAsync(A.out_status, 0, sizeof(int32_t) * A.n, st));  // CTAs OR their flags in
-    OptKernel kern = pick_build(L.threads, L.compact, L.solo, A.out_cycles != nullptr)->kern;
+    OptKernel kern = pick_build(L.threads, L.compact, L.solo, A.out_cycles != nullptr, objective_build(A))->kern;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof cfg);
     cfg.gridDim = dim3(A.n * L.cluster); cfg.blockDim = dim3(L.threads); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
@@ -1418,6 +1466,24 @@ static int check_opt_args(const OptArgs &A, int representation)
     return ODAM_SQ_OK;
 }
 
+// obj (may be NULL) -> the objective fields of A and the host schedule, after the checks include/odam_sq.h lists for
+// both entries (the host entry checks its weights itself, once it knows how many views there are)
+static int objective_args(const odam_sq_objective *obj, const odam_sq_options *opt, OptArgs &A, const float *&lr_scale)
+{
+    lr_scale = nullptr;
+    if (!obj) return ODAM_SQ_OK;
+    const bool robust = obj->loss != ODAM_SQ_LOSS_L1;
+    if (obj->loss < ODAM_SQ_LOSS_L1 || obj->loss > ODAM_SQ_LOSS_CAUCHY) return ODAM_SQ_ERR_ARG;
+    if (robust && !(std::isfinite(obj->loss_scale) && obj->loss_scale > 0.f)) return ODAM_SQ_ERR_ARG;
+    if (obj->lr_scale)
+        for (int it = 0; it < A.n_iters; it++)
+            if (!(std::isfinite(obj->lr_scale[it]) && obj->lr_scale[it] >= 0.f)) return ODAM_SQ_ERR_ARG;
+    A.side_weight = obj->side_weight; A.loss_kind = obj->loss; A.loss_scale = robust ? obj->loss_scale : 0.f;
+    if (objective_build(A) && opt && opt->out_cycles) return ODAM_SQ_ERR_ARG;   // no cycle-mark twin
+    lr_scale = obj->lr_scale;
+    return ODAM_SQ_OK;
+}
+
 }  // namespace odam
 
 using namespace odam;
@@ -1489,9 +1555,21 @@ int odam_sq_optimize(const float *init, const int32_t *cls, const int32_t *view_
                      int representation, float lr, float lr_shape, float *out_params, float *out_loss,
                      int32_t *out_status, const odam_sq_options *opt, void *stream)
 {
+    return odam_sq_optimize_objective(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, lr, lr_shape,
+                                      out_params, out_loss, out_status, nullptr, opt, stream);
+}
+
+int odam_sq_optimize_objective(const float *init, const int32_t *cls, const int32_t *view_off, const float *Ms,
+                               const float *box, const uint8_t *mask, const float *prior, int n, int n_iters,
+                               int representation, float lr, float lr_shape, float *out_params, float *out_loss,
+                               int32_t *out_status, const odam_sq_objective *obj, const odam_sq_options *opt,
+                               void *stream)
+{
     OptArgs A = opt_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
                          out_status, opt);
+    const float *lr_scale;
     int rc = check_opt_args(A, representation);
+    if (!rc) rc = objective_args(obj, opt, A, lr_scale);
     if (rc || n_iters == 0) return rc;
     return on_current_device(n, [&](DeviceState &D) {
         cudaStream_t st = (cudaStream_t)stream;
@@ -1509,7 +1587,7 @@ int odam_sq_optimize(const float *init, const int32_t *cls, const int32_t *view_
         LaunchCfg L;
         rc = choose_launch(maxv, meanv, n, opt, D.sm_count, D.max_smem_optin, D.excl_clusters, L);
         if (rc) return rc;
-        rc = adam_table(D, st, n_iters, opt ? opt->step0 : 0, lr, lr_shape, A.adam_tab);
+        rc = adam_table(D, st, n_iters, opt ? opt->step0 : 0, lr, lr_shape, lr_scale, A.adam_tab);
         if (rc) return rc;
         rc = launch_optimize(A, L, st);
         if (rc || !(opt && opt->out_corners)) return rc;
@@ -1580,9 +1658,21 @@ int odam_sq_optimize_host(const float *init, const int32_t *cls, const int32_t *
                           int representation, float lr, float lr_shape, float *out_params, float *out_loss,
                           int32_t *out_status, const odam_sq_options *opt, int device)
 {
+    return odam_sq_optimize_objective_host(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, lr,
+                                           lr_shape, out_params, out_loss, out_status, nullptr, opt, device);
+}
+
+int odam_sq_optimize_objective_host(const float *init, const int32_t *cls, const int32_t *view_off, const float *Ms,
+                                    const float *box, const uint8_t *mask, const float *prior, int n, int n_iters,
+                                    int representation, float lr, float lr_shape, float *out_params, float *out_loss,
+                                    int32_t *out_status, const odam_sq_objective *obj, const odam_sq_options *opt,
+                                    int device)
+{
     OptArgs A = opt_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
                          out_status, opt);
+    const float *lr_scale;
     int maxv, rc = check_opt_args(A, representation);
+    if (!rc) rc = objective_args(obj, opt, A, lr_scale);
     if (rc || n == 0 || n_iters == 0) return rc;
     rc = check_view_off(view_off, n, maxv);
     if (rc) return rc;
@@ -1590,6 +1680,9 @@ int odam_sq_optimize_host(const float *init, const int32_t *cls, const int32_t *
         for (int i = 0; i < n; i++)
             if (cls[i] < 0 || cls[i] > 7) return ODAM_SQ_ERR_ARG;   // 8 classes (sq_libs.py:13-22)
     const size_t SV = (size_t)view_off[n];
+    if (A.side_weight)
+        for (size_t k = 0; k < SV * 4; k++)
+            if (!(std::isfinite(A.side_weight[k]) && A.side_weight[k] >= 0.f)) return ODAM_SQ_ERR_ARG;
     rc = ensure_init(device);
     if (rc) return rc;
     const DeviceState &D = g_dev[device];
@@ -1597,7 +1690,7 @@ int odam_sq_optimize_host(const float *init, const int32_t *cls, const int32_t *
     rc = choose_launch(maxv, (double)SV / n, n, opt, D.sm_count, D.max_smem_optin, D.excl_clusters, L);
     if (rc) return rc;
     std::vector<float> tab;
-    fill_adam_tab(tab, n_iters, opt ? opt->step0 : 0, (double)lr, (double)lr_shape);
+    fill_adam_tab(tab, n_iters, opt ? opt->step0 : 0, (double)lr, (double)lr_shape, lr_scale);
     A.adam_tab = tab.data();
     A.out_cycles = nullptr;   // a device-pointer option
     double *corners = opt ? opt->out_corners : nullptr;
@@ -1605,7 +1698,7 @@ int odam_sq_optimize_host(const float *init, const int32_t *cls, const int32_t *
     const size_t n9 = (size_t)n * 9;
     Staging S;
     S.in(A.init, n9); S.in(A.cls, n); S.in(A.view_off, n + 1); S.in(A.Ms, SV * 12); S.in(A.box, SV * 4);
-    S.in(A.mask, SV * 4); S.in(A.prior, 72); S.in(A.adam_tab, tab.size());
+    S.in(A.mask, SV * 4); S.in(A.prior, 72); S.in(A.adam_tab, tab.size()); S.in(A.side_weight, SV * 4);
     S.in(A.m0, n9); S.in(A.v0, n9); S.in(A.s0, (size_t)n * 3);
     S.out(A.out_params, n9); S.out(A.out_loss, (size_t)n * n_iters); S.out(A.out_status, n);
     S.out(A.out_m, n9); S.out(A.out_v, n9); S.out(A.out_grad, n9); S.out(A.out_pred, SV * 4); S.out(A.out_arg, SV * 4);
