@@ -165,6 +165,54 @@ int odam_sq_optimize_objective_host(const float *init, const int32_t *cls, const
                                     float *out_params, float *out_loss, int32_t *out_status,
                                     const odam_sq_objective *obj, const odam_sq_options *opt, int device);
 
+/* Opt-in early stopping of odam_sq_optimize_converge[_host]: each object stops once its loss stops improving, and may
+ * return its lowest-loss iterate instead of the last one.
+ *
+ * The rule is per object.  L[k] is the loss before step k, the value written to out_loss.  keep is
+ * (float)(1.0 - (double)rel_tol), computed on the host.  All comparisons are in fp32.
+ *
+ *     best = +inf; b = -1; last = 0
+ *     for k in 0 .. n_iters-1:
+ *         (iteration k: loss L[k] at the current params, then the Adam step)
+ *         if isfinite(L[k]):
+ *             if b < 0 or L[k] < best * keep:  last = k       # a significant improvement (fp32 product, round to nearest)
+ *             if b < 0 or L[k] < best:         best = L[k]; b = k   # strict: first index on ties
+ *         if patience > 0 and k - last >= patience:  stop; iters = k + 1
+ *
+ * Outputs of an object that stopped: out_loss[iters:] and the rows out_param_hist[iters:] are NaN.  out_params holds
+ * the parameters after step iters - 1; with keep_best, those at which L[b] was evaluated instead (init when b = 0, else
+ * the parameters after step b - 1; the last ones when no loss was finite).  out_m, out_v and out_grad describe the
+ * last step run, and out_corners the boxes of whatever out_params holds.  The status flags keep their meaning;
+ * out_iters < n_iters is the signal that an object stopped.
+ * Until an object stops, it runs the arithmetic of odam_sq_optimize_objective: with patience = 0 and keep_best = 0
+ * every output equals that entry's.  The kernel build with the rule has no cycle-mark twin. */
+typedef struct odam_sq_convergence {
+    int patience;            /* 0 = never stop early; else stop after `patience` iterations without improvement   */
+    float rel_tol;           /* finite, 0 <= rel_tol < 1                                                          */
+    int keep_best;           /* 1: out_params = the parameters at which the lowest loss was evaluated               */
+    int32_t *out_iters;      /* [n] iterations run (may be NULL)                                                  */
+    int32_t *out_best_iter;  /* [n] iteration of the lowest finite loss, -1 if none (may be NULL)                  */
+} odam_sq_convergence;
+
+/* odam_sq_optimize_objective[_host] with the convergence rule above; conv == NULL is exactly that entry, and obj ==
+ * NULL means the reference's objective.  out_iters and out_best_iter are device pointers for odam_sq_optimize_converge
+ * and host pointers for the _host entry, as the other outputs.  Besides the checks of odam_sq_optimize_objective
+ * [_host], ODAM_SQ_ERR_ARG (before any CUDA call) for patience < 0, a rel_tol that is not finite or outside [0, 1),
+ * keep_best other than 0 or 1, and conv together with opt->out_pred, out_arg, out_eta_idx, out_grids or out_cycles:
+ * those describe the last iteration, which the kernel only knows once it has run it. */
+int odam_sq_optimize_converge(const float *init, const int32_t *cls, const int32_t *view_off,
+                              const float *Ms, const float *box, const uint8_t *mask, const float *prior,
+                              int n, int n_iters, int representation, float lr, float lr_shape,
+                              float *out_params, float *out_loss, int32_t *out_status,
+                              const odam_sq_objective *obj, const odam_sq_convergence *conv,
+                              const odam_sq_options *opt, void *stream);
+int odam_sq_optimize_converge_host(const float *init, const int32_t *cls, const int32_t *view_off,
+                                   const float *Ms, const float *box, const uint8_t *mask, const float *prior,
+                                   int n, int n_iters, int representation, float lr, float lr_shape,
+                                   float *out_params, float *out_loss, int32_t *out_status,
+                                   const odam_sq_objective *obj, const odam_sq_convergence *conv,
+                                   const odam_sq_options *opt, int device);
+
 /* compute_ellipsoid_points (sq_libs.py:577-595): params[n][9] -> xyz[n][1000][3] world points. */
 int odam_sq_sample_points(const float *params, int n, float *out_xyz, void *stream);
 int odam_sq_sample_points_host(const float *params, int n, float *out_xyz, int device);

@@ -34,6 +34,12 @@ class Objective(C.Structure):
     _fields_ = [("side_weight", C.c_void_p), ("loss", C.c_int), ("loss_scale", C.c_float), ("lr_scale", C.c_void_p)]
 
 
+class Convergence(C.Structure):
+    """odam_sq_convergence (include/odam_sq.h)."""
+    _fields_ = [("patience", C.c_int), ("rel_tol", C.c_float), ("keep_best", C.c_int), ("out_iters", C.c_void_p),
+                ("out_best_iter", C.c_void_p)]
+
+
 class OdamSqError(RuntimeError):
     pass
 
@@ -50,6 +56,9 @@ ARGTYPES = {
     "odam_sq_optimize_host": _OPT + [_ci],
     "odam_sq_optimize_objective": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Options), _vp],
     "odam_sq_optimize_objective_host": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Options), _ci],
+    "odam_sq_optimize_converge": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Convergence), C.POINTER(Options), _vp],
+    "odam_sq_optimize_converge_host": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Convergence), C.POINTER(Options),
+                                                   _ci],
     "odam_sq_sample_points": [_vp, _ci, _vp, _vp],
     "odam_sq_sample_points_host": [_vp, _ci, _vp, _ci],
     "odam_sq_project_boxes": [_vp, _vp, _vp, _ci, _vp, _vp],

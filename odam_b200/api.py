@@ -190,9 +190,34 @@ def _objective(side_weight, loss, loss_scale, lr_scale, n_iters):
     return obj, sched
 
 
+# the options that describe the last iteration (and the cycle counts): the convergence build refuses them
+# (include/odam_sq.h)
+NOT_WITH_CONVERGENCE = ("out_pred", "out_arg", "out_eta_idx", "out_grids", "out_cycles")
+
+
+def _convergence(patience, rel_tol, keep_best, extras=()):
+    """odam_sq_convergence of the early-stopping keywords, or None when all are at their defaults: then the entries
+    without the rule run.  The output pointers are the caller's to set."""
+    if isinstance(patience, bool) or not isinstance(patience, (int, np.integer)) or patience < 0:
+        raise ValueError(f"patience must be an integer >= 0, got {patience!r}")
+    if not (np.isfinite(rel_tol) and 0.0 <= rel_tol < 1.0):
+        raise ValueError(f"rel_tol must be finite and in [0, 1), got {rel_tol!r}")
+    if keep_best not in (False, True):
+        raise ValueError(f"keep_best must be a bool, got {keep_best!r}")
+    if patience == 0 and rel_tol == 0.0 and not keep_best:
+        return None
+    bad = [name for name in extras if name in NOT_WITH_CONVERGENCE]
+    if bad:
+        raise ValueError(f"{', '.join(bad)} cannot be asked for with early stopping (patience, rel_tol, keep_best)")
+    conv = _lib.Convergence()
+    conv.patience, conv.rel_tol, conv.keep_best = int(patience), float(rel_tol), int(bool(keep_best))
+    return conv
+
+
 def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric", lr=0.01, lr_shape=0.1,
                   device=0, threads=0, max_slices=0, m0=None, v0=None, step0=0, s0=None, extras=(), cluster=0,
-                  code_layout=0, side_weight=None, loss="l1", loss_scale=None, lr_scale=None):
+                  code_layout=0, side_weight=None, loss="l1", loss_scale=None, lr_scale=None, patience=0, rel_tol=0.0,
+                  keep_best=False):
     """Run the fused optimiser on packed host arrays.  Returns dict(params[n,9], loss[n,n_iters], status[n], ...extras).
 
     prior: None (no prior term) or an [8,9] float32 table (see prior_table()).
@@ -204,12 +229,20 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
       loss: "l1", "smooth_l1" (torch's smooth_l1_loss, beta = loss_scale) or "cauchy" (0.5 c^2 log1p((r/c)^2),
             c = loss_scale), loss_scale in pixels;
       lr_scale: [n_iters] multipliers of both learning rates, one per iteration of this call (a schedule).
+    Early stopping (odam_sq_convergence; all defaults = every object runs n_iters iterations):
+      patience: stop an object once `patience` iterations have passed without a loss below best * (1 - rel_tol)
+                (0 = never);
+      keep_best: return the parameters at which the object's lowest loss was evaluated, not the last ones.
+      The result then has iters[n] (iterations run) and best_iter[n] (iteration of the lowest finite loss, -1 if
+      none), int32; the loss and out_param_hist rows of iterations not run are NaN.  out_pred, out_arg, out_eta_idx
+      and out_grids cannot be asked for with it.
     """
     L = _lib.load()
     init, cls, voff, Ms, box, mask = _track_arrays(tracks)
     n, SV = len(init), int(voff[-1])
     w = _lib.host_array("side_weight", side_weight, np.float32, (SV, 4))
     obj, _sched = _objective(_lib.ptr(w), loss, loss_scale, lr_scale, n_iters)
+    conv = _convergence(patience, rel_tol, keep_best, extras)
     pr = _lib.host_array("prior", prior, np.float32, (8, 9))
     if pr is not None:
         check_classes(cls)
@@ -231,7 +264,12 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
     args = (_lib.ptr(init), _lib.ptr(cls), _lib.ptr(voff), _lib.ptr(Ms), _lib.ptr(box), _lib.ptr(mask), _lib.ptr(pr),
             n, n_iters, _lib.REPR[representation], lr, lr_shape, _lib.ptr(out["params"]), _lib.ptr(out["loss"]),
             _lib.ptr(out["status"]))
-    if obj is None:
+    if conv is not None:
+        out.update(iters=np.zeros(n, np.int32), best_iter=np.zeros(n, np.int32))
+        conv.out_iters, conv.out_best_iter = _lib.ptr(out["iters"]), _lib.ptr(out["best_iter"])
+        rc = L.odam_sq_optimize_converge_host(*args, None if obj is None else C.byref(obj), C.byref(conv), C.byref(o),
+                                              device)
+    elif obj is None:
         rc = L.odam_sq_optimize_host(*args, C.byref(o), device)
     else:
         rc = L.odam_sq_optimize_objective_host(*args, C.byref(obj), C.byref(o), device)
@@ -333,7 +371,7 @@ class DeviceTracks:
 
 def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr_shape=0.1, threads=0,
                     max_slices=0, out=None, cycles=None, cluster=0, code_layout=0, corners=None, side_weight=None,
-                    loss="l1", loss_scale=None, lr_scale=None):
+                    loss="l1", loss_scale=None, lr_scale=None, patience=0, rel_tol=0.0, keep_best=False):
     """Enqueue one fused launch on torch's current stream; returns dict of CUDA tensors (no sync).
     out: the dict of a previous call with the same n and n_iters, to be written again.
     cycles: optional int64 CUDA tensor [n, 16], per-phase SM cycles (diagnostics; slot names in tools/prof_run.py).
@@ -341,16 +379,24 @@ def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr
     enqueued right behind the optimiser (odam_sq_options.out_corners).
     side_weight, loss, loss_scale, lr_scale: the objective of optimize_host; side_weight is a float32 CUDA tensor
     [SV, 4] on the tracks' device, read in place and not validated (negative or non-finite weights are the caller's to
-    exclude); lr_scale is a host array [n_iters]."""
+    exclude); lr_scale is a host array [n_iters].
+    patience, rel_tol, keep_best: the early stopping of optimize_host; the result then has int32 CUDA tensors iters
+    [n] and best_iter [n] (added to `out` when it lacks them)."""
+    conv = _convergence(patience, rel_tol, keep_best, () if cycles is None else ("out_cycles",))
     torch = dt.torch
     dev = dt.init.device   # the tracks' device, with its index
     if side_weight is not None:
         _lib.check_tensor("side_weight", side_weight, torch.float32, (dt.total_views, 4), dev)
     obj, _sched = _objective(_lib.tensor_ptr(side_weight), loss, loss_scale, lr_scale, n_iters)
     shapes = dict(params=(torch.float32, (dt.n, 9)), loss=(torch.float32, (dt.n, n_iters)), status=(torch.int32, (dt.n,)))
+    if conv is not None:
+        shapes.update(iters=(torch.int32, (dt.n,)), best_iter=(torch.int32, (dt.n,)))
     if out is None:
         out = {k: torch.empty(shape, dtype=dtype, device=dev) for k, (dtype, shape) in shapes.items()}
     else:
+        if conv is not None:   # the dict of a call without early stopping
+            for k in ("iters", "best_iter"):
+                out.setdefault(k, torch.empty(shapes[k][1], dtype=shapes[k][0], device=dev))
         for k, (dtype, shape) in shapes.items():
             _lib.check_tensor(f"out[{k!r}]", out[k], dtype, shape, dev)
     if cycles is not None:
@@ -371,7 +417,11 @@ def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr
             _lib.REPR[representation], lr, lr_shape, p(out["params"]), p(out["loss"]), p(out["status"]))
     L = _lib.load()
     with torch.cuda.device(dev):
-        if obj is None:
+        if conv is not None:
+            conv.out_iters, conv.out_best_iter = p(out["iters"]), p(out["best_iter"])
+            rc = L.odam_sq_optimize_converge(*args, None if obj is None else C.byref(obj), C.byref(conv), C.byref(o),
+                                             _lib.current_stream(dev))
+        elif obj is None:
             rc = L.odam_sq_optimize(*args, C.byref(o), _lib.current_stream(dev))
         else:
             rc = L.odam_sq_optimize_objective(*args, C.byref(obj), C.byref(o), _lib.current_stream(dev))

@@ -84,7 +84,25 @@ struct OptArgs {
     const float *side_weight;   // [SV][4] or NULL = 1
     int loss_kind;              // ODAM_SQ_LOSS_*
     float loss_scale;           // beta / c of the robust kinds
+    // the convergence build only (odam_sq_convergence), appended likewise
+    int converge;               // 1: odam_sq_convergence given, the convergence build runs
+    int patience, keep_best;
+    float keep;                 // (float)(1 - rel_tol): L is a significant improvement when L < best * keep
+    int32_t *out_iters, *out_best_iter;
 };
+
+// The convergence build's per-object state, kept by the loss lane of phase G.  It lives in Smem::cyc, which the
+// convergence builds do not use (they have no cycle-mark twin), so that their shared memory, and with it the launch
+// configuration and the CTAs per SM, are those of their objective twins.
+struct ConvState {
+    float prev[9];    // the parameters of this iteration before its Adam step: those at which its loss was evaluated
+    float bestp[9];   // prev of the iteration with the lowest finite loss so far
+    float best;       // that loss
+    int b, last;      // its iteration (-1: none yet); the iteration of the last significant improvement
+    int iters;        // iterations run so far
+    int newbest, stop;
+};
+static_assert(sizeof(ConvState) <= sizeof(Smem::cyc), "ConvState must fit the cycle counters it reuses");
 
 // phase A: what the sampler and the surface need of parameter `k` (one lane per parameter), plus the per-iteration
 // resets of the sampler state (lane 9).  Runs once before the first iteration and then fused with the Adam update.
@@ -381,11 +399,16 @@ __device__ __forceinline__ void residual_loss(int kind, float s, float r, float 
 // 2.6 % (config 2) to 4.8 % (config 5) of the throughput even when no count is taken.
 // kObjective: the build of odam_sq_optimize_objective with per-side weights and a robust residual loss (phase F only);
 // the other builds form the reference's masked L1.
-template <int kMaxThreads, bool kCompact, bool kSolo = false, bool kProf = false, bool kObjective = false>
+// kConverge (only with kObjective): the build of odam_sq_optimize_converge, which stops an object once its loss stops
+// improving and keeps the lowest-loss iterate.  Until it stops, it runs the objective build's arithmetic.
+template <int kMaxThreads, bool kCompact, bool kSolo = false, bool kProf = false, bool kObjective = false,
+          bool kConverge = false>
 __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact, kSolo)) sq_optimize_kernel(OptArgs A)
 {
+    static_assert(!kConverge || kObjective, "the convergence build is an objective build");
     // fixed state in static shared memory (compile-time addresses), per-launch scratch in dynamic shared memory
     __shared__ Smem S;
+    ConvState &CV = *reinterpret_cast<ConvState *>(S.cyc);   // kConverge only, in place of the cycle counters
     extern __shared__ __align__(16) unsigned char scratch_raw[];
     constexpr int kGroup = kCompact ? 4 : kChunk;
     const int tid = threadIdx.x, T = blockDim.x;
@@ -418,7 +441,11 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
     if (tid < 3) S.s0[tid] = A.s0 ? A.s0[(size_t)obj * 3 + tid] : A.init[(size_t)obj * 9 + 4 + tid];
     if (tid == 0) {
         S.status = 0;
-        for (int k = 0; k < 16; k++) S.cyc[k] = 0;
+        if constexpr (kConverge) {
+            CV.best = INFINITY; CV.b = -1; CV.last = 0; CV.iters = 0; CV.newbest = 0; CV.stop = 0;
+        } else {
+            for (int k = 0; k < 16; k++) S.cyc[k] = 0;
+        }
         S.tmark = clock64();
         init_grid_roots(S);
         if (C > 1) {
@@ -653,11 +680,24 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
                     loss = __fadd_rn(loss, __fmul_rn(q3, 20.f));
                 }
                 if (crank == 0) A.out_loss[(size_t)obj * A.n_iters + it] = loss;
+                if constexpr (kConverge) {
+                    // the stopping rule of include/odam_sq.h, in fp32.  It reads the loss and this CTA's own copy of
+                    // the rule's state only, and the loss is the same in every CTA of a cluster (same rank order,
+                    // identical sums): so every CTA of a cluster takes the same decisions.
+                    const bool fin = isfinite(loss), first = CV.b < 0;
+                    if (fin && (first || loss < __fmul_rn(CV.best, A.keep))) CV.last = it;
+                    const bool nb = fin && (first || loss < CV.best);   // strict: the first index on ties
+                    if (nb) { CV.best = loss; CV.b = it; }
+                    CV.newbest = nb;
+                    CV.iters = it + 1;
+                    CV.stop = A.patience > 0 && it - CV.last >= A.patience;
+                }
                 if (!isfinite(loss)) atomicOr(&S.status, ODAM_SQ_ST_NONFINITE);
                 if (S.bad[0] | S.bad[1]) atomicOr(&S.status, ODAM_SQ_ST_SAMPLER);
                 derive_param(S, 9);  // per-iteration resets of the sampler state
             }
             if (k >= 0) {
+                if constexpr (kConverge) CV.prev[k] = S.par[k];
                 if (k < 7 || A.optimize_shapes) {
                     float g = S.grad[k], m = S.m[k], v = S.v[k], p = S.par[k];
                     const float alpha = S.adam_now[k < 7 ? 0 : 1], bc2s = S.adam_now[2];
@@ -682,12 +722,33 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
         }
         __syncthreads();
         SQ_MARK(S, tid, 6);
+        if constexpr (kConverge) {
+            // Invariant: every CTA of a cluster leaves the loop after the same iteration, here, behind the iteration's
+            // last barrier.  CV.stop derives from the loss alone (phase G), which every CTA of the cluster computes
+            // identically; the exchange's mbarrier parities and the exit cluster.sync() depend on it.
+            if (CV.newbest && tid < 9) CV.bestp[tid] = CV.prev[tid];
+            if (CV.stop) break;
+        }
     }
-    if (tid == 0) S.cyc[11] = S.ge.rebuilds + S.go.rebuilds;  // slot 11: tree rebuilds (both grids)
+    if (!kConverge && tid == 0) S.cyc[11] = S.ge.rebuilds + S.go.rebuilds;  // slot 11: tree rebuilds (both grids)
     __syncthreads();
     if (A.out_cycles && crank == 0 && tid < 16) A.out_cycles[(size_t)obj * 16 + tid] = S.cyc[tid];
+    if constexpr (kConverge) {
+        if (crank == 0) {   // the iterations an early stop skipped: NaN loss and parameter rows
+            const int iters = CV.iters;
+            const float nan = __int_as_float(0x7fc00000);
+            for (int i = iters + tid; i < A.n_iters; i += T) A.out_loss[(size_t)obj * A.n_iters + i] = nan;
+            if (A.out_param_hist)
+                for (int i = iters * 9 + tid; i < A.n_iters * 9; i += T)
+                    A.out_param_hist[(size_t)obj * A.n_iters * 9 + i] = nan;
+            if (tid == 0 && A.out_iters) A.out_iters[obj] = iters;
+            if (tid == 0 && A.out_best_iter) A.out_best_iter[obj] = CV.b;
+        }
+    }
     if (tid < 9 && crank == 0) {
         float p = S.par[tid];
+        if constexpr (kConverge)
+            if (A.keep_best && CV.b >= 0) p = CV.bestp[tid];
         A.out_params[(size_t)obj * 9 + tid] = p;
         if (!isfinite(p)) atomicOr(&S.status, ODAM_SQ_ST_NONFINITE);
         if (A.out_m) A.out_m[(size_t)obj * 9 + tid] = S.m[tid];
@@ -1018,42 +1079,49 @@ static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, f
 using OptKernel = void (*)(OptArgs);
 
 // The builds of sq_optimize_kernel, each with its cycle-mark twin (prof), in ascending CTA size within each layout;
-// then the objective builds (weights and robust losses, odam_sq_optimize_objective), which have no twin.
+// then the objective builds (weights and robust losses, odam_sq_optimize_objective), which have no twin, and their
+// convergence twins (odam_sq_optimize_converge).
 // Their register budget follows from __launch_bounds__: min_blocks() CTAs of `threads` share the 64K registers.
 // The compact layout only exists for CTAs of up to 256 threads (it is for many small CTAs per SM).
-struct OptBuild { int threads; bool compact, solo, prof, objective; OptKernel kern; };
+struct OptBuild { int threads; bool compact, solo, prof, objective, converge; OptKernel kern; };
 static const OptBuild kOptBuilds[] = {
-    {256, false, false, false, false, sq_optimize_kernel<256, false, false, false>},
-    {512, false, false, false, false, sq_optimize_kernel<512, false, false, false>},
-    {1024, false, false, false, false, sq_optimize_kernel<1024, false, false, false>},
-    {256, true, false, false, false, sq_optimize_kernel<256, true, false, false>},
-    {512, false, true, false, false, sq_optimize_kernel<512, false, true, false>},
-    {256, false, false, true, false, sq_optimize_kernel<256, false, false, true>},
-    {512, false, false, true, false, sq_optimize_kernel<512, false, false, true>},
-    {1024, false, false, true, false, sq_optimize_kernel<1024, false, false, true>},
-    {256, true, false, true, false, sq_optimize_kernel<256, true, false, true>},
-    {512, false, true, true, false, sq_optimize_kernel<512, false, true, true>},
-    {256, false, false, false, true, sq_optimize_kernel<256, false, false, false, true>},
-    {512, false, false, false, true, sq_optimize_kernel<512, false, false, false, true>},
-    {1024, false, false, false, true, sq_optimize_kernel<1024, false, false, false, true>},
-    {256, true, false, false, true, sq_optimize_kernel<256, true, false, false, true>},
-    {512, false, true, false, true, sq_optimize_kernel<512, false, true, false, true>},
+    {256, false, false, false, false, false, sq_optimize_kernel<256, false, false, false>},
+    {512, false, false, false, false, false, sq_optimize_kernel<512, false, false, false>},
+    {1024, false, false, false, false, false, sq_optimize_kernel<1024, false, false, false>},
+    {256, true, false, false, false, false, sq_optimize_kernel<256, true, false, false>},
+    {512, false, true, false, false, false, sq_optimize_kernel<512, false, true, false>},
+    {256, false, false, true, false, false, sq_optimize_kernel<256, false, false, true>},
+    {512, false, false, true, false, false, sq_optimize_kernel<512, false, false, true>},
+    {1024, false, false, true, false, false, sq_optimize_kernel<1024, false, false, true>},
+    {256, true, false, true, false, false, sq_optimize_kernel<256, true, false, true>},
+    {512, false, true, true, false, false, sq_optimize_kernel<512, false, true, true>},
+    {256, false, false, false, true, false, sq_optimize_kernel<256, false, false, false, true>},
+    {512, false, false, false, true, false, sq_optimize_kernel<512, false, false, false, true>},
+    {1024, false, false, false, true, false, sq_optimize_kernel<1024, false, false, false, true>},
+    {256, true, false, false, true, false, sq_optimize_kernel<256, true, false, false, true>},
+    {512, false, true, false, true, false, sq_optimize_kernel<512, false, true, false, true>},
+    {256, false, false, false, true, true, sq_optimize_kernel<256, false, false, false, true, true>},
+    {512, false, false, false, true, true, sq_optimize_kernel<512, false, false, false, true, true>},
+    {1024, false, false, false, true, true, sq_optimize_kernel<1024, false, false, false, true, true>},
+    {256, true, false, false, true, true, sq_optimize_kernel<256, true, false, false, true, true>},
+    {512, false, true, false, true, true, sq_optimize_kernel<512, false, true, false, true, true>},
 };
 
 // the smallest build of the layout that fits `threads` CTA threads; the solo build when every CTA has an SM to itself
 // and it fits, else the shared one; NULL: no such build
-static const OptBuild *pick_build(int threads, bool compact, bool solo, bool prof, bool objective = false)
+static const OptBuild *pick_build(int threads, bool compact, bool solo, bool prof, bool objective = false,
+                                  bool converge = false)
 {
     for (int want_solo = solo && !compact; want_solo >= 0; want_solo--)
         for (const OptBuild &B : kOptBuilds)
             if (B.compact == compact && B.solo == (bool)want_solo && B.prof == prof && B.objective == objective &&
-                threads <= B.threads)
+                B.converge == converge && threads <= B.threads)
                 return &B;
     return nullptr;
 }
 
-// whether a launch with these arguments runs an objective build
-static bool objective_build(const OptArgs &A) { return A.side_weight || A.loss_kind != ODAM_SQ_LOSS_L1; }
+// whether a launch with these arguments runs an objective build (every convergence build is one)
+static bool objective_build(const OptArgs &A) { return A.side_weight || A.loss_kind != ODAM_SQ_LOSS_L1 || A.converge; }
 
 static int opt_regs(const OptBuild &B) { return 65536 / (B.threads * min_blocks(B.threads, B.compact, B.solo)); }
 
@@ -1306,7 +1374,8 @@ static int launch_optimize(const OptArgs &A0, const LaunchCfg &L, cudaStream_t s
     A.red_offset = L.red_offset;
     A.stage_offset = L.stage_offset; A.stage_views = L.stage_views;
     if (A.out_status) CU(cudaMemsetAsync(A.out_status, 0, sizeof(int32_t) * A.n, st));  // CTAs OR their flags in
-    OptKernel kern = pick_build(L.threads, L.compact, L.solo, A.out_cycles != nullptr, objective_build(A))->kern;
+    OptKernel kern =
+        pick_build(L.threads, L.compact, L.solo, A.out_cycles != nullptr, objective_build(A), A.converge)->kern;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof cfg);
     cfg.gridDim = dim3(A.n * L.cluster); cfg.blockDim = dim3(L.threads); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
@@ -1484,6 +1553,22 @@ static int objective_args(const odam_sq_objective *obj, const odam_sq_options *o
     return ODAM_SQ_OK;
 }
 
+// conv (may be NULL) -> the convergence fields of A, after the checks include/odam_sq.h lists.  The options that
+// describe the last iteration are refused with it: the kernel knows which iteration is the last only once it has run it.
+static int convergence_args(const odam_sq_convergence *conv, const odam_sq_options *opt, OptArgs &A)
+{
+    if (!conv) return ODAM_SQ_OK;
+    if (conv->patience < 0 || !(std::isfinite(conv->rel_tol) && conv->rel_tol >= 0.f && conv->rel_tol < 1.f) ||
+        (conv->keep_best != 0 && conv->keep_best != 1))
+        return ODAM_SQ_ERR_ARG;
+    if (opt && (opt->out_pred || opt->out_arg || opt->out_eta_idx || opt->out_grids || opt->out_cycles))
+        return ODAM_SQ_ERR_ARG;
+    A.converge = 1; A.patience = conv->patience; A.keep_best = conv->keep_best;
+    A.keep = (float)(1.0 - (double)conv->rel_tol);
+    A.out_iters = conv->out_iters; A.out_best_iter = conv->out_best_iter;
+    return ODAM_SQ_OK;
+}
+
 }  // namespace odam
 
 using namespace odam;
@@ -1565,11 +1650,22 @@ int odam_sq_optimize_objective(const float *init, const int32_t *cls, const int3
                                int32_t *out_status, const odam_sq_objective *obj, const odam_sq_options *opt,
                                void *stream)
 {
+    return odam_sq_optimize_converge(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, lr,
+                                     lr_shape, out_params, out_loss, out_status, obj, nullptr, opt, stream);
+}
+
+int odam_sq_optimize_converge(const float *init, const int32_t *cls, const int32_t *view_off, const float *Ms,
+                              const float *box, const uint8_t *mask, const float *prior, int n, int n_iters,
+                              int representation, float lr, float lr_shape, float *out_params, float *out_loss,
+                              int32_t *out_status, const odam_sq_objective *obj, const odam_sq_convergence *conv,
+                              const odam_sq_options *opt, void *stream)
+{
     OptArgs A = opt_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
                          out_status, opt);
     const float *lr_scale;
     int rc = check_opt_args(A, representation);
     if (!rc) rc = objective_args(obj, opt, A, lr_scale);
+    if (!rc) rc = convergence_args(conv, opt, A);
     if (rc || n_iters == 0) return rc;
     return on_current_device(n, [&](DeviceState &D) {
         cudaStream_t st = (cudaStream_t)stream;
@@ -1668,11 +1764,22 @@ int odam_sq_optimize_objective_host(const float *init, const int32_t *cls, const
                                     int32_t *out_status, const odam_sq_objective *obj, const odam_sq_options *opt,
                                     int device)
 {
+    return odam_sq_optimize_converge_host(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, lr,
+                                          lr_shape, out_params, out_loss, out_status, obj, nullptr, opt, device);
+}
+
+int odam_sq_optimize_converge_host(const float *init, const int32_t *cls, const int32_t *view_off, const float *Ms,
+                                   const float *box, const uint8_t *mask, const float *prior, int n, int n_iters,
+                                   int representation, float lr, float lr_shape, float *out_params, float *out_loss,
+                                   int32_t *out_status, const odam_sq_objective *obj,
+                                   const odam_sq_convergence *conv, const odam_sq_options *opt, int device)
+{
     OptArgs A = opt_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
                          out_status, opt);
     const float *lr_scale;
     int maxv, rc = check_opt_args(A, representation);
     if (!rc) rc = objective_args(obj, opt, A, lr_scale);
+    if (!rc) rc = convergence_args(conv, opt, A);
     if (rc || n == 0 || n_iters == 0) return rc;
     rc = check_view_off(view_off, n, maxv);
     if (rc) return rc;
@@ -1704,6 +1811,7 @@ int odam_sq_optimize_objective_host(const float *init, const int32_t *cls, const
     S.out(A.out_m, n9); S.out(A.out_v, n9); S.out(A.out_grad, n9); S.out(A.out_pred, SV * 4); S.out(A.out_arg, SV * 4);
     S.out(A.out_eta_idx, (size_t)n * kN); S.out(A.out_grids, (size_t)n * 2 * kG);
     S.out(A.out_param_hist, n9 * n_iters); S.out(corners, (size_t)n * 24); S.out(box_flag, n);
+    S.out(A.out_iters, n); S.out(A.out_best_iter, n);
     return S.run(device, [&](cudaStream_t st) {
         rc = launch_optimize(A, L, st);
         if (rc || !corners) return rc;
