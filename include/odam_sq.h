@@ -213,6 +213,54 @@ int odam_sq_optimize_converge_host(const float *init, const int32_t *cls, const 
                                    const odam_sq_objective *obj, const odam_sq_convergence *conv,
                                    const odam_sq_options *opt, int device);
 
+/* Opt-in step reduction on a plateau for odam_sq_optimize_plateau[_host], as torch's ReduceLROnPlateau but per object:
+ * when the rule of odam_sq_convergence runs out of patience, the object's learning rates shrink by `factor` and the
+ * window restarts; only after R = max_reductions reductions does it stop.
+ *
+ * patience and rel_tol are those of odam_sq_convergence, keep as there, and all comparisons are in fp32:
+ *
+ *     best = +inf; b = -1; last = 0; r = 0
+ *     for k in 0 .. n_iters-1:
+ *         (iteration k at level r: loss L[k] at the current params, then the Adam step with both learning rates
+ *          scaled by s_r[k])
+ *         if isfinite(L[k]):
+ *             if b < 0 or L[k] < best * keep:  last = k            # as odam_sq_convergence, fp32
+ *             if b < 0 or L[k] < best:         best = L[k]; b = k
+ *         if k - last >= patience:
+ *             if r < R:  r += 1; last = k; reduce_iter[r-1] = k + 1   # the new level applies from iteration k+1
+ *             else:      stop; iters = k + 1
+ *
+ * best is not reset by a reduction, and the Adam step count and moments carry on unchanged.  The scale of level r is
+ * f_r = (float)pow((double)factor, r) (f_0 = 1), computed on the host, and s_r[k] = lr_scale[k] * f_r, an fp32
+ * product rounded to nearest (f_r when obj->lr_scale is NULL).  Iteration k at level r takes the Adam step sizes that
+ * odam_sq_optimize_objective takes for a schedule whose entry k is s_r[k]: an object re-run through that entry with
+ * lr_scale'[k] = s_{r(k)}[k], the scale it actually saw, reproduces its run bit for bit.  With R = 0 this is the rule
+ * of odam_sq_convergence.  The outputs of an object that stopped are those of odam_sq_convergence. */
+typedef struct odam_sq_plateau {
+    int max_reductions;         /* R: 1 .. 8                                                                       */
+    float factor;               /* finite, 0 < factor < 1: each reduction multiplies both learning rates by it       */
+    int32_t *out_reductions;    /* [n] reductions taken (may be NULL)                                              */
+    int32_t *out_reduce_iter;   /* [n][R] k + 1 of each reduction taken (its first iteration at the new level), -1
+                                   for those not taken (may be NULL)                                               */
+} odam_sq_plateau;
+
+/* odam_sq_optimize_converge[_host] with the step reduction above; plat == NULL is exactly that entry.  out_reductions
+ * and out_reduce_iter are device pointers for odam_sq_optimize_plateau and host pointers for the _host entry.  Besides
+ * the checks of odam_sq_optimize_converge[_host], ODAM_SQ_ERR_ARG (before any CUDA call) for plat with conv == NULL or
+ * conv->patience == 0, max_reductions outside 1 .. 8, and a factor that is not finite or outside (0, 1). */
+int odam_sq_optimize_plateau(const float *init, const int32_t *cls, const int32_t *view_off,
+                             const float *Ms, const float *box, const uint8_t *mask, const float *prior,
+                             int n, int n_iters, int representation, float lr, float lr_shape,
+                             float *out_params, float *out_loss, int32_t *out_status,
+                             const odam_sq_objective *obj, const odam_sq_convergence *conv,
+                             const odam_sq_plateau *plat, const odam_sq_options *opt, void *stream);
+int odam_sq_optimize_plateau_host(const float *init, const int32_t *cls, const int32_t *view_off,
+                                  const float *Ms, const float *box, const uint8_t *mask, const float *prior,
+                                  int n, int n_iters, int representation, float lr, float lr_shape,
+                                  float *out_params, float *out_loss, int32_t *out_status,
+                                  const odam_sq_objective *obj, const odam_sq_convergence *conv,
+                                  const odam_sq_plateau *plat, const odam_sq_options *opt, int device);
+
 /* compute_ellipsoid_points (sq_libs.py:577-595): params[n][9] -> xyz[n][1000][3] world points. */
 int odam_sq_sample_points(const float *params, int n, float *out_xyz, void *stream);
 int odam_sq_sample_points_host(const float *params, int n, float *out_xyz, int device);

@@ -40,6 +40,12 @@ class Convergence(C.Structure):
                 ("out_best_iter", C.c_void_p)]
 
 
+class Plateau(C.Structure):
+    """odam_sq_plateau (include/odam_sq.h)."""
+    _fields_ = [("max_reductions", C.c_int), ("factor", C.c_float), ("out_reductions", C.c_void_p),
+                ("out_reduce_iter", C.c_void_p)]
+
+
 class OdamSqError(RuntimeError):
     pass
 
@@ -59,6 +65,10 @@ ARGTYPES = {
     "odam_sq_optimize_converge": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Convergence), C.POINTER(Options), _vp],
     "odam_sq_optimize_converge_host": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Convergence), C.POINTER(Options),
                                                    _ci],
+    "odam_sq_optimize_plateau": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Convergence), C.POINTER(Plateau),
+                                             C.POINTER(Options), _vp],
+    "odam_sq_optimize_plateau_host": _OPT[:-1] + [C.POINTER(Objective), C.POINTER(Convergence), C.POINTER(Plateau),
+                                                  C.POINTER(Options), _ci],
     "odam_sq_sample_points": [_vp, _ci, _vp, _vp],
     "odam_sq_sample_points_host": [_vp, _ci, _vp, _ci],
     "odam_sq_project_boxes": [_vp, _vp, _vp, _ci, _vp, _vp],

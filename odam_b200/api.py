@@ -214,10 +214,30 @@ def _convergence(patience, rel_tol, keep_best, extras=()):
     return conv
 
 
+def _plateau(max_reductions, lr_factor, patience):
+    """odam_sq_plateau of the step-reduction keywords, or None when max_reductions is 0: then the entries without
+    reductions run.  patience has been checked by _convergence.  The output pointers are the caller's to set."""
+    if isinstance(max_reductions, bool) or not isinstance(max_reductions, (int, np.integer)) or \
+            not 0 <= max_reductions <= 8:
+        raise ValueError(f"max_reductions must be an integer in 0 .. 8, got {max_reductions!r}")
+    if max_reductions == 0:
+        if lr_factor is not None:
+            raise ValueError("lr_factor has no effect without max_reductions > 0")
+        return None
+    if patience == 0:
+        raise ValueError("max_reductions > 0 needs patience > 0: a reduction happens where early stopping would stop")
+    if lr_factor is None or isinstance(lr_factor, bool) or not isinstance(lr_factor, (int, float, np.number)) or \
+            not (np.isfinite(lr_factor) and 0.0 < np.float32(lr_factor) < 1.0):
+        raise ValueError(f"max_reductions > 0 needs an lr_factor, finite and in (0, 1), got {lr_factor!r}")
+    plat = _lib.Plateau()
+    plat.max_reductions, plat.factor = int(max_reductions), float(lr_factor)
+    return plat
+
+
 def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric", lr=0.01, lr_shape=0.1,
                   device=0, threads=0, max_slices=0, m0=None, v0=None, step0=0, s0=None, extras=(), cluster=0,
                   code_layout=0, side_weight=None, loss="l1", loss_scale=None, lr_scale=None, patience=0, rel_tol=0.0,
-                  keep_best=False):
+                  keep_best=False, max_reductions=0, lr_factor=None):
     """Run the fused optimiser on packed host arrays.  Returns dict(params[n,9], loss[n,n_iters], status[n], ...extras).
 
     prior: None (no prior term) or an [8,9] float32 table (see prior_table()).
@@ -236,6 +256,11 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
       The result then has iters[n] (iterations run) and best_iter[n] (iteration of the lowest finite loss, -1 if
       none), int32; the loss and out_param_hist rows of iterations not run are NaN.  out_pred, out_arg, out_eta_idx
       and out_grids cannot be asked for with it.
+    Step reduction on a plateau (odam_sq_plateau; needs patience > 0):
+      max_reductions: 1 .. 8; when an object runs out of patience, both its learning rates are multiplied by
+                      lr_factor (in (0, 1)) and its patience window restarts, up to max_reductions times; only then
+                      does it stop.  The result then also has reductions[n] (reductions taken) and reduce_iter[n,
+                      max_reductions] (the first iteration at each new step size, -1 for those not taken), int32.
     """
     L = _lib.load()
     init, cls, voff, Ms, box, mask = _track_arrays(tracks)
@@ -243,6 +268,7 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
     w = _lib.host_array("side_weight", side_weight, np.float32, (SV, 4))
     obj, _sched = _objective(_lib.ptr(w), loss, loss_scale, lr_scale, n_iters)
     conv = _convergence(patience, rel_tol, keep_best, extras)
+    plat = _plateau(max_reductions, lr_factor, patience)
     pr = _lib.host_array("prior", prior, np.float32, (8, 9))
     if pr is not None:
         check_classes(cls)
@@ -267,8 +293,11 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
     if conv is not None:
         out.update(iters=np.zeros(n, np.int32), best_iter=np.zeros(n, np.int32))
         conv.out_iters, conv.out_best_iter = _lib.ptr(out["iters"]), _lib.ptr(out["best_iter"])
-        rc = L.odam_sq_optimize_converge_host(*args, None if obj is None else C.byref(obj), C.byref(conv), C.byref(o),
-                                              device)
+        if plat is not None:
+            out.update(reductions=np.zeros(n, np.int32), reduce_iter=np.zeros((n, plat.max_reductions), np.int32))
+            plat.out_reductions, plat.out_reduce_iter = _lib.ptr(out["reductions"]), _lib.ptr(out["reduce_iter"])
+        rc = L.odam_sq_optimize_plateau_host(*args, None if obj is None else C.byref(obj), C.byref(conv),
+                                             None if plat is None else C.byref(plat), C.byref(o), device)
     elif obj is None:
         rc = L.odam_sq_optimize_host(*args, C.byref(o), device)
     else:
@@ -371,7 +400,8 @@ class DeviceTracks:
 
 def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr_shape=0.1, threads=0,
                     max_slices=0, out=None, cycles=None, cluster=0, code_layout=0, corners=None, side_weight=None,
-                    loss="l1", loss_scale=None, lr_scale=None, patience=0, rel_tol=0.0, keep_best=False):
+                    loss="l1", loss_scale=None, lr_scale=None, patience=0, rel_tol=0.0, keep_best=False,
+                    max_reductions=0, lr_factor=None):
     """Enqueue one fused launch on torch's current stream; returns dict of CUDA tensors (no sync).
     out: the dict of a previous call with the same n and n_iters, to be written again.
     cycles: optional int64 CUDA tensor [n, 16], per-phase SM cycles (diagnostics; slot names in tools/prof_run.py).
@@ -381,8 +411,11 @@ def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr
     [SV, 4] on the tracks' device, read in place and not validated (negative or non-finite weights are the caller's to
     exclude); lr_scale is a host array [n_iters].
     patience, rel_tol, keep_best: the early stopping of optimize_host; the result then has int32 CUDA tensors iters
-    [n] and best_iter [n] (added to `out` when it lacks them)."""
+    [n] and best_iter [n] (added to `out` when it lacks them).
+    max_reductions, lr_factor: the step reduction of optimize_host; the result then also has int32 CUDA tensors
+    reductions [n] and reduce_iter [n, max_reductions] (added to `out` when it lacks them)."""
     conv = _convergence(patience, rel_tol, keep_best, () if cycles is None else ("out_cycles",))
+    plat = _plateau(max_reductions, lr_factor, patience)
     torch = dt.torch
     dev = dt.init.device   # the tracks' device, with its index
     if side_weight is not None:
@@ -391,11 +424,14 @@ def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr
     shapes = dict(params=(torch.float32, (dt.n, 9)), loss=(torch.float32, (dt.n, n_iters)), status=(torch.int32, (dt.n,)))
     if conv is not None:
         shapes.update(iters=(torch.int32, (dt.n,)), best_iter=(torch.int32, (dt.n,)))
+    if plat is not None:
+        shapes.update(reductions=(torch.int32, (dt.n,)), reduce_iter=(torch.int32, (dt.n, plat.max_reductions)))
     if out is None:
         out = {k: torch.empty(shape, dtype=dtype, device=dev) for k, (dtype, shape) in shapes.items()}
     else:
-        if conv is not None:   # the dict of a call without early stopping
-            for k in ("iters", "best_iter"):
+        # the dict of a call without early stopping or without reductions
+        for k in ("iters", "best_iter", "reductions", "reduce_iter"):
+            if k in shapes:
                 out.setdefault(k, torch.empty(shapes[k][1], dtype=shapes[k][0], device=dev))
         for k, (dtype, shape) in shapes.items():
             _lib.check_tensor(f"out[{k!r}]", out[k], dtype, shape, dev)
@@ -419,8 +455,11 @@ def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr
     with torch.cuda.device(dev):
         if conv is not None:
             conv.out_iters, conv.out_best_iter = p(out["iters"]), p(out["best_iter"])
-            rc = L.odam_sq_optimize_converge(*args, None if obj is None else C.byref(obj), C.byref(conv), C.byref(o),
-                                             _lib.current_stream(dev))
+            if plat is not None:
+                plat.out_reductions, plat.out_reduce_iter = p(out["reductions"]), p(out["reduce_iter"])
+            rc = L.odam_sq_optimize_plateau(*args, None if obj is None else C.byref(obj), C.byref(conv),
+                                            None if plat is None else C.byref(plat), C.byref(o),
+                                            _lib.current_stream(dev))
         elif obj is None:
             rc = L.odam_sq_optimize(*args, C.byref(o), _lib.current_stream(dev))
         else:

@@ -73,7 +73,7 @@ struct OptArgs {
     const float *Ms; const float *box; const uint8_t *mask; const float *prior;
     int n, n_iters, optimize_shapes, max_slices, cluster, red_offset;
     int stage_offset, stage_views;   // >0: this many views per CTA fit the staging area at scratch + stage_offset
-    const float *adam_tab;  // [n_iters][4]: -lr/bc1, -lr_shape/bc1, sqrt(bc2), unused
+    const float *adam_tab;  // [max_reductions + 1][n_iters][4]: -lr/bc1, -lr_shape/bc1, sqrt(bc2), unused
     float beta1w, beta2, beta2w, eps;
     const float *m0, *v0, *s0;
     float *out_params, *out_loss; int32_t *out_status;
@@ -89,6 +89,9 @@ struct OptArgs {
     int patience, keep_best;
     float keep;                 // (float)(1 - rel_tol): L is a significant improvement when L < best * keep
     int32_t *out_iters, *out_best_iter;
+    // the plateau rule (odam_sq_plateau), appended likewise; 0 and NULL without it
+    int max_reductions;         // R: adam_tab holds one level of n_iters rows per step size, R + 1 in all
+    int32_t *out_reductions, *out_reduce_iter;
 };
 
 // The convergence build's per-object state, kept by the loss lane of phase G.  It lives in Smem::cyc, which the
@@ -101,6 +104,7 @@ struct ConvState {
     int b, last;      // its iteration (-1: none yet); the iteration of the last significant improvement
     int iters;        // iterations run so far
     int newbest, stop;
+    int r;            // kPlateau: the step-size level, i.e. reductions taken so far and the level of adam_tab in use
 };
 static_assert(sizeof(ConvState) <= sizeof(Smem::cyc), "ConvState must fit the cycle counters it reuses");
 
@@ -401,11 +405,15 @@ __device__ __forceinline__ void residual_loss(int kind, float s, float r, float 
 // the other builds form the reference's masked L1.
 // kConverge (only with kObjective): the build of odam_sq_optimize_converge, which stops an object once its loss stops
 // improving and keeps the lowest-loss iterate.  Until it stops, it runs the objective build's arithmetic.
+// kPlateau (only with kConverge): the build of odam_sq_optimize_plateau, which first shrinks the step of an object whose
+// loss stops improving, up to max_reductions times, and only then stops it.  A build of its own: the level costs the
+// convergence build 0.3 % at config 5 with no reduction asked for (DESIGN.md §12).
 template <int kMaxThreads, bool kCompact, bool kSolo = false, bool kProf = false, bool kObjective = false,
-          bool kConverge = false>
+          bool kConverge = false, bool kPlateau = false>
 __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact, kSolo)) sq_optimize_kernel(OptArgs A)
 {
     static_assert(!kConverge || kObjective, "the convergence build is an objective build");
+    static_assert(!kPlateau || kConverge, "the plateau build is a convergence build");
     // fixed state in static shared memory (compile-time addresses), per-launch scratch in dynamic shared memory
     __shared__ Smem S;
     ConvState &CV = *reinterpret_cast<ConvState *>(S.cyc);   // kConverge only, in place of the cycle counters
@@ -443,6 +451,7 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
         S.status = 0;
         if constexpr (kConverge) {
             CV.best = INFINITY; CV.b = -1; CV.last = 0; CV.iters = 0; CV.newbest = 0; CV.stop = 0;
+            if constexpr (kPlateau) CV.r = 0;
         } else {
             for (int k = 0; k < 16; k++) S.cyc[k] = 0;
         }
@@ -486,7 +495,14 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
 
     for (int it = 0; it < A.n_iters; it++) {
         // this iteration's Adam step sizes, fetched now: the load is off the critical path by the time phase G wants them
-        if (tid < 3) S.adam_now[tid] = A.adam_tab[it * 4 + tid];
+        if constexpr (kPlateau) {
+            // the row of this iteration at the object's step-size level (odam_sq_plateau).  CV.r changes only in phase
+            // G, behind the previous iteration's last barrier, and derives from the loss alone: every CTA of a cluster
+            // reads the same row (see the invariant at the end of the loop)
+            if (tid < 3) S.adam_now[tid] = A.adam_tab[((size_t)CV.r * A.n_iters + it) * 4 + tid];
+        } else {
+            if (tid < 3) S.adam_now[tid] = A.adam_tab[it * 4 + tid];
+        }
         sample_surface<kCompact>(S, reinterpret_cast<GridSpec *>(scratch_raw), tid, T, it > 0, prof);
         const bool last = it == A.n_iters - 1;
 
@@ -691,6 +707,13 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
                     CV.newbest = nb;
                     CV.iters = it + 1;
                     CV.stop = A.patience > 0 && it - CV.last >= A.patience;
+                    if constexpr (kPlateau) {
+                        if (CV.stop && CV.r < A.max_reductions) {   // reduce instead: the next level from it + 1
+                            CV.r++; CV.last = it; CV.stop = 0;
+                            if (crank == 0 && A.out_reduce_iter)
+                                A.out_reduce_iter[(size_t)obj * A.max_reductions + CV.r - 1] = it + 1;
+                        }
+                    }
                 }
                 if (!isfinite(loss)) atomicOr(&S.status, ODAM_SQ_ST_NONFINITE);
                 if (S.bad[0] | S.bad[1]) atomicOr(&S.status, ODAM_SQ_ST_SAMPLER);
@@ -725,7 +748,9 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
         if constexpr (kConverge) {
             // Invariant: every CTA of a cluster leaves the loop after the same iteration, here, behind the iteration's
             // last barrier.  CV.stop derives from the loss alone (phase G), which every CTA of the cluster computes
-            // identically; the exchange's mbarrier parities and the exit cluster.sync() depend on it.
+            // identically; the exchange's mbarrier parities and the exit cluster.sync() depend on it.  In the plateau
+            // build the step-size level CV.r is decided in the same place from the same loss, so every CTA of a
+            // cluster also fetches the same Adam row at the top of the next iteration and keeps identical parameters.
             if (CV.newbest && tid < 9) CV.bestp[tid] = CV.prev[tid];
             if (CV.stop) break;
         }
@@ -743,6 +768,12 @@ __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact,
                     A.out_param_hist[(size_t)obj * A.n_iters * 9 + i] = nan;
             if (tid == 0 && A.out_iters) A.out_iters[obj] = iters;
             if (tid == 0 && A.out_best_iter) A.out_best_iter[obj] = CV.b;
+            if constexpr (kPlateau) {
+                if (tid == 0 && A.out_reductions) A.out_reductions[obj] = CV.r;
+                if (A.out_reduce_iter)   // the reductions not taken; those taken were written as they happened
+                    for (int i = CV.r + tid; i < A.max_reductions; i += T)
+                        A.out_reduce_iter[(size_t)obj * A.max_reductions + i] = -1;
+            }
         }
     }
     if (tid < 9 && crank == 0) {
@@ -1001,8 +1032,9 @@ struct DeviceGuard {
 };
 
 struct AdamTab {   // bias-correction table of one (stream, schedule): kept until evicted, never shared across streams
-    cudaStream_t stream; int iters, step0; double lr, lrs; float *dev; int cap;
+    cudaStream_t stream; int iters, step0; double lr, lrs; float *dev; size_t cap;   // cap: rows
     std::vector<float> lr_scale;   // odam_sq_objective::lr_scale of the table (empty = constant)
+    int reductions; float factor;  // odam_sq_plateau: levels beyond the first and their factor; 0 and 1 without
 };
 
 struct DeviceState {
@@ -1021,19 +1053,27 @@ struct DeviceState {
 static DeviceState g_dev[64];
 static std::mutex g_mu;
 
-// lr_scale (NULL = constant): group["lr"] = lr * lr_scale[it] of a torch scheduler, in double as Python computes it
+// lr_scale (NULL = constant): group["lr"] = lr * lr_scale[it] of a torch scheduler, in double as Python computes it.
+// reductions = R > 0 (odam_sq_plateau): R + 1 levels of n_iters rows, level r being exactly the table of the schedule
+// s_r[it] = lr_scale[it] * f_r (an fp32 product, f_r = (float)factor^r), so that an object's run can be replayed
+// through the level-0 table of the schedule it saw.
 static void fill_adam_tab(std::vector<float> &tab, int n_iters, int step0, double lr, double lr_shape,
-                          const float *lr_scale = nullptr)
+                          const float *lr_scale = nullptr, int reductions = 0, float factor = 1.f)
 {
-    tab.resize((size_t)n_iters * 4);
-    for (int it = 0; it < n_iters; it++) {
-        double step = (double)(step0 + it + 1);
-        double bc1 = 1.0 - pow(0.9, step), bc2 = 1.0 - pow(0.999, step);
-        const double sc = lr_scale ? (double)lr_scale[it] : 1.0;
-        tab[it * 4 + 0] = (float)(-((lr * sc) / bc1));
-        tab[it * 4 + 1] = (float)(-((lr_shape * sc) / bc1));
-        tab[it * 4 + 2] = (float)pow(bc2, 0.5);
-        tab[it * 4 + 3] = 0.f;
+    tab.resize((size_t)(reductions + 1) * n_iters * 4);
+    for (int r = 0; r <= reductions; r++) {
+        const float f = (float)pow((double)factor, (double)r);
+        float *row = tab.data() + (size_t)r * n_iters * 4;
+        for (int it = 0; it < n_iters; it++) {
+            double step = (double)(step0 + it + 1);
+            double bc1 = 1.0 - pow(0.9, step), bc2 = 1.0 - pow(0.999, step);
+            const float s = lr_scale ? lr_scale[it] * f : f;   // level 0: lr_scale[it] (or 1) unchanged
+            const double sc = (double)s;
+            row[it * 4 + 0] = (float)(-((lr * sc) / bc1));
+            row[it * 4 + 1] = (float)(-((lr_shape * sc) / bc1));
+            row[it * 4 + 2] = (float)pow(bc2, 0.5);
+            row[it * 4 + 3] = 0.f;
+        }
     }
 }
 
@@ -1041,14 +1081,15 @@ static void fill_adam_tab(std::vector<float> &tab, int n_iters, int step0, doubl
 // floats); one cached table per (stream, schedule), so launches on different streams never share -- or overwrite --
 // each other's table
 static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, float lr, float lr_shape,
-                      const float *lr_scale, const float *&dev)
+                      const float *lr_scale, int reductions, float factor, const float *&dev)
 {
     std::lock_guard<std::mutex> lk(g_mu);
     dev = nullptr;
     const std::vector<float> sched = lr_scale ? std::vector<float>(lr_scale, lr_scale + n_iters) : std::vector<float>();
+    const size_t rows = (size_t)(reductions + 1) * n_iters;
     for (const AdamTab &t : D.tabs)
         if (t.stream == st && t.iters == n_iters && t.step0 == step0 && t.lr == (double)lr && t.lrs == (double)lr_shape &&
-            t.lr_scale == sched)
+            t.lr_scale == sched && t.reductions == reductions && t.factor == factor)
             dev = t.dev;
     if (dev) return ODAM_SQ_OK;
     AdamTab *slot = nullptr;
@@ -1057,21 +1098,21 @@ static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, f
     if (!slot && D.tabs.size() >= 16) slot = &D.tabs[0];  // bounded cache: recycle the oldest entry
     if (slot) {
         CU(cudaStreamSynchronize(slot->stream));          // its last launch may still read the table
-        if (slot->cap < n_iters) { cudaFree(slot->dev); slot->dev = nullptr; slot->cap = 0; }
+        if (slot->cap < rows) { cudaFree(slot->dev); slot->dev = nullptr; slot->cap = 0; }
     } else {
-        D.tabs.push_back(AdamTab{st, 0, 0, 0, 0, nullptr, 0, {}});
+        D.tabs.push_back(AdamTab{st, 0, 0, 0, 0, nullptr, 0, {}, 0, 1.f});
         slot = &D.tabs.back();
     }
     if (!slot->dev) {
-        CU(cudaMalloc(&slot->dev, sizeof(float) * 4 * n_iters));
-        slot->cap = n_iters;
+        CU(cudaMalloc(&slot->dev, sizeof(float) * 4 * rows));
+        slot->cap = rows;
     }
     std::vector<float> tab;
-    fill_adam_tab(tab, n_iters, step0, (double)lr, (double)lr_shape, lr_scale);
+    fill_adam_tab(tab, n_iters, step0, (double)lr, (double)lr_shape, lr_scale, reductions, factor);
     // pageable source: the copy has left the host vector when the call returns
     CU(cudaMemcpyAsync(slot->dev, tab.data(), sizeof(float) * tab.size(), cudaMemcpyHostToDevice, st));
     slot->stream = st; slot->iters = n_iters; slot->step0 = step0; slot->lr = (double)lr; slot->lrs = (double)lr_shape;
-    slot->lr_scale = sched;
+    slot->lr_scale = sched; slot->reductions = reductions; slot->factor = factor;
     dev = slot->dev;
     return ODAM_SQ_OK;
 }
@@ -1079,43 +1120,48 @@ static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, f
 using OptKernel = void (*)(OptArgs);
 
 // The builds of sq_optimize_kernel, each with its cycle-mark twin (prof), in ascending CTA size within each layout;
-// then the objective builds (weights and robust losses, odam_sq_optimize_objective), which have no twin, and their
-// convergence twins (odam_sq_optimize_converge).
+// then the objective builds (weights and robust losses, odam_sq_optimize_objective), which have no twin, their
+// convergence twins (odam_sq_optimize_converge) and the plateau twins of those (odam_sq_optimize_plateau).
 // Their register budget follows from __launch_bounds__: min_blocks() CTAs of `threads` share the 64K registers.
 // The compact layout only exists for CTAs of up to 256 threads (it is for many small CTAs per SM).
-struct OptBuild { int threads; bool compact, solo, prof, objective, converge; OptKernel kern; };
+struct OptBuild { int threads; bool compact, solo, prof, objective, converge, plateau; OptKernel kern; };
 static const OptBuild kOptBuilds[] = {
-    {256, false, false, false, false, false, sq_optimize_kernel<256, false, false, false>},
-    {512, false, false, false, false, false, sq_optimize_kernel<512, false, false, false>},
-    {1024, false, false, false, false, false, sq_optimize_kernel<1024, false, false, false>},
-    {256, true, false, false, false, false, sq_optimize_kernel<256, true, false, false>},
-    {512, false, true, false, false, false, sq_optimize_kernel<512, false, true, false>},
-    {256, false, false, true, false, false, sq_optimize_kernel<256, false, false, true>},
-    {512, false, false, true, false, false, sq_optimize_kernel<512, false, false, true>},
-    {1024, false, false, true, false, false, sq_optimize_kernel<1024, false, false, true>},
-    {256, true, false, true, false, false, sq_optimize_kernel<256, true, false, true>},
-    {512, false, true, true, false, false, sq_optimize_kernel<512, false, true, true>},
-    {256, false, false, false, true, false, sq_optimize_kernel<256, false, false, false, true>},
-    {512, false, false, false, true, false, sq_optimize_kernel<512, false, false, false, true>},
-    {1024, false, false, false, true, false, sq_optimize_kernel<1024, false, false, false, true>},
-    {256, true, false, false, true, false, sq_optimize_kernel<256, true, false, false, true>},
-    {512, false, true, false, true, false, sq_optimize_kernel<512, false, true, false, true>},
-    {256, false, false, false, true, true, sq_optimize_kernel<256, false, false, false, true, true>},
-    {512, false, false, false, true, true, sq_optimize_kernel<512, false, false, false, true, true>},
-    {1024, false, false, false, true, true, sq_optimize_kernel<1024, false, false, false, true, true>},
-    {256, true, false, false, true, true, sq_optimize_kernel<256, true, false, false, true, true>},
-    {512, false, true, false, true, true, sq_optimize_kernel<512, false, true, false, true, true>},
+    {256, false, false, false, false, false, false, sq_optimize_kernel<256, false, false, false>},
+    {512, false, false, false, false, false, false, sq_optimize_kernel<512, false, false, false>},
+    {1024, false, false, false, false, false, false, sq_optimize_kernel<1024, false, false, false>},
+    {256, true, false, false, false, false, false, sq_optimize_kernel<256, true, false, false>},
+    {512, false, true, false, false, false, false, sq_optimize_kernel<512, false, true, false>},
+    {256, false, false, true, false, false, false, sq_optimize_kernel<256, false, false, true>},
+    {512, false, false, true, false, false, false, sq_optimize_kernel<512, false, false, true>},
+    {1024, false, false, true, false, false, false, sq_optimize_kernel<1024, false, false, true>},
+    {256, true, false, true, false, false, false, sq_optimize_kernel<256, true, false, true>},
+    {512, false, true, true, false, false, false, sq_optimize_kernel<512, false, true, true>},
+    {256, false, false, false, true, false, false, sq_optimize_kernel<256, false, false, false, true>},
+    {512, false, false, false, true, false, false, sq_optimize_kernel<512, false, false, false, true>},
+    {1024, false, false, false, true, false, false, sq_optimize_kernel<1024, false, false, false, true>},
+    {256, true, false, false, true, false, false, sq_optimize_kernel<256, true, false, false, true>},
+    {512, false, true, false, true, false, false, sq_optimize_kernel<512, false, true, false, true>},
+    {256, false, false, false, true, true, false, sq_optimize_kernel<256, false, false, false, true, true>},
+    {512, false, false, false, true, true, false, sq_optimize_kernel<512, false, false, false, true, true>},
+    {1024, false, false, false, true, true, false, sq_optimize_kernel<1024, false, false, false, true, true>},
+    {256, true, false, false, true, true, false, sq_optimize_kernel<256, true, false, false, true, true>},
+    {512, false, true, false, true, true, false, sq_optimize_kernel<512, false, true, false, true, true>},
+    {256, false, false, false, true, true, true, sq_optimize_kernel<256, false, false, false, true, true, true>},
+    {512, false, false, false, true, true, true, sq_optimize_kernel<512, false, false, false, true, true, true>},
+    {1024, false, false, false, true, true, true, sq_optimize_kernel<1024, false, false, false, true, true, true>},
+    {256, true, false, false, true, true, true, sq_optimize_kernel<256, true, false, false, true, true, true>},
+    {512, false, true, false, true, true, true, sq_optimize_kernel<512, false, true, false, true, true, true>},
 };
 
 // the smallest build of the layout that fits `threads` CTA threads; the solo build when every CTA has an SM to itself
 // and it fits, else the shared one; NULL: no such build
 static const OptBuild *pick_build(int threads, bool compact, bool solo, bool prof, bool objective = false,
-                                  bool converge = false)
+                                  bool converge = false, bool plateau = false)
 {
     for (int want_solo = solo && !compact; want_solo >= 0; want_solo--)
         for (const OptBuild &B : kOptBuilds)
             if (B.compact == compact && B.solo == (bool)want_solo && B.prof == prof && B.objective == objective &&
-                B.converge == converge && threads <= B.threads)
+                B.converge == converge && B.plateau == plateau && threads <= B.threads)
                 return &B;
     return nullptr;
 }
@@ -1375,7 +1421,8 @@ static int launch_optimize(const OptArgs &A0, const LaunchCfg &L, cudaStream_t s
     A.stage_offset = L.stage_offset; A.stage_views = L.stage_views;
     if (A.out_status) CU(cudaMemsetAsync(A.out_status, 0, sizeof(int32_t) * A.n, st));  // CTAs OR their flags in
     OptKernel kern =
-        pick_build(L.threads, L.compact, L.solo, A.out_cycles != nullptr, objective_build(A), A.converge)->kern;
+        pick_build(L.threads, L.compact, L.solo, A.out_cycles != nullptr, objective_build(A), A.converge,
+                   A.max_reductions > 0)->kern;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof cfg);
     cfg.gridDim = dim3(A.n * L.cluster); cfg.blockDim = dim3(L.threads); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
@@ -1569,6 +1616,21 @@ static int convergence_args(const odam_sq_convergence *conv, const odam_sq_optio
     return ODAM_SQ_OK;
 }
 
+// plat (may be NULL) -> the plateau fields of A and the factor of the Adam table's levels (1 without), after the checks
+// include/odam_sq.h lists.  A reduction happens where the convergence rule would stop, so it needs a rule that can.
+static int plateau_args(const odam_sq_plateau *plat, const odam_sq_convergence *conv, OptArgs &A, float &factor)
+{
+    factor = 1.f;
+    if (!plat) return ODAM_SQ_OK;
+    if (!conv || conv->patience == 0 || plat->max_reductions < 1 || plat->max_reductions > 8 ||
+        !(std::isfinite(plat->factor) && plat->factor > 0.f && plat->factor < 1.f))
+        return ODAM_SQ_ERR_ARG;
+    A.max_reductions = plat->max_reductions;
+    A.out_reductions = plat->out_reductions; A.out_reduce_iter = plat->out_reduce_iter;
+    factor = plat->factor;
+    return ODAM_SQ_OK;
+}
+
 }  // namespace odam
 
 using namespace odam;
@@ -1660,12 +1722,24 @@ int odam_sq_optimize_converge(const float *init, const int32_t *cls, const int32
                               int32_t *out_status, const odam_sq_objective *obj, const odam_sq_convergence *conv,
                               const odam_sq_options *opt, void *stream)
 {
+    return odam_sq_optimize_plateau(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, lr, lr_shape,
+                                    out_params, out_loss, out_status, obj, conv, nullptr, opt, stream);
+}
+
+int odam_sq_optimize_plateau(const float *init, const int32_t *cls, const int32_t *view_off, const float *Ms,
+                             const float *box, const uint8_t *mask, const float *prior, int n, int n_iters,
+                             int representation, float lr, float lr_shape, float *out_params, float *out_loss,
+                             int32_t *out_status, const odam_sq_objective *obj, const odam_sq_convergence *conv,
+                             const odam_sq_plateau *plat, const odam_sq_options *opt, void *stream)
+{
     OptArgs A = opt_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
                          out_status, opt);
     const float *lr_scale;
+    float factor;
     int rc = check_opt_args(A, representation);
     if (!rc) rc = objective_args(obj, opt, A, lr_scale);
     if (!rc) rc = convergence_args(conv, opt, A);
+    if (!rc) rc = plateau_args(plat, conv, A, factor);
     if (rc || n_iters == 0) return rc;
     return on_current_device(n, [&](DeviceState &D) {
         cudaStream_t st = (cudaStream_t)stream;
@@ -1683,7 +1757,8 @@ int odam_sq_optimize_converge(const float *init, const int32_t *cls, const int32
         LaunchCfg L;
         rc = choose_launch(maxv, meanv, n, opt, D.sm_count, D.max_smem_optin, D.excl_clusters, L);
         if (rc) return rc;
-        rc = adam_table(D, st, n_iters, opt ? opt->step0 : 0, lr, lr_shape, lr_scale, A.adam_tab);
+        rc = adam_table(D, st, n_iters, opt ? opt->step0 : 0, lr, lr_shape, lr_scale, A.max_reductions, factor,
+                        A.adam_tab);
         if (rc) return rc;
         rc = launch_optimize(A, L, st);
         if (rc || !(opt && opt->out_corners)) return rc;
@@ -1774,12 +1849,24 @@ int odam_sq_optimize_converge_host(const float *init, const int32_t *cls, const 
                                    int32_t *out_status, const odam_sq_objective *obj,
                                    const odam_sq_convergence *conv, const odam_sq_options *opt, int device)
 {
+    return odam_sq_optimize_plateau_host(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, lr,
+                                         lr_shape, out_params, out_loss, out_status, obj, conv, nullptr, opt, device);
+}
+
+int odam_sq_optimize_plateau_host(const float *init, const int32_t *cls, const int32_t *view_off, const float *Ms,
+                                  const float *box, const uint8_t *mask, const float *prior, int n, int n_iters,
+                                  int representation, float lr, float lr_shape, float *out_params, float *out_loss,
+                                  int32_t *out_status, const odam_sq_objective *obj, const odam_sq_convergence *conv,
+                                  const odam_sq_plateau *plat, const odam_sq_options *opt, int device)
+{
     OptArgs A = opt_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
                          out_status, opt);
     const float *lr_scale;
+    float factor;
     int maxv, rc = check_opt_args(A, representation);
     if (!rc) rc = objective_args(obj, opt, A, lr_scale);
     if (!rc) rc = convergence_args(conv, opt, A);
+    if (!rc) rc = plateau_args(plat, conv, A, factor);
     if (rc || n == 0 || n_iters == 0) return rc;
     rc = check_view_off(view_off, n, maxv);
     if (rc) return rc;
@@ -1797,7 +1884,7 @@ int odam_sq_optimize_converge_host(const float *init, const int32_t *cls, const 
     rc = choose_launch(maxv, (double)SV / n, n, opt, D.sm_count, D.max_smem_optin, D.excl_clusters, L);
     if (rc) return rc;
     std::vector<float> tab;
-    fill_adam_tab(tab, n_iters, opt ? opt->step0 : 0, (double)lr, (double)lr_shape, lr_scale);
+    fill_adam_tab(tab, n_iters, opt ? opt->step0 : 0, (double)lr, (double)lr_shape, lr_scale, A.max_reductions, factor);
     A.adam_tab = tab.data();
     A.out_cycles = nullptr;   // a device-pointer option
     double *corners = opt ? opt->out_corners : nullptr;
@@ -1812,6 +1899,7 @@ int odam_sq_optimize_converge_host(const float *init, const int32_t *cls, const 
     S.out(A.out_eta_idx, (size_t)n * kN); S.out(A.out_grids, (size_t)n * 2 * kG);
     S.out(A.out_param_hist, n9 * n_iters); S.out(corners, (size_t)n * 24); S.out(box_flag, n);
     S.out(A.out_iters, n); S.out(A.out_best_iter, n);
+    S.out(A.out_reductions, n); S.out(A.out_reduce_iter, (size_t)n * A.max_reductions);
     return S.run(device, [&](cudaStream_t st) {
         rc = launch_optimize(A, L, st);
         if (rc || !corners) return rc;

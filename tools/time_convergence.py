@@ -1,7 +1,7 @@
-"""Device time and fit quality of the fused optimiser's early stopping (odam_sq_optimize_converge) against the default
-entry, with CUDA events.
+"""Device time and fit quality of the fused optimiser's early stopping (odam_sq_optimize_converge) and step reduction
+on a plateau (odam_sq_optimize_plateau) against the default entry, with CUDA events.
 
-    python tools/time_convergence.py [--configs 2,3,4,5] [--out profiles/converge_timing.txt]
+    python tools/time_convergence.py [--configs 2,3,4,5] [--out profiles/plateau_timing.txt]
 
 Per config (synthetic.make_config, its own iteration count and prior) every variant is launched device-resident
 (api.optimize_device, launch options fixed from the host copy of view_off):
@@ -9,10 +9,16 @@ Per config (synthetic.make_config, its own iteration count and prior) every vari
   never       the convergence build with patience 0: it never stops, so this is the cost of the build itself
   stop        patience 20, rel_tol 1e-3
   stop+best   the same, returning each object's lowest-loss iterate (keep_best)
-Every shape is warmed up first.  The variants alternate window by window in one process; each figure is the median
-over 7 windows of at least 100 ms.  Per variant the report gives the mean and largest iterations run and the median
-centre error (m) and relative dimension error against the scene's ground truth.  The card's name and power limit are
-printed in the same run."""
+  stop10      patience 10, rel_tol 1e-3: the stop rule at the patience of the step-reduction variants
+  p10 f.3 R2  patience 10, rel_tol 1e-3; on a plateau the step shrinks by 0.3, twice, before the object stops
+  (+best)     the same with keep_best
+  p10 f.5 R3  factor 0.5, three reductions
+  p20 f.3 R1  patience 20 (that of `stop`), one reduction by 0.3
+Every setting tried is reported.  Every shape is warmed up first.  The variants alternate window by window in one
+process; each figure is the median over 7 windows of at least 100 ms.  Per variant the report gives the mean and
+largest iterations run, the mean reductions taken, the median over objects of the ratio of the object's lowest loss
+to its lowest loss in the default run, and the median centre error (m) and relative dimension error against the
+scene's ground truth.  The card's name and power limit are printed in the same run."""
 import argparse
 import os
 import sys
@@ -26,7 +32,11 @@ from tools.time_autograd import card  # noqa: E402
 from tools.time_objective import window_ms  # noqa: E402
 
 VARIANTS = {"default": {}, "never": dict(patience=0, rel_tol=1e-3), "stop": dict(patience=20, rel_tol=1e-3),
-            "stop+best": dict(patience=20, rel_tol=1e-3, keep_best=True)}
+            "stop+best": dict(patience=20, rel_tol=1e-3, keep_best=True), "stop10": dict(patience=10, rel_tol=1e-3),
+            "p10 f.3 R2": dict(patience=10, rel_tol=1e-3, max_reductions=2, lr_factor=0.3),
+            "(+best)": dict(patience=10, rel_tol=1e-3, max_reductions=2, lr_factor=0.3, keep_best=True),
+            "p10 f.5 R3": dict(patience=10, rel_tol=1e-3, max_reductions=3, lr_factor=0.5),
+            "p20 f.3 R1": dict(patience=20, rel_tol=1e-3, max_reductions=1, lr_factor=0.3)}
 
 
 def errors(params, gt):
@@ -77,13 +87,18 @@ def main():
         lines.append(f"config {idx}: {cfg['name']}, {n_iters} iterations ({tracks.n} objects, {tracks.total_views} views, "
                      f"{q['threads']} threads, cluster {q['cluster']}, layout {q['code_layout']}; {reps} launches per "
                      f"window)")
+        lowest = lambda o: np.nanmin(o["loss"].cpu().numpy().astype(np.float64), axis=1)   # every first loss is run
+        low0 = lowest(outs["default"])
         for k, v in times.items():
             o = outs[k]
             iters = o["iters"].cpu().numpy() if "iters" in o else np.full(tracks.n, n_iters)
+            red = o["reductions"].cpu().numpy().mean() if "reductions" in o else 0.0
             ce, de = errors(o["params"].cpu().numpy(), scene.gt)
-            lines[-1] += (f"\n  {k:9s} {med[k]:9.3f} ms/launch (window spread {(max(v) - min(v)) / med[k] * 100:.1f} %)"
+            lines[-1] += (f"\n  {k:10s} {med[k]:9.3f} ms/launch (window spread {(max(v) - min(v)) / med[k] * 100:.1f} %)"
                           f"  speed-up {med['default'] / med[k]:.3f}  iterations mean {iters.mean():6.1f} max "
-                          f"{iters.max():3d}  median error centre {ce * 1000:.1f} mm, dims {100 * de:.2f} %")
+                          f"{iters.max():3d}  reductions mean {red:4.2f}  lowest loss / default's, median "
+                          f"{np.nanmedian(lowest(o) / low0):.4f}  median error centre {ce * 1000:.1f} mm, dims "
+                          f"{100 * de:.2f} %")
         print(lines[-1], flush=True)
         del dt, outs
         torch.cuda.empty_cache()
