@@ -234,6 +234,26 @@ def _plateau(max_reductions, lr_factor, patience):
     return plat
 
 
+def _opt_ins(n_iters, side_weight, loss, loss_scale, lr_scale, patience, rel_tol, keep_best, max_reductions,
+             lr_factor, extras):
+    """The optimiser's opt-in keywords as (the obj, conv and plat arguments of odam_sq_optimize_plateau[_host], or ()
+    when all are at their defaults: then odam_sq_optimize[_host] runs; the schedule array obj points into, which must
+    outlive the call; {name: (struct, shape)} of the int32 outputs the opt-ins add, each [n, *shape] and pointed at by
+    struct.out_<name>).  side_weight: the pointer the entry reads, or None.  Bad keywords are ValueErrors."""
+    conv = _convergence(patience, rel_tol, keep_best, extras)
+    plat = _plateau(max_reductions, lr_factor, patience)
+    obj, sched = _objective(side_weight, loss, loss_scale, lr_scale, n_iters)
+    outputs = {}
+    if conv is not None:
+        outputs.update(iters=(conv, ()), best_iter=(conv, ()))
+    if plat is not None:
+        outputs.update(reductions=(plat, ()), reduce_iter=(plat, (plat.max_reductions,)))
+    structs = (obj, conv, plat)
+    if structs == (None, None, None):
+        return (), sched, outputs
+    return tuple(None if s is None else C.byref(s) for s in structs), sched, outputs
+
+
 def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric", lr=0.01, lr_shape=0.1,
                   device=0, threads=0, max_slices=0, m0=None, v0=None, step0=0, s0=None, extras=(), cluster=0,
                   code_layout=0, side_weight=None, loss="l1", loss_scale=None, lr_scale=None, patience=0, rel_tol=0.0,
@@ -266,9 +286,8 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
     init, cls, voff, Ms, box, mask = _track_arrays(tracks)
     n, SV = len(init), int(voff[-1])
     w = _lib.host_array("side_weight", side_weight, np.float32, (SV, 4))
-    obj, _sched = _objective(_lib.ptr(w), loss, loss_scale, lr_scale, n_iters)
-    conv = _convergence(patience, rel_tol, keep_best, extras)
-    plat = _plateau(max_reductions, lr_factor, patience)
+    opt_in, _sched, outputs = _opt_ins(n_iters, _lib.ptr(w), loss, loss_scale, lr_scale, patience, rel_tol, keep_best,
+                                       max_reductions, lr_factor, extras)
     pr = _lib.host_array("prior", prior, np.float32, (8, 9))
     if pr is not None:
         check_classes(cls)
@@ -290,19 +309,11 @@ def optimize_host(tracks, prior=None, n_iters=200, representation="super_quadric
     args = (_lib.ptr(init), _lib.ptr(cls), _lib.ptr(voff), _lib.ptr(Ms), _lib.ptr(box), _lib.ptr(mask), _lib.ptr(pr),
             n, n_iters, _lib.REPR[representation], lr, lr_shape, _lib.ptr(out["params"]), _lib.ptr(out["loss"]),
             _lib.ptr(out["status"]))
-    if conv is not None:
-        out.update(iters=np.zeros(n, np.int32), best_iter=np.zeros(n, np.int32))
-        conv.out_iters, conv.out_best_iter = _lib.ptr(out["iters"]), _lib.ptr(out["best_iter"])
-        if plat is not None:
-            out.update(reductions=np.zeros(n, np.int32), reduce_iter=np.zeros((n, plat.max_reductions), np.int32))
-            plat.out_reductions, plat.out_reduce_iter = _lib.ptr(out["reductions"]), _lib.ptr(out["reduce_iter"])
-        rc = L.odam_sq_optimize_plateau_host(*args, None if obj is None else C.byref(obj), C.byref(conv),
-                                             None if plat is None else C.byref(plat), C.byref(o), device)
-    elif obj is None:
-        rc = L.odam_sq_optimize_host(*args, C.byref(o), device)
-    else:
-        rc = L.odam_sq_optimize_objective_host(*args, C.byref(obj), C.byref(o), device)
-    _lib.check(rc)
+    for name, (struct, shape) in outputs.items():
+        out[name] = np.zeros((n,) + shape, np.int32)
+        setattr(struct, "out_" + name, _lib.ptr(out[name]))
+    entry = L.odam_sq_optimize_plateau_host if opt_in else L.odam_sq_optimize_host
+    _lib.check(entry(*args, *opt_in, C.byref(o), device))
     out.update((name, keep[name]) for name in extras)
     return out
 
@@ -414,25 +425,21 @@ def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr
     [n] and best_iter [n] (added to `out` when it lacks them).
     max_reductions, lr_factor: the step reduction of optimize_host; the result then also has int32 CUDA tensors
     reductions [n] and reduce_iter [n, max_reductions] (added to `out` when it lacks them)."""
-    conv = _convergence(patience, rel_tol, keep_best, () if cycles is None else ("out_cycles",))
-    plat = _plateau(max_reductions, lr_factor, patience)
+    opt_in, _sched, outputs = _opt_ins(n_iters, _lib.tensor_ptr(side_weight), loss, loss_scale, lr_scale, patience,
+                                       rel_tol, keep_best, max_reductions, lr_factor,
+                                       () if cycles is None else ("out_cycles",))
     torch = dt.torch
     dev = dt.init.device   # the tracks' device, with its index
     if side_weight is not None:
         _lib.check_tensor("side_weight", side_weight, torch.float32, (dt.total_views, 4), dev)
-    obj, _sched = _objective(_lib.tensor_ptr(side_weight), loss, loss_scale, lr_scale, n_iters)
     shapes = dict(params=(torch.float32, (dt.n, 9)), loss=(torch.float32, (dt.n, n_iters)), status=(torch.int32, (dt.n,)))
-    if conv is not None:
-        shapes.update(iters=(torch.int32, (dt.n,)), best_iter=(torch.int32, (dt.n,)))
-    if plat is not None:
-        shapes.update(reductions=(torch.int32, (dt.n,)), reduce_iter=(torch.int32, (dt.n, plat.max_reductions)))
+    shapes.update((k, (torch.int32, (dt.n,) + shape)) for k, (_, shape) in outputs.items())
     if out is None:
         out = {k: torch.empty(shape, dtype=dtype, device=dev) for k, (dtype, shape) in shapes.items()}
     else:
-        # the dict of a call without early stopping or without reductions
-        for k in ("iters", "best_iter", "reductions", "reduce_iter"):
-            if k in shapes:
-                out.setdefault(k, torch.empty(shapes[k][1], dtype=shapes[k][0], device=dev))
+        # the dict of a call without some of these opt-ins
+        for k in outputs:
+            out.setdefault(k, torch.empty(shapes[k][1], dtype=torch.int32, device=dev))
         for k, (dtype, shape) in shapes.items():
             _lib.check_tensor(f"out[{k!r}]", out[k], dtype, shape, dev)
     if cycles is not None:
@@ -451,19 +458,12 @@ def optimize_device(dt, n_iters=200, representation="super_quadric", lr=0.01, lr
     o.out_cycles, o.out_corners = p(cycles), p(corners)
     args = (p(dt.init), p(dt.cls), p(dt.view_off), p(dt.Ms), p(dt.box), p(dt.mask), p(dt.prior), dt.n, n_iters,
             _lib.REPR[representation], lr, lr_shape, p(out["params"]), p(out["loss"]), p(out["status"]))
+    for k, (struct, _) in outputs.items():
+        setattr(struct, "out_" + k, p(out[k]))
     L = _lib.load()
+    entry = L.odam_sq_optimize_plateau if opt_in else L.odam_sq_optimize
     with torch.cuda.device(dev):
-        if conv is not None:
-            conv.out_iters, conv.out_best_iter = p(out["iters"]), p(out["best_iter"])
-            if plat is not None:
-                plat.out_reductions, plat.out_reduce_iter = p(out["reductions"]), p(out["reduce_iter"])
-            rc = L.odam_sq_optimize_plateau(*args, None if obj is None else C.byref(obj), C.byref(conv),
-                                            None if plat is None else C.byref(plat), C.byref(o),
-                                            _lib.current_stream(dev))
-        elif obj is None:
-            rc = L.odam_sq_optimize(*args, C.byref(o), _lib.current_stream(dev))
-        else:
-            rc = L.odam_sq_optimize_objective(*args, C.byref(obj), C.byref(o), _lib.current_stream(dev))
+        rc = entry(*args, *opt_in, C.byref(o), _lib.current_stream(dev))
     _lib.check(rc)
     return out
 

@@ -397,23 +397,32 @@ __device__ __forceinline__ void residual_loss(int kind, float s, float r, float 
     }
 }
 
+// What a build of sq_optimize_kernel computes besides the reference's optimisation.  Each variant from Objective on
+// does everything the one before it does, and variant_of() picks the variant of a call.
+enum class Variant {
+    // the reference: masked L1 at the Adam table's step sizes
+    Reference,
+    // the reference plus the per-phase cycle counts (odam_sq_options::out_cycles).  The marks are compiled out of the
+    // other builds: a predicate test, a branch and a volatile clock read at 15 places cost 2.6 % (config 2) to 4.8 %
+    // (config 5) of the throughput even when no count is taken.
+    Prof,
+    // odam_sq_optimize_objective: per-side weights and a robust residual loss (phase F only)
+    Objective,
+    // odam_sq_optimize_converge: stops an object once its loss stops improving and keeps the lowest-loss iterate.
+    // Until it stops, it runs the objective's arithmetic.
+    Converge,
+    // odam_sq_optimize_plateau: first shrinks the step of an object whose loss stops improving, up to max_reductions
+    // times, and only then stops it.  A variant of its own: the level costs the convergence build 0.3 % at config 5
+    // with no reduction asked for (DESIGN.md §12).
+    Plateau,
+};
+
 // kCompact selects the small-instruction-footprint build (odam_sq_options::code_layout): same arithmetic either way.
-// kProf: the instantiation that accumulates the per-phase cycle counts (odam_sq_options::out_cycles).  The marks are
-// compiled out of the production kernels: a predicate test, a branch and a volatile clock read at 15 places cost
-// 2.6 % (config 2) to 4.8 % (config 5) of the throughput even when no count is taken.
-// kObjective: the build of odam_sq_optimize_objective with per-side weights and a robust residual loss (phase F only);
-// the other builds form the reference's masked L1.
-// kConverge (only with kObjective): the build of odam_sq_optimize_converge, which stops an object once its loss stops
-// improving and keeps the lowest-loss iterate.  Until it stops, it runs the objective build's arithmetic.
-// kPlateau (only with kConverge): the build of odam_sq_optimize_plateau, which first shrinks the step of an object whose
-// loss stops improving, up to max_reductions times, and only then stops it.  A build of its own: the level costs the
-// convergence build 0.3 % at config 5 with no reduction asked for (DESIGN.md §12).
-template <int kMaxThreads, bool kCompact, bool kSolo = false, bool kProf = false, bool kObjective = false,
-          bool kConverge = false, bool kPlateau = false>
+template <int kMaxThreads, bool kCompact, bool kSolo, Variant kV>
 __global__ void __launch_bounds__(kMaxThreads, min_blocks(kMaxThreads, kCompact, kSolo)) sq_optimize_kernel(OptArgs A)
 {
-    static_assert(!kConverge || kObjective, "the convergence build is an objective build");
-    static_assert(!kPlateau || kConverge, "the plateau build is a convergence build");
+    constexpr bool kProf = kV == Variant::Prof, kObjective = kV >= Variant::Objective;
+    constexpr bool kConverge = kV >= Variant::Converge, kPlateau = kV == Variant::Plateau;
     // fixed state in static shared memory (compile-time addresses), per-launch scratch in dynamic shared memory
     __shared__ Smem S;
     ConvState &CV = *reinterpret_cast<ConvState *>(S.cyc);   // kConverge only, in place of the cycle counters
@@ -1119,55 +1128,41 @@ static int adam_table(DeviceState &D, cudaStream_t st, int n_iters, int step0, f
 
 using OptKernel = void (*)(OptArgs);
 
-// The builds of sq_optimize_kernel, each with its cycle-mark twin (prof), in ascending CTA size within each layout;
-// then the objective builds (weights and robust losses, odam_sq_optimize_objective), which have no twin, their
-// convergence twins (odam_sq_optimize_converge) and the plateau twins of those (odam_sq_optimize_plateau).
-// Their register budget follows from __launch_bounds__: min_blocks() CTAs of `threads` share the 64K registers.
-// The compact layout only exists for CTAs of up to 256 threads (it is for many small CTAs per SM).
-struct OptBuild { int threads; bool compact, solo, prof, objective, converge, plateau; OptKernel kern; };
+// The builds of sq_optimize_kernel: every variant of each production shape, the shapes in ascending CTA size within
+// each layout.  Their register budget follows from __launch_bounds__: min_blocks() CTAs of `threads` share the 64K
+// registers.  The compact layout only exists for CTAs of up to 256 threads (it is for many small CTAs per SM).
+struct OptBuild { int threads; bool compact, solo; Variant variant; OptKernel kern; };
+#define SQ_OPT_SHAPES(V)                                                                                  \
+    {256, false, false, V, sq_optimize_kernel<256, false, false, V>},                                    \
+    {512, false, false, V, sq_optimize_kernel<512, false, false, V>},                                    \
+    {1024, false, false, V, sq_optimize_kernel<1024, false, false, V>},                                  \
+    {256, true, false, V, sq_optimize_kernel<256, true, false, V>},                                      \
+    {512, false, true, V, sq_optimize_kernel<512, false, true, V>}
 static const OptBuild kOptBuilds[] = {
-    {256, false, false, false, false, false, false, sq_optimize_kernel<256, false, false, false>},
-    {512, false, false, false, false, false, false, sq_optimize_kernel<512, false, false, false>},
-    {1024, false, false, false, false, false, false, sq_optimize_kernel<1024, false, false, false>},
-    {256, true, false, false, false, false, false, sq_optimize_kernel<256, true, false, false>},
-    {512, false, true, false, false, false, false, sq_optimize_kernel<512, false, true, false>},
-    {256, false, false, true, false, false, false, sq_optimize_kernel<256, false, false, true>},
-    {512, false, false, true, false, false, false, sq_optimize_kernel<512, false, false, true>},
-    {1024, false, false, true, false, false, false, sq_optimize_kernel<1024, false, false, true>},
-    {256, true, false, true, false, false, false, sq_optimize_kernel<256, true, false, true>},
-    {512, false, true, true, false, false, false, sq_optimize_kernel<512, false, true, true>},
-    {256, false, false, false, true, false, false, sq_optimize_kernel<256, false, false, false, true>},
-    {512, false, false, false, true, false, false, sq_optimize_kernel<512, false, false, false, true>},
-    {1024, false, false, false, true, false, false, sq_optimize_kernel<1024, false, false, false, true>},
-    {256, true, false, false, true, false, false, sq_optimize_kernel<256, true, false, false, true>},
-    {512, false, true, false, true, false, false, sq_optimize_kernel<512, false, true, false, true>},
-    {256, false, false, false, true, true, false, sq_optimize_kernel<256, false, false, false, true, true>},
-    {512, false, false, false, true, true, false, sq_optimize_kernel<512, false, false, false, true, true>},
-    {1024, false, false, false, true, true, false, sq_optimize_kernel<1024, false, false, false, true, true>},
-    {256, true, false, false, true, true, false, sq_optimize_kernel<256, true, false, false, true, true>},
-    {512, false, true, false, true, true, false, sq_optimize_kernel<512, false, true, false, true, true>},
-    {256, false, false, false, true, true, true, sq_optimize_kernel<256, false, false, false, true, true, true>},
-    {512, false, false, false, true, true, true, sq_optimize_kernel<512, false, false, false, true, true, true>},
-    {1024, false, false, false, true, true, true, sq_optimize_kernel<1024, false, false, false, true, true, true>},
-    {256, true, false, false, true, true, true, sq_optimize_kernel<256, true, false, false, true, true, true>},
-    {512, false, true, false, true, true, true, sq_optimize_kernel<512, false, true, false, true, true, true>},
+    SQ_OPT_SHAPES(Variant::Reference), SQ_OPT_SHAPES(Variant::Prof), SQ_OPT_SHAPES(Variant::Objective),
+    SQ_OPT_SHAPES(Variant::Converge), SQ_OPT_SHAPES(Variant::Plateau),
 };
+#undef SQ_OPT_SHAPES
 
-// the smallest build of the layout that fits `threads` CTA threads; the solo build when every CTA has an SM to itself
-// and it fits, else the shared one; NULL: no such build
-static const OptBuild *pick_build(int threads, bool compact, bool solo, bool prof, bool objective = false,
-                                  bool converge = false, bool plateau = false)
+// the smallest build of the layout and variant that fits `threads` CTA threads; the solo build when every CTA has an
+// SM to itself and it fits, else the shared one; NULL: no such build
+static const OptBuild *pick_build(int threads, bool compact, bool solo, Variant v = Variant::Reference)
 {
     for (int want_solo = solo && !compact; want_solo >= 0; want_solo--)
         for (const OptBuild &B : kOptBuilds)
-            if (B.compact == compact && B.solo == (bool)want_solo && B.prof == prof && B.objective == objective &&
-                B.converge == converge && B.plateau == plateau && threads <= B.threads)
+            if (B.compact == compact && B.solo == (bool)want_solo && B.variant == v && threads <= B.threads)
                 return &B;
     return nullptr;
 }
 
-// whether a launch with these arguments runs an objective build (every convergence build is one)
-static bool objective_build(const OptArgs &A) { return A.side_weight || A.loss_kind != ODAM_SQ_LOSS_L1 || A.converge; }
+// the variant a call with these arguments runs: the least one that computes everything it asks for
+static Variant variant_of(const OptArgs &A)
+{
+    if (A.max_reductions > 0) return Variant::Plateau;
+    if (A.converge) return Variant::Converge;
+    if (A.side_weight || A.loss_kind != ODAM_SQ_LOSS_L1) return Variant::Objective;
+    return A.out_cycles ? Variant::Prof : Variant::Reference;
+}
 
 static int opt_regs(const OptBuild &B) { return 65536 / (B.threads * min_blocks(B.threads, B.compact, B.solo)); }
 
@@ -1224,7 +1219,7 @@ static int ensure_init(int device)
         attr.val.clusterDim.x = c; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
         cfg.attrs = &attr; cfg.numAttrs = 1;
         int num = 0;
-        if (cudaOccupancyMaxActiveClusters(&num, pick_build(512, false, false, false)->kern, &cfg) == cudaSuccess)
+        if (cudaOccupancyMaxActiveClusters(&num, pick_build(512, false, false)->kern, &cfg) == cudaSuccess)
             D.excl_clusters[c] = num;
         else cudaGetLastError();
     }
@@ -1389,7 +1384,7 @@ static int choose_launch(int max_views, double mean_views, int n, const odam_sq_
     if (threads % 32 || threads < 64 || threads > 1024) return ODAM_SQ_ERR_ARG;  // two warps share the sampler's tail
     // a layout with no build of this CTA size (the compact one above 256 threads, also when it was asked for with
     // threads chosen here): every configuration this returns has a build, and pick_build() relies on it
-    if (!pick_build(threads, layout == 2, !dense, false)) return ODAM_SQ_ERR_ARG;
+    if (!pick_build(threads, layout == 2, !dense)) return ODAM_SQ_ERR_ARG;
     long items = std::max(threads, max_views);  // V * min(max_slices, threads / V) <= threads when V <= threads
     long red_offset = std::max<long>(items * 4 * 8, (long)kSpecBytes);  // phase-E results alias the B0 scratch
     long smem = red_offset + (threads / 32) * (kRed + 3) * 4;            // + cross-warp reduction rows
@@ -1420,9 +1415,7 @@ static int launch_optimize(const OptArgs &A0, const LaunchCfg &L, cudaStream_t s
     A.red_offset = L.red_offset;
     A.stage_offset = L.stage_offset; A.stage_views = L.stage_views;
     if (A.out_status) CU(cudaMemsetAsync(A.out_status, 0, sizeof(int32_t) * A.n, st));  // CTAs OR their flags in
-    OptKernel kern =
-        pick_build(L.threads, L.compact, L.solo, A.out_cycles != nullptr, objective_build(A), A.converge,
-                   A.max_reductions > 0)->kern;
+    OptKernel kern = pick_build(L.threads, L.compact, L.solo, variant_of(A))->kern;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof cfg);
     cfg.gridDim = dim3(A.n * L.cluster); cfg.blockDim = dim3(L.threads); cfg.dynamicSmemBytes = L.smem; cfg.stream = st;
@@ -1553,12 +1546,16 @@ static int check_sides_vjp(const float *params, const int32_t *view_off, const f
                                                                                                   : ODAM_SQ_OK;
 }
 
-// the arguments of odam_sq_optimize(_host); the launch fields and adam_tab are set later
-static OptArgs opt_args(const float *init, const int32_t *cls, const int32_t *view_off, const float *Ms, const float *box,
-                        const uint8_t *mask, const float *prior, int n, int n_iters, int representation,
-                        float *out_params, float *out_loss, int32_t *out_status, const odam_sq_options *opt)
+// The arguments of odam_sq_optimize_plateau(_host) -> A (its launch fields and adam_tab are set later), the host
+// schedule and the factor of the Adam table's levels (1 without reductions), after the checks include/odam_sq.h lists
+// for both entries and before any CUDA call.  The host entry checks its weights itself, once it knows how many views
+// there are.
+static int optimize_args(const float *init, const int32_t *cls, const int32_t *view_off, const float *Ms,
+                         const float *box, const uint8_t *mask, const float *prior, int n, int n_iters,
+                         int representation, float *out_params, float *out_loss, int32_t *out_status,
+                         const odam_sq_objective *obj, const odam_sq_convergence *conv, const odam_sq_plateau *plat,
+                         const odam_sq_options *opt, OptArgs &A, const float *&lr_scale, float &factor)
 {
-    OptArgs A;
     memset(&A, 0, sizeof A);
     A.init = init; A.cls = cls; A.view_off = view_off; A.Ms = Ms; A.box = box; A.mask = mask; A.prior = prior;
     A.n = n; A.n_iters = n_iters; A.optimize_shapes = representation == ODAM_SQ_REPR_SUPER_QUADRIC;
@@ -1570,64 +1567,43 @@ static OptArgs opt_args(const float *init, const int32_t *cls, const int32_t *vi
         A.out_param_hist = opt->out_param_hist;
         A.out_cycles = (long long *)opt->out_cycles;
     }
-    return A;
-}
-
-static int check_opt_args(const OptArgs &A, int representation)
-{
-    if (!A.init || !A.view_off || !A.Ms || !A.box || !A.mask || !A.out_params || !A.out_loss || A.n < 0 || A.n_iters < 0)
-        return ODAM_SQ_ERR_ARG;
-    if (A.prior && !A.cls) return ODAM_SQ_ERR_ARG;
-    if (representation < 0 || representation > 2) return ODAM_SQ_ERR_ARG;
-    return ODAM_SQ_OK;
-}
-
-// obj (may be NULL) -> the objective fields of A and the host schedule, after the checks include/odam_sq.h lists for
-// both entries (the host entry checks its weights itself, once it knows how many views there are)
-static int objective_args(const odam_sq_objective *obj, const odam_sq_options *opt, OptArgs &A, const float *&lr_scale)
-{
     lr_scale = nullptr;
-    if (!obj) return ODAM_SQ_OK;
-    const bool robust = obj->loss != ODAM_SQ_LOSS_L1;
-    if (obj->loss < ODAM_SQ_LOSS_L1 || obj->loss > ODAM_SQ_LOSS_CAUCHY) return ODAM_SQ_ERR_ARG;
-    if (robust && !(std::isfinite(obj->loss_scale) && obj->loss_scale > 0.f)) return ODAM_SQ_ERR_ARG;
-    if (obj->lr_scale)
-        for (int it = 0; it < A.n_iters; it++)
-            if (!(std::isfinite(obj->lr_scale[it]) && obj->lr_scale[it] >= 0.f)) return ODAM_SQ_ERR_ARG;
-    A.side_weight = obj->side_weight; A.loss_kind = obj->loss; A.loss_scale = robust ? obj->loss_scale : 0.f;
-    if (objective_build(A) && opt && opt->out_cycles) return ODAM_SQ_ERR_ARG;   // no cycle-mark twin
-    lr_scale = obj->lr_scale;
-    return ODAM_SQ_OK;
-}
-
-// conv (may be NULL) -> the convergence fields of A, after the checks include/odam_sq.h lists.  The options that
-// describe the last iteration are refused with it: the kernel knows which iteration is the last only once it has run it.
-static int convergence_args(const odam_sq_convergence *conv, const odam_sq_options *opt, OptArgs &A)
-{
-    if (!conv) return ODAM_SQ_OK;
-    if (conv->patience < 0 || !(std::isfinite(conv->rel_tol) && conv->rel_tol >= 0.f && conv->rel_tol < 1.f) ||
-        (conv->keep_best != 0 && conv->keep_best != 1))
-        return ODAM_SQ_ERR_ARG;
-    if (opt && (opt->out_pred || opt->out_arg || opt->out_eta_idx || opt->out_grids || opt->out_cycles))
-        return ODAM_SQ_ERR_ARG;
-    A.converge = 1; A.patience = conv->patience; A.keep_best = conv->keep_best;
-    A.keep = (float)(1.0 - (double)conv->rel_tol);
-    A.out_iters = conv->out_iters; A.out_best_iter = conv->out_best_iter;
-    return ODAM_SQ_OK;
-}
-
-// plat (may be NULL) -> the plateau fields of A and the factor of the Adam table's levels (1 without), after the checks
-// include/odam_sq.h lists.  A reduction happens where the convergence rule would stop, so it needs a rule that can.
-static int plateau_args(const odam_sq_plateau *plat, const odam_sq_convergence *conv, OptArgs &A, float &factor)
-{
     factor = 1.f;
-    if (!plat) return ODAM_SQ_OK;
-    if (!conv || conv->patience == 0 || plat->max_reductions < 1 || plat->max_reductions > 8 ||
-        !(std::isfinite(plat->factor) && plat->factor > 0.f && plat->factor < 1.f))
+    if (!init || !view_off || !Ms || !box || !mask || !out_params || !out_loss || n < 0 || n_iters < 0)
         return ODAM_SQ_ERR_ARG;
-    A.max_reductions = plat->max_reductions;
-    A.out_reductions = plat->out_reductions; A.out_reduce_iter = plat->out_reduce_iter;
-    factor = plat->factor;
+    if (prior && !cls) return ODAM_SQ_ERR_ARG;
+    if (representation < 0 || representation > 2) return ODAM_SQ_ERR_ARG;
+    if (obj) {
+        const bool robust = obj->loss != ODAM_SQ_LOSS_L1;
+        if (obj->loss < ODAM_SQ_LOSS_L1 || obj->loss > ODAM_SQ_LOSS_CAUCHY) return ODAM_SQ_ERR_ARG;
+        if (robust && !(std::isfinite(obj->loss_scale) && obj->loss_scale > 0.f)) return ODAM_SQ_ERR_ARG;
+        if (obj->lr_scale)
+            for (int it = 0; it < n_iters; it++)
+                if (!(std::isfinite(obj->lr_scale[it]) && obj->lr_scale[it] >= 0.f)) return ODAM_SQ_ERR_ARG;
+        A.side_weight = obj->side_weight; A.loss_kind = obj->loss; A.loss_scale = robust ? obj->loss_scale : 0.f;
+        lr_scale = obj->lr_scale;
+    }
+    if (conv) {
+        if (conv->patience < 0 || !(std::isfinite(conv->rel_tol) && conv->rel_tol >= 0.f && conv->rel_tol < 1.f) ||
+            (conv->keep_best != 0 && conv->keep_best != 1))
+            return ODAM_SQ_ERR_ARG;
+        // the options that describe the last iteration: the kernel knows which iteration is the last only once it
+        // has run it
+        if (A.out_pred || A.out_arg || A.out_eta_idx || A.out_grids) return ODAM_SQ_ERR_ARG;
+        A.converge = 1; A.patience = conv->patience; A.keep_best = conv->keep_best;
+        A.keep = (float)(1.0 - (double)conv->rel_tol);
+        A.out_iters = conv->out_iters; A.out_best_iter = conv->out_best_iter;
+    }
+    if (plat) {
+        // a reduction happens where the convergence rule would stop, so it needs a rule that can
+        if (!conv || conv->patience == 0 || plat->max_reductions < 1 || plat->max_reductions > 8 ||
+            !(std::isfinite(plat->factor) && plat->factor > 0.f && plat->factor < 1.f))
+            return ODAM_SQ_ERR_ARG;
+        A.max_reductions = plat->max_reductions;
+        A.out_reductions = plat->out_reductions; A.out_reduce_iter = plat->out_reduce_iter;
+        factor = plat->factor;
+    }
+    if (A.out_cycles && variant_of(A) >= Variant::Objective) return ODAM_SQ_ERR_ARG;   // cycle marks: Prof only
     return ODAM_SQ_OK;
 }
 
@@ -1690,7 +1666,7 @@ int odam_sq_query_launch(const int32_t *view_off, int n, const odam_sq_options *
     if (max_slices) *max_slices = L.max_slices;
     if (smem_bytes) *smem_bytes = L.smem;
     if (smem_bytes) *smem_bytes += (int)sizeof(Smem);
-    const int regs = opt_regs(*pick_build(L.threads, L.compact, L.solo, false));
+    const int regs = opt_regs(*pick_build(L.threads, L.compact, L.solo));
     if (ctas_per_sm) *ctas_per_sm = std::min({32, 2048 / L.threads, 65536 / (regs * L.threads), (233472 - 1024) / (L.smem + (int)sizeof(Smem) + 1024)});
     return ODAM_SQ_OK;
 }
@@ -1732,14 +1708,11 @@ int odam_sq_optimize_plateau(const float *init, const int32_t *cls, const int32_
                              int32_t *out_status, const odam_sq_objective *obj, const odam_sq_convergence *conv,
                              const odam_sq_plateau *plat, const odam_sq_options *opt, void *stream)
 {
-    OptArgs A = opt_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
-                         out_status, opt);
+    OptArgs A;
     const float *lr_scale;
     float factor;
-    int rc = check_opt_args(A, representation);
-    if (!rc) rc = objective_args(obj, opt, A, lr_scale);
-    if (!rc) rc = convergence_args(conv, opt, A);
-    if (!rc) rc = plateau_args(plat, conv, A, factor);
+    int rc = optimize_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
+                           out_status, obj, conv, plat, opt, A, lr_scale, factor);
     if (rc || n_iters == 0) return rc;
     return on_current_device(n, [&](DeviceState &D) {
         cudaStream_t st = (cudaStream_t)stream;
@@ -1859,14 +1832,11 @@ int odam_sq_optimize_plateau_host(const float *init, const int32_t *cls, const i
                                   int32_t *out_status, const odam_sq_objective *obj, const odam_sq_convergence *conv,
                                   const odam_sq_plateau *plat, const odam_sq_options *opt, int device)
 {
-    OptArgs A = opt_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params, out_loss,
-                         out_status, opt);
+    OptArgs A;
     const float *lr_scale;
     float factor;
-    int maxv, rc = check_opt_args(A, representation);
-    if (!rc) rc = objective_args(obj, opt, A, lr_scale);
-    if (!rc) rc = convergence_args(conv, opt, A);
-    if (!rc) rc = plateau_args(plat, conv, A, factor);
+    int maxv, rc = optimize_args(init, cls, view_off, Ms, box, mask, prior, n, n_iters, representation, out_params,
+                                 out_loss, out_status, obj, conv, plat, opt, A, lr_scale, factor);
     if (rc || n == 0 || n_iters == 0) return rc;
     rc = check_view_off(view_off, n, maxv);
     if (rc) return rc;

@@ -21,7 +21,7 @@ import pytest
 from convergence_rule import stop_rule
 from launch_checks import object_row
 from test_launch_shapes_gpu import LATENCY, SHAPES
-from test_objective_gpu import _row_tracks, _weights
+from test_objective_gpu import _objective, _row_tracks
 
 pytestmark = pytest.mark.gpu
 
@@ -35,14 +35,6 @@ HIST = ("out_param_hist", "out_m", "out_v", "out_grad")
 def api():
     from odam_b200 import api
     return api
-
-
-def _objective(tracks, kind):
-    """The keywords of no objective, or of Cauchy with random weights and a cosine schedule."""
-    if kind is None:
-        return {}
-    sched = (0.5 * (1 + np.cos(np.pi * np.arange(N_ITERS) / N_ITERS))).astype(np.float32)
-    return dict(side_weight=_weights(tracks, 9), loss="cauchy", loss_scale=8.0, lr_scale=sched)
 
 
 def _check_against_full(tracks, full, run, keep_best):
@@ -75,7 +67,7 @@ def _check_against_full(tracks, full, run, keep_best):
 def test_rule_against_full_run(api, row, kind):
     """Checks 1-3 on one launch-shape row, without and with an objective."""
     tracks, prior = _row_tracks(row), api.prior_table()
-    obj = _objective(tracks, kind)
+    obj = _objective(tracks, kind, N_ITERS)
     kw = dict(prior=prior, n_iters=N_ITERS, extras=HIST, **row.options, **obj)
     full = api.optimize_host(tracks, **kw)
     stopped = None
@@ -122,7 +114,7 @@ def test_device_entry_and_fused_boxes(api, row):
     oriented boxes equal oriented_boxes_host of the returned parameters."""
     import torch
     tracks, prior = _row_tracks(row), api.prior_table()
-    obj = _objective(tracks, "cauchy")
+    obj = _objective(tracks, "cauchy", N_ITERS)
     kw = dict(n_iters=N_ITERS, keep_best=True, **RULE, **row.options)
     host = api.optimize_host(tracks, prior=prior, extras=("out_corners", "out_box_flag"), **kw, **obj)
     dt = api.DeviceTracks(tracks, "cuda:0", prior)

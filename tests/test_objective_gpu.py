@@ -60,6 +60,14 @@ def _weights(tracks, seed, zeros=0.2):
     return w
 
 
+def _objective(tracks, kind, n_iters):
+    """The keywords of no objective, or of Cauchy with random weights and a cosine schedule."""
+    if kind is None:
+        return {}
+    sched = (0.5 * (1 + np.cos(np.pi * np.arange(n_iters) / n_iters))).astype(np.float32)
+    return dict(side_weight=_weights(tracks, 9), loss="cauchy", loss_scale=8.0, lr_scale=sched)
+
+
 def _same(a, b, keys, label):
     for k in keys:
         assert np.array_equal(a[k], b[k], equal_nan=True), (label, k)
